@@ -1,12 +1,16 @@
 #!/usr/bin/env python
 """Benchmark of the DQNFlappyBird hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--envs-per-gpu E]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--envs-per-gpu E] [--dump-outputs DIR]
 
 One "step" = one batched ``frame_step`` (physics + render + cv2-exact preprocess into the device
 frame ring) over every env of the job, with i.i.d. Bernoulli(0.5) actions (BASELINE.json
 configs[1]: "batched frame_step + preprocess only, random actions").  Metric: env frames/s, whole
 job.  Prints ONE JSON line (rank 0).  See DESIGN.md "Measurement" for every field.
+
+``--dump-outputs DIR`` writes what the last timed step returned on rank 0 as float32 ``DIR/<name>.npy``
+(see ``dump_outputs``).  The inputs are seeded, so two builds run with the same arguments can be
+compared output for output.
 """
 from __future__ import annotations
 
@@ -154,7 +158,7 @@ def cpu_port_updates_per_s(budget_s: float = 6.0):
 def cpu_reference_figures(budget_s: float):
     """The three labelled CPU figures of SURVEY 8(d) for the env half of the path, on this box's host cores:
     as shipped (30 frames/s/process), the reference verbatim on the pygame shim (clock neutralised, one process per core),
-    and the C port (what SDL + cv2 would do natively).  None for the verbatim figure when baseline/_ref was not staged."""
+    and the C port (what SDL + cv2 would do natively).  None for the verbatim figure when oracle/_ref was not staged."""
     from oracle import ref_verbatim as rv
     cores = os.cpu_count() or 1
     out = {"as_shipped_frames_per_s_per_process": 30.0,
@@ -179,10 +183,10 @@ def cpu_reference_figures(budget_s: float):
 
 def run_reference(args, rank: int, world: int):
     """--impl reference: the reference's own CPU implementation of the path for the same metric / config on the box's host
-    cores.  With baseline/_ref staged (build() does it whenever /root/reference is present) this is the reference's
+    cores.  With oracle/_ref staged (build() does it whenever a reference checkout is present) this is the reference's
     game/wrapped_flappy_bird.py run VERBATIM on the pygame shim, one process per core, the 30 frames/s clock neutralised,
     plus the real cv2 preprocess (kind "reference"); the C port's figure (kind "port": what SDL's C blits would cost) and the
-    as-shipped 30 frames/s/process are reported beside it.  Without baseline/_ref: the C port alone."""
+    as-shipped 30 frames/s/process are reported beside it.  Without oracle/_ref: the C port alone."""
     if rank != 0:
         return
     import numpy as np
@@ -228,7 +232,7 @@ def run_reference(args, rank: int, world: int):
         total_t = sum(run(n_steps) for _ in range(args.steps))
         value = n_envs * n_steps * args.steps / total_t
         kind, used = "port", threads
-        sample = f"each bench step = {n_envs} envs x {n_steps} frame_steps of the C port (baseline/_ref not staged: no reference checkout at build time)"
+        sample = f"each bench step = {n_envs} envs x {n_steps} frame_steps of the C port (oracle/_ref not staged: no reference checkout at build time)"
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
         "warmup": args.warmup, "ms_per_step": 1e3 * total_t / args.steps, "higher_is_better": True, "scaling": "weak",
@@ -245,6 +249,31 @@ def run_reference(args, rank: int, world: int):
 
 
 # ------------------------------------------------------------------------------------ GPU arm
+
+DUMP_MAX_ENVS = 1 << 18            # reward / terminal / score / state of at most this many envs: 20 MB
+DUMP_OBS_ENVS = 512                # 80x80 observations of this many envs: 13 MB
+
+
+def dump_outputs(out_dir: str, gs, reward, terminal, score):
+    """What ``frame_step`` hands its caller after the last timed step, as float32 .npy files: reward, terminal and score
+    per env (every env up to DUMP_MAX_ENVS, else a fixed seeded sample, listed in env_index), the 80x80 observation of a
+    fixed seeded sample of DUMP_OBS_ENVS envs (listed in obs_env_index), and the 16-int env state after the step
+    (``GameState.export_state``) of the envs in env_index.  The state carries what every earlier step did: with random
+    actions at p = 0.5 every env crashes on the same step, once every 50 steps, and none ever scores, so the last step
+    alone usually holds no crash and no score.  The samples depend only on the env count."""
+    import numpy as np
+    import torch
+    E = gs.num_envs
+    rng = np.random.default_rng(0)
+    envs = np.arange(E) if E <= DUMP_MAX_ENVS else np.sort(rng.choice(E, DUMP_MAX_ENVS, replace=False))
+    obs_envs = np.sort(rng.choice(E, min(E, DUMP_OBS_ENVS), replace=False))
+    pick = lambda t, idx: t[torch.from_numpy(idx).to(t.device)].cpu().numpy()
+    arrays = {"reward": pick(reward, envs), "terminal": pick(terminal, envs), "score": pick(score, envs), "env_index": envs,
+              "obs": pick(gs.ring[:, gs.slot], obs_envs), "obs_env_index": obs_envs, "state": pick(gs.export_state(), envs)}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.astype(np.float32))
+
 
 def run_ours(args, rank: int, world: int, local_rank: int):
     import torch
@@ -289,6 +318,8 @@ def run_ours(args, rank: int, world: int, local_rank: int):
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     ms_max = float(t.item())
     gs.check_errors()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, gs, rew, term, score)
 
     # ---- e2e: the reference-facing call with HOST buffers (actions in, reward/terminal/score out EVERY step).
     # Measured twice: strictly synchronous (one step in flight), and as a user would drive a throughput job --
@@ -753,7 +784,12 @@ def main():
     ap.add_argument("--no-learner-variants", action="store_true")
     ap.add_argument("--no-closed-loop", action="store_true")
     ap.add_argument("--reference-budget-s", type=float, default=120.0, help="--impl reference: CPU seconds for warm-up + all steps")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="--impl ours: write the last timed step's reward / terminal / score / observations / env state (rank 0) "
+                         "as float32 DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the device path's outputs: it needs --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

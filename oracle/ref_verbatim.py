@@ -8,10 +8,11 @@ need TensorFlow 1.12, neither of which exists in this image.  What CAN run unmod
     ``FlappyBirdDQN.py:31-34``;
   * the ``SumTree`` / ``Memory`` classes of ``BrainPrioritizedReplyDQN.py:32-151`` (AST-extracted, numpy only).
 
-``stage()`` copies exactly those files (plus the sprites they load and the five run logs) from ``/root/reference`` into the
-git-ignored ``baseline/_ref/`` -- the one place the contract allows reference files to live; it is NOT gpurun-ignored, so it
-travels to the GPU box, where ``/root/reference`` does not exist.  ``__graft_entry__.build()`` calls it whenever the reference
-checkout is present.  Nothing under ``dqnflappybird_b200/`` imports this module.
+``stage()`` copies exactly those files (plus the sprites they load and the five run logs) from the reference checkout
+(``$FLAPPY_REFERENCE``, default ``/root/reference``, the ``reference_path`` of BASELINE.json) into the git-ignored
+``oracle/_ref/``; the reference is not part of this repository, and a copied tree that keeps ``oracle/_ref/`` can run the
+verbatim baseline where there is no checkout.  ``__graft_entry__.build()`` calls it; it does nothing when there is no
+checkout.  Nothing under ``dqnflappybird_b200/`` imports this module.
 
 Three env figures are reported by ``bench.py`` (SURVEY 8d), each labelled:
   1. as shipped: 30 frames/s/process -- ``FPSCLOCK.tick(FPS)`` sleeps every frame (wrapped_flappy_bird.py:14,179);
@@ -30,12 +31,14 @@ import sys
 import time
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-DST = os.path.join(ROOT, "baseline", "_ref")
+DST = os.path.join(ROOT, "oracle", "_ref")
 SHIM = os.path.join(ROOT, "oracle", "pygame_shim")
 
 
-def stage(ref_root: str = "/root/reference", dst: str = DST) -> bool:
-    """Copy the files named above from the reference checkout into baseline/_ref (idempotent).  False if there is no checkout."""
+def stage(ref_root: str | None = None, dst: str = DST) -> bool:
+    """Copy the files named above from the reference checkout (default: $FLAPPY_REFERENCE, else /root/reference) into
+    oracle/_ref (idempotent).  False if there is no checkout."""
+    ref_root = ref_root or os.environ.get("FLAPPY_REFERENCE", "/root/reference")
     if not os.path.isdir(os.path.join(ref_root, "game")):
         return False
     os.makedirs(os.path.join(dst, "game"), exist_ok=True)

@@ -1,8 +1,9 @@
 #!/usr/bin/env python
 """Generate the golden fixtures under tests/golden/ from the REAL reference.
 
-Runs only where /root/reference exists (the build container).  Nothing here is
-imported by the tests; the tests read the committed .npz files.
+Needs a checkout of the reference project: $FLAPPY_REFERENCE, default
+/root/reference (as oracle/ref_verbatim.stage).  Nothing here is imported by the
+tests; the tests read the committed .npz files.
 
   ref_env_trajectories.npz
       The reference's own game/wrapped_flappy_bird.py + game/flappy_bird_utils.py,
@@ -148,9 +149,10 @@ def gen_env_trajectories():
         out[f"t{ti}_gaps"] = gaps
         out[f"t{ti}_actions"] = acts; out[f"t{ti}_reward"] = rew; out[f"t{ti}_terminal"] = term
         out[f"t{ti}_score"] = score; out[f"t{ti}_state"] = st; out[f"t{ti}_obsbits"] = obs
-        out[f"t{ti}_frame_idx"] = np.array(keep_idx, np.int32)
-        out[f"t{ti}_frames"] = np.stack(keep_frames)
-        n_frames_kept += len(keep_idx)
+        # every other kept frame: full 288x512x3 frames dominate the file, which stays under 1 MB this way
+        out[f"t{ti}_frame_idx"] = np.array(keep_idx[::2], np.int32)
+        out[f"t{ti}_frames"] = np.stack(keep_frames[::2])
+        n_frames_kept += len(keep_idx[::2])
         print(f"traj {ti} {kind:10s} T={T} crashes={int(term.sum())} scores={int((rew == 3).sum())} "
               f"max_pipes={int(st[:, 7].max())} gaps_used={game.random.used}")
     out["n_traj"] = np.array(len(specs))
@@ -280,6 +282,7 @@ def gen_cv2():
     # low-intensity frames exercise the `> 1` threshold boundary
     frames[2] = rng.integers(0, 6, (288, 512, 3), dtype=np.uint8)
     frames[3] = (rng.random((288, 512, 3)) < 0.02) * rng.integers(0, 256, (288, 512, 3), dtype=np.uint8)
+    frames = frames[[0, 2, 3]]        # one frame of each kind (full range, low intensity, sparse): the file stays under 1 MB
     gray = np.stack([cv2.cvtColor(cv2.resize(f, (80, 80)), cv2.COLOR_BGR2GRAY) for f in frames])
     obs = np.stack([preprocess(f)[:, :, 0] for f in frames])
     np.savez_compressed(os.path.join(HERE, "cv2_preprocess.npz"), frames=frames, gray=gray, obs=obs,

@@ -19,7 +19,7 @@ def test_reference_arm_prints_the_contract_line():
     line = json.loads(r.stdout.strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["unit"] == "frames/s" and line["higher_is_better"] is True
     from oracle import ref_verbatim as rv
-    kind = "reference" if rv.available() else "port"     # baseline/_ref staged by build(): the reference itself, verbatim
+    kind = "reference" if rv.available() else "port"     # oracle/_ref staged by build(): the reference itself, verbatim
     assert line["value"] > 0 and line["cpu_baseline"]["kind"] == kind and line["cpu_baseline"]["cores"] >= 1
     assert line["cpu_baseline"]["c_port"]["kind"] == "port" and line["cpu_baseline"]["c_port"]["value"] > line["value"] * (1 if kind == "reference" else 0)
     assert "30 frames/s" in line["cpu_baseline"]["as_shipped"]
@@ -40,6 +40,14 @@ def test_reference_arm_is_bounded_for_any_step_count():
     line = json.loads(r.stdout.strip().splitlines()[-1])
     assert line["steps"] == 2000 and line["value"] > 0
     assert dt < 120, dt                     # 8 s of samples + interpreter / library start-up
+
+
+def test_reference_arm_refuses_dump_outputs(tmp_path):
+    """--dump-outputs writes the device path's outputs; the reference arm has none, so the combination is an error"""
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1", "--warmup", "1",
+                        "--dump-outputs", str(tmp_path / "out")], capture_output=True, text=True, timeout=600, cwd=ROOT)
+    assert r.returncode == 2 and "--dump-outputs" in r.stderr and r.stdout == ""
+    assert not (tmp_path / "out").exists()
 
 
 def test_learner_cpu_baseline_runs():
@@ -70,14 +78,15 @@ def test_oracle_bf16_emulation_is_close_to_exact_and_rounds_where_the_device_doe
 
 
 def test_reference_runs_verbatim_and_agrees_with_the_port():
-    """baseline/_ref (staged by build() from /root/reference): the reference's env module on the pygame shim, its clock
-    neutralised, gives the same rewards / terminals as the C port driven with the same gaps is checked in test_oracle_env;
-    here: the staging is complete, the worker protocol works, and the reference's PER classes load and sample"""
+    """oracle/_ref (staged by build() from the reference checkout, $FLAPPY_REFERENCE or /root/reference): the reference's env
+    module on the pygame shim, its clock neutralised, gives the same rewards / terminals as the C port driven with the same
+    gaps is checked in test_oracle_env; here: the staging is complete, the worker protocol works, and the reference's PER
+    classes load and sample"""
     import pytest
     from oracle import ref_verbatim as rv
     if not rv.available():
         if not rv.stage():
-            pytest.skip("no reference checkout and baseline/_ref not staged")
+            pytest.skip("no reference checkout ($FLAPPY_REFERENCE, default /root/reference) and oracle/_ref not staged")
     assert rv.available()
     segs = rv.env_segments(2, 12, 2)
     assert len(segs) == 2 and all(t > 0 for t in segs)
