@@ -82,7 +82,8 @@ class StepSampling(C.Structure):
                 ("frames_out_dev", C.c_void_p), ("act_out_dev", C.c_void_p), ("rew_out_dev", C.c_void_p), ("term_out_dev", C.c_void_p),
                 ("env_out_dev", C.c_void_p), ("k_out_dev", C.c_void_p),
                 ("prioritized", C.c_int), ("per_mode", C.c_int), ("beta", C.c_double), ("tree_idx_out_dev", C.c_void_p),
-                ("is_weights_out_dev", C.c_void_p), ("prio_out_dev", C.c_void_p), ("is_weights_f32_out_dev", C.c_void_p)]
+                ("is_weights_out_dev", C.c_void_p), ("prio_out_dev", C.c_void_p), ("is_weights_f32_out_dev", C.c_void_p),
+                ("n_step", C.c_int), ("ret_out_dev", C.c_void_p), ("disc_out_dev", C.c_void_p)]
 
 _SIGNATURES = {
     "fb_last_error": ([], C.c_char_p),

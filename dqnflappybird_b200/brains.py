@@ -19,6 +19,10 @@ head; Q3: the PER brain never syncs its target net; and the PER cost as TensorFl
 ``ISWeights[B,1] * squared_difference[B]`` -- broadcast to [B,B], i.e. mean(w) * mean(err^2),
 BrainPrioritizedReplyDQN.py:243-251); the default runs the intended algorithm (mean of w_i * err_i^2).
 
+``n_step`` (default 1, the reference's target) trains on n-step TD targets: y = R_k + gamma^n X(s_{k+n-1}), cut at the
+first terminal inside the window (replay.py, csrc/fb_replay.cu).  It needs the minibatch drawn inside the update
+(``fuse_sampling``), and for prioritized replay on several ranks the in-step gradient exchange.
+
 All math runs in libflappy_b200.so; with torch.distributed initialised every rank trains on its own env /
 replay shard and the replicated learner sums the ranks' gradients inside the update's CUDA graph over NVLink
 peer memory (fb_dist.cu), or with an NCCL all-reduce before the Adam step when ``peer_exchange=False``.
@@ -63,7 +67,7 @@ class BrainDQN:
                  hidden: int = 512, lr: float = 1e-6, seed: int = 0, first_env_id: int = 0, updates_per_step: int = 1,
                  reference_quirks: bool = False, copy_target_at_init: bool = False, record: bool = False, max_act_batch: int = 4096,
                  precision: str = "fp16", peer_exchange: bool | None = None, root_dir: str | None = None, save_every: int = SAVE_EVERY,
-                 log_capacity: int = 1 << 20):
+                 log_capacity: int = 1 << 20, n_step: int = 1):
         if actionNum != 2:
             raise ValueError("the Flappy Bird hot path has two actions (FlappyBirdDQN.py:38)")
         self.actionNum, self.gameName = actionNum, gameName
@@ -77,6 +81,7 @@ class BrainDQN:
         self.record = record
         self.fuse_sampling = True                  # uniform replay on one GPU: draw the minibatch inside the update's graph
         self.seed, self.first_env_id = seed, first_env_id
+        self.n_step = int(n_step)
         # distributed: one process per GPU, replicated learner (SURVEY 8e)
         self.world = torch.distributed.get_world_size() if torch.distributed.is_available() and torch.distributed.is_initialized() else 1
         from .dist import local_batch as _local_batch
@@ -84,13 +89,13 @@ class BrainDQN:
         self.rank = torch.distributed.get_rank() if self.world > 1 else 0
         # init replay memory (BrainDQN.py:35): REPLAY_MEMORY transitions per env, frames shared with the env's ring
         C = replay_memory_per_env if replay_memory_per_env is not None else (REPLAY_MEMORY if N == 1 else 60)
-        L = C + 4
+        L = C + self.n_step + 3                      # s_{k-1} .. s_{k+n-1} of the oldest live transition (C + 4 for 1-step)
         if ring is None:
             ring = torch.zeros((N, L, 80, 80), dtype=torch.uint8, device=self.device)
-        assert ring.shape == (N, L, 80, 80), f"ring must be u8[{N}][{L}][80][80] (capacity {C} + 4 frames)"
+        assert ring.shape == (N, L, 80, 80), f"ring must be u8[{N}][{L}][80][80] (capacity {C} + {self.n_step + 3} frames)"
         self.ring = ring
         mem_cls = PrioritizedMemory if self.prioritized else ReplayMemory
-        self.replayMemory = mem_cls(ring, C, seed=seed + 1, max_batch=max(self.local_batch, 8))
+        self.replayMemory = mem_cls(ring, C, seed=seed + 1, max_batch=max(self.local_batch, 8), n_step=self.n_step)
         # init other parameters (BrainDQN.py:37-41)
         self.onlineTimeStep = 0
         self.timeStep = 0
@@ -108,6 +113,8 @@ class BrainDQN:
             peer_exchange = self.world > 1 and torch.distributed.get_backend() == "nccl"
         if peer_exchange and self.world > 1:
             self.net.enable_peer_exchange()
+        if self.n_step > 1 and self.prioritized and self.world > 1 and not self.net.exchange_in_step:
+            raise ValueError("n_step > 1 with prioritized replay on several ranks needs the in-step gradient exchange")
         if self.prioritized and self.world > 1:
             self.replayMemory.use_global_min()     # min_prob of Memory.sample over every shard's leaves (one scalar, MIN all-reduce)
         self._k = 0                               # time index of the newest frame in the ring
@@ -243,6 +250,9 @@ class BrainDQN:
         sampling = None
         if self.fuse_sampling and (self.world == 1 or not self.prioritized or self.net.exchange_in_step):
             sampling, mb = mem.step_sampling(self.local_batch)    # random.sample + gather ride at the head of the step's graph
+        elif self.n_step > 1:
+            raise ValueError("n_step > 1 draws its minibatch inside the update: fuse_sampling must stay on (and prioritized replay "
+                             "on several ranks needs the in-step gradient exchange)")
         else:
             mb = mem.sample(self.local_batch)
         isw = mb.is_weights_f32 if mb.is_weights is not None else None   # the placeholder is tf.float32 (BrainPrioritizedReplyDQN.py:243)

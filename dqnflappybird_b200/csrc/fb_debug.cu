@@ -84,7 +84,8 @@ extern "C" int fb_debug_step_sampling_layout(int32_t *out, int capacity) {
                          (int32_t)offsetof(fb_step_sampling, prioritized), (int32_t)offsetof(fb_step_sampling, per_mode),
                          (int32_t)offsetof(fb_step_sampling, beta), (int32_t)offsetof(fb_step_sampling, tree_idx_out_dev),
                          (int32_t)offsetof(fb_step_sampling, is_weights_out_dev), (int32_t)offsetof(fb_step_sampling, prio_out_dev),
-                         (int32_t)offsetof(fb_step_sampling, is_weights_f32_out_dev)};
+                         (int32_t)offsetof(fb_step_sampling, is_weights_f32_out_dev), (int32_t)offsetof(fb_step_sampling, n_step),
+                         (int32_t)offsetof(fb_step_sampling, ret_out_dev), (int32_t)offsetof(fb_step_sampling, disc_out_dev)};
     const int n = (int)(sizeof(v) / sizeof(v[0]));
     FB_REQUIRE(out != nullptr && capacity >= n, "fb_debug_step_sampling_layout: buffer too small");
     for (int i = 0; i < n; i++) out[i] = v[i];

@@ -222,12 +222,13 @@ __global__ void head_forward_kernel(const float *h1, const float *params, QnetLa
 //   variant 0 vanilla: X = max_a Q_online(s')          (BrainDQN.py:204-214)
 //   variant 1 nature : X = max_a Q_target(s')          (BrainDQNNature.py:163-175)
 //   variant 2 double : X = Q_target(s', argmax_a Q_online(s'))   (BrainDoubleDQN.py:51-61)
-//   y = r if terminal else r + gamma * X, built in float64 like the Python loop, fed as fp32.
+//   y = r if terminal else r + gamma * X, built in float64 like the Python loop, fed as fp32 (td_target in fb_qnet.cuh; with
+//   ret / disc the n-step target disc == 0 ? R : R + disc * X).
 //   loss = sum (y-q)^2 (loss_sum, BrainDQN.py:162) | mean (BrainDQNNature.py:119) | mean w (y-q)^2 (PER :251)
 __global__ void td_loss_kernel(const float *q_s, const float *q_next, const float *q_next_online, const uint8_t *actions,
                                const float *rewards, const uint8_t *terminals, const float *isw, int B, int global_batch,
                                int variant, double gamma, int loss_sum, float *dq, float *loss_out, float *abs_err,
-                               float *q_target, int isw_mean) {
+                               float *q_target, int isw_mean, const double *ret, const double *disc) {
     __shared__ float red[32];
     __shared__ float wmean_s;
     float local = 0.f;
@@ -241,9 +242,7 @@ __global__ void td_loss_kernel(const float *q_s, const float *q_next, const floa
         float x;
         if (variant == 2) { int am = q_next_online[b * 2 + 1] > q_next_online[b * 2] ? 1 : 0; x = q_next[b * 2 + am]; }
         else x = fmaxf(q_next[b * 2], q_next[b * 2 + 1]);
-        float rf = rewards[b];
-        double r = rf == 0.1f ? 0.1 : (double)rf;          // the env returns the Python float 0.1
-        float y = (float)(terminals[b] ? r : r + gamma * (double)x);
+        float y = td_target(x, rewards[b], terminals[b], ret, disc, b, gamma);
         int a = actions[b] ? 1 : 0;
         float qa = q_s[b * 2 + a];
         float err = y - qa;
@@ -304,9 +303,10 @@ void qnet_launch_head_forward(const float *h1, const float *params, const QnetLa
 }
 void qnet_launch_td_loss(const float *q_s, const float *q_next, const float *q_next_online, const uint8_t *actions,
                          const float *rewards, const uint8_t *terminals, const float *isw, int B, int global_batch, int variant,
-                         double gamma, int loss_sum, float *dq, float *loss_out, float *abs_err, float *q_target, cudaStream_t st) {
+                         double gamma, int loss_sum, float *dq, float *loss_out, float *abs_err, float *q_target, cudaStream_t st,
+                         const double *ret, const double *disc) {
     td_loss_kernel<<<1, 256, 0, st>>>(q_s, q_next, q_next_online, actions, rewards, terminals, isw, B, global_batch, variant, gamma,
-                                       loss_sum, dq, loss_out, abs_err, q_target, 0);
+                                       loss_sum, dq, loss_out, abs_err, q_target, 0, ret, disc);
 }
 void qnet_launch_head_backward(const float *h1, const float *dq, const float *params, const QnetLayout &L, int B, float *grads,
                                float *dh1_f32, __nv_bfloat16 *dh1_bf16, cudaStream_t st) {
@@ -470,7 +470,7 @@ extern "C" int fb_qnet_layout(const fb_qnet *n, int32_t *o) {
 }
 
 static FrameView make_view(const uint8_t *frames, long long stride, const int32_t *chan_off) {
-    FrameView fv; fv.base = frames; fv.sample_stride = stride; fv.tab = nullptr;
+    FrameView fv; fv.base = frames; fv.sample_stride = stride; fv.tab = nullptr; fv.tab_stride = 0;
     for (int c = 0; c < 4; c++) fv.chan_off[c] = chan_off[c];
     return fv;
 }
@@ -505,12 +505,13 @@ extern "C" int fb_qnet_act(fb_qnet *n, const float *params_dev, const uint8_t *f
     return FB_OK;
 }
 
-extern "C" int fb_qnet_loss_backward(fb_qnet *n, int variant, const float *params_dev, const float *target_params_dev,
-                                     const uint8_t *frames_dev, long long sample_stride, const int32_t *chan_off_s,
-                                     const int32_t *chan_off_next, const uint8_t *actions_dev, const float *rewards_dev,
-                                     const uint8_t *terminals_dev, const float *is_weights_dev, int batch, int global_batch,
-                                     double gamma, int loss_sum, float *grads_dev, float *loss_out_dev, float *abs_err_out_dev,
-                                     float *q_target_out_dev, void *stream) {
+// fb_qnet_loss_backward; ret / disc (f64[batch] or nullptr): the n-step return and discount of each sample (td_target)
+static int loss_backward_impl(fb_qnet *n, int variant, const float *params_dev, const float *target_params_dev,
+                              const uint8_t *frames_dev, long long sample_stride, const int32_t *chan_off_s,
+                              const int32_t *chan_off_next, const uint8_t *actions_dev, const float *rewards_dev,
+                              const uint8_t *terminals_dev, const float *is_weights_dev, int batch, int global_batch,
+                              double gamma, int loss_sum, float *grads_dev, float *loss_out_dev, float *abs_err_out_dev,
+                              float *q_target_out_dev, const double *ret, const double *disc, void *stream) {
     FB_REQUIRE(n && params_dev && frames_dev && chan_off_s && chan_off_next && actions_dev && rewards_dev && terminals_dev && grads_dev,
                "fb_qnet_loss_backward: NULL argument");
     FB_REQUIRE(batch > 0 && batch <= n->max_batch, "fb_qnet_loss_backward: batch exceeds max_batch");
@@ -526,6 +527,7 @@ extern "C" int fb_qnet_loss_backward(fb_qnet *n, int variant, const float *param
         TcTrainArgs ta{variant, params_dev, target_params_dev, fs, fn, actions_dev, rewards_dev, terminals_dev, is_weights_dev, B,
                        global_batch, gamma, loss_sum, grads_dev, loss_out_dev ? loss_out_dev : n->loss_dev, abs_err_out_dev,
                        q_target_out_dev};
+        ta.ret = ret; ta.disc = disc;
         return tc_loss_backward(n, ta, st);
     }
     // Q(s') with the net the variant names (and the online net too for Double), then Q(s) last so that its
@@ -535,7 +537,7 @@ extern "C" int fb_qnet_loss_backward(fb_qnet *n, int variant, const float *param
     rc = forward_chunk(n, params_dev, fs, B, n->q, st); if (rc) return rc;
     td_loss_kernel<<<1, 256, 0, st>>>(n->q, n->q_next, n->q_next_online, actions_dev, rewards_dev, terminals_dev, is_weights_dev,
                                        B, global_batch, variant, gamma, loss_sum, n->dq, loss_out_dev ? loss_out_dev : n->loss_dev,
-                                       abs_err_out_dev, q_target_out_dev, n->per_broadcast);
+                                       abs_err_out_dev, q_target_out_dev, n->per_broadcast, ret, disc);
     // ---- backward
     head_backward_w_kernel<<<(L.hidden + 1 + 127) / 128, 128, 0, st>>>(n->h1, n->dq, L, B, grads_dev);
     head_backward_h_kernel<<<(B * L.hidden + 255) / 256, 256, 0, st>>>(n->h1, n->dq, params_dev, L, B, n->dh1, nullptr);
@@ -554,6 +556,17 @@ extern "C" int fb_qnet_loss_backward(fb_qnet *n, int variant, const float *param
     wgrad<false>(n, kK1, kC1, B * 400, 2048, LoadConv1T{fs}, n->dz1, grads_dev + L.w1, st);
     FB_CUDA_OK(cudaGetLastError());
     return FB_OK;
+}
+
+extern "C" int fb_qnet_loss_backward(fb_qnet *n, int variant, const float *params_dev, const float *target_params_dev,
+                                     const uint8_t *frames_dev, long long sample_stride, const int32_t *chan_off_s,
+                                     const int32_t *chan_off_next, const uint8_t *actions_dev, const float *rewards_dev,
+                                     const uint8_t *terminals_dev, const float *is_weights_dev, int batch, int global_batch,
+                                     double gamma, int loss_sum, float *grads_dev, float *loss_out_dev, float *abs_err_out_dev,
+                                     float *q_target_out_dev, void *stream) {
+    return loss_backward_impl(n, variant, params_dev, target_params_dev, frames_dev, sample_stride, chan_off_s, chan_off_next, actions_dev,
+                              rewards_dev, terminals_dev, is_weights_dev, batch, global_batch, gamma, loss_sum, grads_dev, loss_out_dev,
+                              abs_err_out_dev, q_target_out_dev, nullptr, nullptr, stream);
 }
 
 extern "C" int fb_qnet_adam(fb_qnet *n, float *params_dev, const float *grads_dev, float *m_dev, float *v_dev, float alpha,
@@ -599,7 +612,8 @@ extern "C" int fb_qnet_train_step(fb_qnet *n, int variant, float *params_dev, co
 }
 
 // The same with the minibatch drawn by the step's first two kernels (uniform replay): on the tensor-core path sampling,
-// gather, forward, backward and Adam are one CUDA graph launch.
+// gather, forward, backward and Adam are one CUDA graph launch.  With sp->n_step >= 1 the minibatch rows hold F frames and the
+// TD target is the n-step one (fb_step_sampling).
 extern "C" int fb_qnet_train_step_sampled(fb_qnet *n, const fb_step_sampling *sp, int variant, float *params_dev,
                                           const float *target_params_dev, const int32_t *chan_off_s, const int32_t *chan_off_next,
                                           int global_batch, double gamma, int loss_sum, float *grads_dev, float *loss_out_dev,
@@ -609,40 +623,53 @@ extern "C" int fb_qnet_train_step_sampled(fb_qnet *n, const fb_step_sampling *sp
                "fb_qnet_train_step_sampled: NULL argument");
     const bool adam = m_dev != nullptr;            // without Adam slots: gradients only (the caller applies Adam, e.g. fb_dist_adam)
     const int batch = sp->batch;
+    const int F = replay_frames_per_sample(*sp);   // frames per minibatch row: 5, or 4 + min(n, 4) with n-step returns
+    const double *ret = sp->n_step > 0 ? sp->ret_out_dev : nullptr, *disc = sp->n_step > 0 ? sp->disc_out_dev : nullptr;
     if (tc_precision(n->precision) && n->tc != nullptr) {
         FB_REQUIRE(batch > 0 && batch <= n->max_batch, "fb_qnet_train_step_sampled: batch exceeds max_batch");
         FB_REQUIRE(variant >= 0 && variant <= 2, "fb_qnet_train_step_sampled: variant must be 0 (vanilla), 1 (nature) or 2 (double)");
         FB_REQUIRE(variant == 0 || target_params_dev != nullptr, "fb_qnet_train_step_sampled: target parameters required");
         if (global_batch <= 0) global_batch = batch;
-        FrameView fs = make_view(sp->frames_out_dev, 5 * 6400, chan_off_s), fn = make_view(sp->frames_out_dev, 5 * 6400, chan_off_next);
+        FrameView fs = make_view(sp->frames_out_dev, F * 6400, chan_off_s), fn = make_view(sp->frames_out_dev, F * 6400, chan_off_next);
         // channels that are whole frames of the minibatch buffer (the usual 0..3 / 1..4): the convolutions read them in place from
         // the ring through the offsets the sampler leaves behind; the gather into frames_out_dev runs beside the forward passes
         bool in_place = sp->ring_dev != nullptr;
-        for (int c = 0; c < 4; c++) in_place = in_place && chan_off_s[c] % 6400 == 0 && chan_off_s[c] / 6400 <= 4 && chan_off_s[c] >= 0 &&
-                                               chan_off_next[c] % 6400 == 0 && chan_off_next[c] / 6400 <= 4 && chan_off_next[c] >= 0;
+        for (int c = 0; c < 4; c++) in_place = in_place && chan_off_s[c] % 6400 == 0 && chan_off_s[c] / 6400 < F && chan_off_s[c] >= 0 &&
+                                               chan_off_next[c] % 6400 == 0 && chan_off_next[c] / 6400 < F && chan_off_next[c] >= 0;
         if (in_place) {
             fs.base = fn.base = sp->ring_dev; fs.sample_stride = fn.sample_stride = 0; fs.tab = fn.tab = replay_frame_tab(sp->replay);
+            fs.tab_stride = fn.tab_stride = F;
             for (int c = 0; c < 4; c++) { fs.chan_off[c] = chan_off_s[c] / 6400; fn.chan_off[c] = chan_off_next[c] / 6400; }
         }
         FB_REQUIRE(!sp->prioritized || abs_err_out_dev != nullptr, "fb_qnet_train_step_sampled: prioritized replay needs abs_err_out_dev");
         TcTrainArgs ta{variant, params_dev, target_params_dev, fs, fn, sp->act_out_dev, sp->rew_out_dev, sp->term_out_dev,
                        sp->prioritized ? sp->is_weights_f32_out_dev : nullptr, batch,
                        global_batch, gamma, loss_sum, grads_dev, loss_out_dev ? loss_out_dev : n->loss_dev, abs_err_out_dev,
-                       q_target_out_dev, AdamFuse{adam ? 1 : 0, m_dev, v_dev, lr, beta1, beta2, eps, grad_scale}, adam ? n->xch : nullptr, *sp};
+                       q_target_out_dev, AdamFuse{adam ? 1 : 0, m_dev, v_dev, lr, beta1, beta2, eps, grad_scale}, adam ? n->xch : nullptr, *sp,
+                       ret, disc};
         return adam ? tc_train_step(n, ta, beta1_power, beta2_power, (cudaStream_t)stream) : tc_loss_backward(n, ta, (cudaStream_t)stream);
     }
     FB_REQUIRE(!sp->prioritized || abs_err_out_dev != nullptr, "fb_qnet_train_step_sampled: prioritized replay needs abs_err_out_dev");
-    int rc = replay_launch_sample_gather(*sp, (cudaStream_t)stream);
+    int rc = replay_launch_sample_gather(*sp, gamma, (cudaStream_t)stream);
     if (rc) return rc;
     if (!adam)
-        rc = fb_qnet_loss_backward(n, variant, params_dev, target_params_dev, sp->frames_out_dev, 5 * 6400, chan_off_s, chan_off_next,
-                                   sp->act_out_dev, sp->rew_out_dev, sp->term_out_dev, sp->prioritized ? sp->is_weights_f32_out_dev : nullptr,
-                                   batch, global_batch, gamma, loss_sum, grads_dev, loss_out_dev, abs_err_out_dev, q_target_out_dev, stream);
-    else
+        rc = loss_backward_impl(n, variant, params_dev, target_params_dev, sp->frames_out_dev, F * 6400, chan_off_s, chan_off_next,
+                                sp->act_out_dev, sp->rew_out_dev, sp->term_out_dev, sp->prioritized ? sp->is_weights_f32_out_dev : nullptr,
+                                batch, global_batch, gamma, loss_sum, grads_dev, loss_out_dev, abs_err_out_dev, q_target_out_dev, ret, disc, stream);
+    else if (ret == nullptr)
     rc = fb_qnet_train_step(n, variant, params_dev, target_params_dev, sp->frames_out_dev, 5 * 6400, chan_off_s, chan_off_next,
                             sp->act_out_dev, sp->rew_out_dev, sp->term_out_dev, sp->prioritized ? sp->is_weights_f32_out_dev : nullptr, batch,
                             global_batch, gamma, loss_sum, grads_dev, loss_out_dev, abs_err_out_dev, q_target_out_dev, m_dev, v_dev, lr, beta1,
                             beta2, eps, grad_scale, beta1_power, beta2_power, stream);
+    else {                                         // fb_qnet_train_step's CUDA-core path with the n-step target
+        rc = loss_backward_impl(n, variant, params_dev, target_params_dev, sp->frames_out_dev, F * 6400, chan_off_s, chan_off_next,
+                                sp->act_out_dev, sp->rew_out_dev, sp->term_out_dev, sp->prioritized ? sp->is_weights_f32_out_dev : nullptr,
+                                batch, global_batch, gamma, loss_sum, grads_dev, loss_out_dev, abs_err_out_dev, q_target_out_dev, ret, disc, stream);
+        if (rc == FB_OK) {
+            const float alpha = lr * sqrtf(1.f - beta2_power) / (1.f - beta1_power);
+            rc = fb_qnet_adam(n, params_dev, grads_dev, m_dev, v_dev, alpha, beta1, beta2, eps, grad_scale, stream);
+        }
+    }
     if (rc) return rc;
     return sp->prioritized ? replay_launch_per_update(*sp, abs_err_out_dev, (cudaStream_t)stream) : FB_OK;
 }

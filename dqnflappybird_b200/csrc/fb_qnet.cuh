@@ -42,12 +42,26 @@ struct FrameView {              // where the 4 input channels of each sample liv
     const uint8_t *base;
     long long sample_stride;    // bytes between consecutive samples
     int chan_off[4];            // byte offset of channel c (oldest frame first, newest last: BrainDQN.py:68)
-    const long long *tab;       // nullptr, or [sample][5] byte offsets from `base` (replay samples read in place from the frame ring:
-                                // the sampler wrote them); chan_off[c] is then the FRAME (0..4) channel c is, sample_stride unused
+    const long long *tab;       // nullptr, or [sample][tab_stride] byte offsets from `base` (replay samples read in place from the frame
+                                // ring: the sampler wrote them); chan_off[c] is then the FRAME (0..tab_stride-1) channel c is, sample_stride unused
+    int tab_stride;             // frames per sample in `tab`: 5 (1-step), 4 + min(n, 4) (n-step)
     __host__ __device__ const uint8_t *chan(int b, int c) const {
-        return tab ? base + tab[b * 5 + chan_off[c]] : base + (size_t)b * sample_stride + chan_off[c];
+        return tab ? base + tab[b * tab_stride + chan_off[c]] : base + (size_t)b * sample_stride + chan_off[c];
     }
 };
+
+// The TD target of one sample, as the Python loop builds it in float64 and feeds it as fp32 (BrainDQN.py:208-214).  X is the
+// variant's bootstrap value on s' (fp32).  ret == nullptr: the 1-step target y = r if terminal else r + gamma X, with the env's
+// Python float 0.1.  ret != nullptr: the n-step target of fb_step_sampling.n_step, y = disc == 0 ? R : R + disc X; at n = 1
+// R == r and disc == (terminal ? 0 : gamma) exactly, so both forms give the same bits.
+__device__ __forceinline__ float td_target(float x, float rf, uint8_t terminal, const double *ret, const double *disc, int b, double gamma) {
+    if (ret != nullptr) {
+        const double R = ret[b], d = disc[b];
+        return (float)(d == 0.0 ? R : R + d * (double)x);
+    }
+    const double r = rf == 0.1f ? 0.1 : (double)rf;          // the env returns the Python float 0.1
+    return (float)(terminal ? r : r + gamma * (double)x);
+}
 
 // ---- handle shared by the strict-fp32 path (fb_qnet.cu) and the tcgen05 path (fb_qnet_tc.cu) ------------
 struct fb_dist;                 // multi-GPU gradient exchange (fb_dist.cu)
@@ -70,9 +84,11 @@ struct fb_qnet {
 
 // small CUDA-core stages both paths share (defined in fb_qnet.cu)
 void qnet_launch_head_forward(const float *h1, const float *params, const QnetLayout &L, int B, float *q, cudaStream_t st);
+// ret / disc (f64[B], both or neither): n-step return and discount per sample (td_target); nullptr: the 1-step target
 void qnet_launch_td_loss(const float *q_s, const float *q_next, const float *q_next_online, const uint8_t *actions,
                          const float *rewards, const uint8_t *terminals, const float *isw, int B, int global_batch, int variant,
-                         double gamma, int loss_sum, float *dq, float *loss_out, float *abs_err, float *q_target, cudaStream_t st);
+                         double gamma, int loss_sum, float *dq, float *loss_out, float *abs_err, float *q_target, cudaStream_t st,
+                         const double *ret = nullptr, const double *disc = nullptr);
 void qnet_launch_head_backward(const float *h1, const float *dq, const float *params, const QnetLayout &L, int B, float *grads,
                                float *dh1_f32, __nv_bfloat16 *dh1_bf16, cudaStream_t st);
 
@@ -90,17 +106,21 @@ struct TcTrainArgs {
     AdamFuse ad;                            // ad.on: params is updated in place at the end of the step
     fb_dist *xch;                           // with ad.on: Adam over the SUM of all ranks' gradients (buckets of fb_dist.cu inside the graph)
     fb_step_sampling pro;                   // pro.replay != nullptr: the minibatch is drawn by the step's first two kernels
+    const double *ret, *disc;               // n-step return / discount per sample (pro.n_step >= 1), else nullptr: 1-step target
 };
 // fb_replay.cu: the two kernels of fb_replay_sample_uniform + fb_replay_gather on `st`; and the per-step patch of their
-// nodes in an instantiated graph (`t` is the only argument that changes)
-int replay_launch_sample_gather(const fb_step_sampling &p, cudaStream_t st);
+// nodes in an instantiated graph (`t` -- and through it the n-step horizon t - n + 1 -- is the only argument that changes).
+// gamma: the step's discount, which the n-step gather folds into R and disc.
+int replay_launch_sample_gather(const fb_step_sampling &p, double gamma, cudaStream_t st);
 int replay_launch_sample(const fb_step_sampling &p, bool with_tab, cudaStream_t st);   // with_tab: ring offsets of the drawn frames -> replay_frame_tab
-int replay_launch_gather(const fb_step_sampling &p, cudaStream_t st);
-const long long *replay_frame_tab(const fb_replay *r);                                   // [batch][5] byte offsets into the frame ring
+int replay_launch_gather(const fb_step_sampling &p, double gamma, cudaStream_t st);
+const long long *replay_frame_tab(const fb_replay *r);                                   // [batch][F] byte offsets into the frame ring
+int replay_frames_per_sample(const fb_step_sampling &p);                                 // F: 5 (1-step), 4 + min(n, 4) (n-step)
 int replay_launch_per_update(const fb_step_sampling &p, const float *abs_err_dev, cudaStream_t st);     // Memory.batch_update, prioritized only
 bool replay_is_sampler(const void *func);        // sample_uniform_kernel or per_sample_kernel
 bool replay_is_gather(const void *func);
-int replay_patch_nodes(cudaGraphExec_t exec, cudaGraphNode_t sampler, cudaGraphNode_t gather, const fb_step_sampling &p, bool with_tab);
+int replay_patch_nodes(cudaGraphExec_t exec, cudaGraphNode_t sampler, cudaGraphNode_t gather, const fb_step_sampling &p, double gamma,
+                       bool with_tab);
 inline bool tc_precision(int precision) { return precision == FB_PRECISION_BF16 || precision == FB_PRECISION_FP16; }
 // fb_dist.cu: one bucket of the exchange + Adam as a kernel on `st` (bucket 0 = W_fc1, 1 = the rest), for the exchange buffer of
 // the current parity; the buffer the step's gradients must have been written to

@@ -603,6 +603,7 @@ struct TdFuse {
     const float *q_next, *q_next_online, *rewards, *isw;
     const uint8_t *actions, *terminals;
     float *dq, *abs_err, *q_target, *loss_terms;
+    const double *ret, *disc;         // n-step return / discount per sample, or nullptr: the 1-step target (td_target, fb_qnet.cuh)
 };
 __global__ void __launch_bounds__(128) fc1_head_kernel(const float *__restrict__ part, int splits, size_t split_stride,
                                                       const float *__restrict__ params, QnetLayout L, int B, float *__restrict__ h1,
@@ -638,9 +639,7 @@ __global__ void __launch_bounds__(128) fc1_head_kernel(const float *__restrict__
             float x;
             if (td.variant == 2) { int am = td.q_next_online[b * 2 + 1] > td.q_next_online[b * 2] ? 1 : 0; x = td.q_next[b * 2 + am]; }
             else x = fmaxf(td.q_next[b * 2], td.q_next[b * 2 + 1]);
-            const float rf = td.rewards[b];
-            const double r = rf == 0.1f ? 0.1 : (double)rf;
-            const float y = (float)(td.terminals[b] ? r : r + td.gamma * (double)x);
+            const float y = td_target(x, td.rewards[b], td.terminals[b], td.ret, td.disc, b, td.gamma);
             const int a = td.actions[b] ? 1 : 0;
             const float err = y - q[b * 2 + a];
             float w = td.isw ? td.isw[b] : 1.f;
@@ -768,9 +767,7 @@ __global__ void __launch_bounds__(128) fc1_head_train_kernel(const float *__rest
         float xn;
         if (td.variant == 2) { const int am = td.q_next_online[b * 2 + 1] > td.q_next_online[b * 2] ? 1 : 0; xn = td.q_next[b * 2 + am]; }
         else xn = fmaxf(td.q_next[b * 2], td.q_next[b * 2 + 1]);
-        const float rf = td.rewards[b];
-        const double r = rf == 0.1f ? 0.1 : (double)rf;
-        const float y = (float)(td.terminals[b] ? r : r + td.gamma * (double)xn);
+        const float y = td_target(xn, td.rewards[b], td.terminals[b], td.ret, td.disc, b, td.gamma);
         const int a = td.actions[b] ? 1 : 0;
         const float err = y - (a ? q1 : q0);
         const float w = td.isw ? (td.isw_mean ? wmean : td.isw[b]) : 1.f;
@@ -1837,7 +1834,7 @@ int tc_forward_chunks(fb_qnet *n, int slot, const float *params_dev, const uint8
     for (int b0 = 0; b0 < batch; b0 += n->max_batch, c++) {
         const int B = min(n->max_batch, batch - b0), w = two ? (c & 1) : 0;
         FrameView fv;
-        fv.base = frames_dev + (size_t)b0 * sample_stride; fv.sample_stride = sample_stride; fv.tab = nullptr;
+        fv.base = frames_dev + (size_t)b0 * sample_stride; fv.sample_stride = sample_stride; fv.tab = nullptr; fv.tab_stride = 0;
         for (int k = 0; k < 4; k++) fv.chan_off[k] = chan_off[k];
         int rc = tc_forward(n, slot, w, params_dev, fv, B, q_out_dev + (size_t)b0 * 2, w ? t->aux : st);
         if (rc) return rc;
@@ -1880,9 +1877,9 @@ int train_step_launch(fb_qnet *n, const TcTrainArgs &a, int pack_online, int pac
         if (in_place) {
             FB_CUDA_OK(cudaEventRecord(t->ev[e_gather], st));
             FB_CUDA_OK(cudaStreamWaitEvent(t->aux4, t->ev[e_gather], 0));
-            rc = replay_launch_gather(a.pro, t->aux4); if (rc) return rc;
+            rc = replay_launch_gather(a.pro, a.gamma, t->aux4); if (rc) return rc;
             FB_CUDA_OK(cudaEventRecord(t->ev[e_gather], t->aux4));
-        } else { rc = replay_launch_gather(a.pro, st); if (rc) return rc; }
+        } else { rc = replay_launch_gather(a.pro, a.gamma, st); if (rc) return rc; }
     }
     if (pack_online) { rc = tc_pack_weights(n, a.params, 0, st); if (rc) return rc; }
     FB_CUDA_OK(fork(st, sx));
@@ -1905,7 +1902,7 @@ int train_step_launch(fb_qnet *n, const TcTrainArgs &a, int pack_online, int pac
         FB_CUDA_OK(cudaEventRecord(t->ev[e_x2], t->aux4));
     }
     TdFuse td{1, a.variant, a.loss_sum, a.global_batch, n->per_broadcast, a.gamma, n->q_next, n->q_next_online, a.rewards, a.isw, a.actions,
-              a.terminals, n->dq, a.abs_err, a.q_target, t->loss_terms};
+              a.terminals, n->dq, a.abs_err, a.q_target, t->loss_terms, a.ret, a.disc};
     const AdamPow apow{a.ad.on, t->adam_pow, t->adam_pow + 2, a.ad.lr, a.ad.beta1, a.ad.beta2};
     // fp16 operands: gradient tensors carry a power-of-two factor that keeps them in fp16's normal range (dq ~ err / batch for the
     // mean losses); it is removed exactly where weight / bias gradients are finalised.  bf16: 1.
@@ -2065,7 +2062,8 @@ int tc_loss_backward(fb_qnet *n, const TcTrainArgs &a, cudaStream_t st) {
     key.a.variant = a.variant; key.a.params = a.params; key.a.target = a.target;
     key.a.fs.base = a.fs.base; key.a.fs.sample_stride = a.fs.sample_stride; key.a.fn.base = a.fn.base; key.a.fn.sample_stride = a.fn.sample_stride;
     for (int c = 0; c < 4; c++) { key.a.fs.chan_off[c] = a.fs.chan_off[c]; key.a.fn.chan_off[c] = a.fn.chan_off[c]; }
-    key.a.fs.tab = a.fs.tab; key.a.fn.tab = a.fn.tab;
+    key.a.fs.tab = a.fs.tab; key.a.fn.tab = a.fn.tab; key.a.fs.tab_stride = a.fs.tab_stride; key.a.fn.tab_stride = a.fn.tab_stride;
+    key.a.ret = a.ret; key.a.disc = a.disc;
     key.a.actions = a.actions; key.a.rewards = a.rewards; key.a.terminals = a.terminals; key.a.isw = a.isw;
     key.a.B = a.B; key.a.global_batch = a.global_batch; key.a.gamma = a.gamma; key.a.loss_sum = a.loss_sum;
     key.a.grads = a.grads; key.a.loss_out = a.loss_out; key.a.abs_err = a.abs_err; key.a.q_target = a.q_target;
@@ -2080,6 +2078,7 @@ int tc_loss_backward(fb_qnet *n, const TcTrainArgs &a, cudaStream_t st) {
         k.k_out_dev = q.k_out_dev;
         k.prioritized = q.prioritized; k.per_mode = q.per_mode; k.tree_idx_out_dev = q.tree_idx_out_dev;       // (beta is patched like t)
         k.is_weights_out_dev = q.is_weights_out_dev; k.prio_out_dev = q.prio_out_dev; k.is_weights_f32_out_dev = q.is_weights_f32_out_dev;
+        k.n_step = q.n_step; k.ret_out_dev = q.ret_out_dev; k.disc_out_dev = q.disc_out_dev;     // n: frames per row, gather grid, horizon
     }
     key.pack_online = n->packed_src[0] != a.params;
     key.pack_target = a.variant != 0 && n->packed_src[1] != a.target;
@@ -2094,7 +2093,7 @@ int tc_loss_backward(fb_qnet *n, const TcTrainArgs &a, cudaStream_t st) {
         }
     }
     if (ge && ge->exec) {
-        if (a.pro.replay != nullptr) { rc = replay_patch_nodes(ge->exec, ge->n_sampler, ge->n_gather, a.pro, a.fs.tab != nullptr); if (rc) return rc; }
+        if (a.pro.replay != nullptr) { rc = replay_patch_nodes(ge->exec, ge->n_sampler, ge->n_gather, a.pro, a.gamma, a.fs.tab != nullptr); if (rc) return rc; }
         FB_CUDA_OK(cudaGraphLaunch(ge->exec, st));
     } else if (ge && ge->seen >= 1) {            // second identical call: capture (everything lazy was initialised by the first)
         cudaGraph_t graph = nullptr;

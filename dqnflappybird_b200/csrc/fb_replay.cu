@@ -13,6 +13,13 @@
 // transitions per env the live set at time t is k in [max(1, t-C+1), t]; the population index of
 // random.sample / the SumTree data index is   j = e * cnt + (k - k_lo)   resp.   e * C + (k-1) % C,
 // which for N = 1 is exactly the reference's deque / data_pointer order.
+//
+// n-step returns (fb_step_sampling.n_step = n >= 1) need nothing stored beyond that: transition k becomes
+// (s_{k-1}, a_k, R_k, s_{k+n-1}, disc_k) -- the same lookup, n reward / terminal rows and a later frame window.  It can be drawn
+// once its horizon is complete (k + n - 1 <= t), so every index is decoded at t_eff = t - n + 1: the uniform population at t
+// is exactly the 1-step population at t_eff, and a prioritized memory stores transition t_eff at time t.  Frames then span
+// s_{k-1} .. s_{k+n-1}, hence L >= C + n + 3.  The gather copies F = 4 + min(n, 4) frames per sample (times k-4..k-1, then
+// k-4+n .. k-1+n without the overlap) and one thread per sample walks the n rows for R_k and disc_k in float64.
 #include <new>
 
 #include "fb_common.cuh"
@@ -49,25 +56,37 @@ __device__ __forceinline__ void decode_transition(int per, long long t, int cap,
         *k = t - back;
     }
 }
-// Where the five frames of each drawn transition live in the ring (byte offsets), written by the sampler itself: the training
+// Frame f of a sample's minibatch row, as a time offset from its transition k: s = k-4..k-1 (f < 4), s' = the n-step window
+// k-4+n .. k-1+n without the frames s already holds (n <= 4: one consecutive run of F = 4 + n frames; n > 4: two runs of four).
+// n = 1 is the 1-step row: five consecutive frames k-4..k.
+__host__ __device__ __forceinline__ int frames_per_sample(int n) { return 4 + (n < 4 ? n : 4); }
+__device__ __forceinline__ int frame_time_offset(int f, int n) { return f < 4 ? f - 4 : f - 4 + n - (n < 4 ? n : 4); }
+
+// Where the F frames of each drawn transition live in the ring (byte offsets), written by the sampler itself: the training
 // step's first convolution reads them in place, so the gather that fills the caller-visible minibatch buffers runs beside the
-// forward passes instead of ahead of them.  tab == nullptr: not wanted.
-struct FrameTabArgs { long long *tab; long long t; int cap, L, per; };
+// forward passes instead of ahead of them.  tab == nullptr: not wanted.  t: the time indices are decoded at (t_eff for
+// n-step); n: the horizon (1 for the 1-step transitions).
+struct FrameTabArgs { long long *tab; long long t; int cap, L, per, n; };
 __device__ __forceinline__ void write_frame_tab(const FrameTabArgs &ft, int b, long long j) {
     int e; long long k;
     decode_transition(ft.per, ft.t, ft.cap, j, &e, &k);
+    const int F = frames_per_sample(ft.n);
+    long long *row = ft.tab + (size_t)b * F;
     if (k >= 4) {
         int slot = (int)((k - 4) % ft.L);                 // one 64-bit remainder, then the ring is walked
 #pragma unroll
-        for (int f = 0; f < 5; f++) {
-            ft.tab[b * 5 + f] = ((long long)e * ft.L + slot) * 6400;
+        for (int f = 0; f < 8; f++) {
+            if (f >= F) break;
+            if (f == 4 && ft.n > 4) slot = (int)((k - 4 + ft.n) % ft.L);   // the second run of four (n > 4)
+            row[f] = ((long long)e * ft.L + slot) * 6400;
             if (++slot == ft.L) slot = 0;
         }
     } else {
 #pragma unroll
-        for (int f = 0; f < 5; f++) {
-            long long tf = k - 4 + f; if (tf < 0) tf = 0;             // setInitState replication of frame 0
-            ft.tab[b * 5 + f] = ((long long)e * ft.L + tf % ft.L) * 6400;
+        for (int f = 0; f < 8; f++) {
+            if (f >= F) break;
+            long long tf = k + frame_time_offset(f, ft.n); if (tf < 0) tf = 0;     // setInitState replication of frame 0
+            row[f] = ((long long)e * ft.L + tf % ft.L) * 6400;
         }
     }
 }
@@ -150,24 +169,27 @@ __global__ void __launch_bounds__(kSampThreads) sample_uniform_kernel(uint32_t n
 struct GatherArgs {
     const uint8_t *ring; int N, L;
     const uint8_t *act; const float *rew; const uint8_t *term;       // [L][N]
-    long long t;                 // time of the newest stored transition
+    long long t;                 // time the indices are decoded at: the newest stored transition (t_eff = t - n + 1 for n-step)
     int cap;                     // C, transitions kept per env
     int per;                     // 0: idx is a population index of random.sample; 1: a SumTree data index
     const int32_t *idx; int batch;
-    uint8_t *frames;             // [batch][5][80][80]
+    uint8_t *frames;             // [batch][F][80][80], F = frames_per_sample(n)
     uint8_t *a_out; float *r_out; uint8_t *t_out;
     int32_t *env_out, *k_out;    // optional
+    int n;                       // horizon: 1 (1-step), or the n-step n, for which ret_out / disc_out are written
+    double gamma;
+    double *ret_out, *disc_out;  // f64[batch] or nullptr (1-step)
 };
 
 // one CTA per (sample, frame): 6,400 bytes, every thread's loads issued together (the ring is HBM-cold)
 __global__ void __launch_bounds__(128) gather_kernel(GatherArgs g) {
-    const int b = blockIdx.x, f = blockIdx.y;
+    const int b = blockIdx.x, f = blockIdx.y, F = gridDim.y;
     if (b >= g.batch) return;
     long long k; int e;
     decode_transition(g.per, g.t, g.cap, g.idx[b], &e, &k);
-    long long tf = k - 4 + f; if (tf < 0) tf = 0;                     // setInitState replication of frame 0
+    long long tf = k + frame_time_offset(f, g.n); if (tf < 0) tf = 0;   // setInitState replication of frame 0
     const uint4 *src = reinterpret_cast<const uint4 *>(g.ring) + ((size_t)e * g.L + (size_t)(tf % g.L)) * 400;
-    uint4 *dst = reinterpret_cast<uint4 *>(g.frames) + (size_t)b * 2000 + f * 400;
+    uint4 *dst = reinterpret_cast<uint4 *>(g.frames) + (size_t)b * F * 400 + f * 400;
     uint4 v[4];
 #pragma unroll
     for (int q = 0; q < 4; q++) { int i = threadIdx.x + q * 128; v[q] = i < 400 ? __ldg(src + i) : make_uint4(0u, 0u, 0u, 0u); }
@@ -178,6 +200,23 @@ __global__ void __launch_bounds__(128) gather_kernel(GatherArgs g) {
         g.a_out[b] = g.act[m]; g.r_out[b] = g.rew[m]; g.t_out[b] = g.term[m];
         if (g.env_out) g.env_out[b] = e;
         if (g.k_out) g.k_out[b] = (int32_t)k;
+        if (g.ret_out) {
+            // R = sum_{i<m} gamma^i r_{k+i}, accumulated forward in float64 (no fused multiply-add: the oracle's roundings),
+            // cut after the first terminal; disc = 0 after a terminal, else the running product gamma^n
+            double R = 0.0, gm = 1.0;
+            bool hit = false;
+            int row = (int)(k % g.L);
+            for (int i = 0; i < g.n && !hit; i++) {
+                const size_t mi = (size_t)row * g.N + e;
+                const float rf = g.rew[mi];
+                R = __dadd_rn(R, __dmul_rn(gm, rf == 0.1f ? 0.1 : (double)rf));      // the env returns the Python float 0.1
+                gm = __dmul_rn(gm, g.gamma);
+                hit = g.term[mi] != 0;
+                if (++row == g.L) row = 0;
+            }
+            g.ret_out[b] = R;
+            g.disc_out[b] = hit ? 0.0 : gm;
+        }
     }
 }
 
@@ -461,7 +500,7 @@ struct fb_replay {
     int N, L, C, cap;
     double *tree;                    // PER only
     double *mn, *mx;                 // min-positive / max trees of the same shape (see the SumTree section)
-    long long *frame_tab;            // [512][5] ring offsets of the drawn transitions' frames (see FrameTabArgs)
+    long long *frame_tab;            // [512][F <= 8] ring offsets of the drawn transitions' frames (see FrameTabArgs)
     const double *gmin;              // nullptr, or the caller's device scalar: smallest positive leaf over ALL shards (several GPUs)
     unsigned int *counters;          // [0] per_store_multi_kernel, [1] per_sample_kernel: "last CTA" counters, self-resetting
     int32_t *leaves; double *prio; double *change;   // scratch, max(N, max_batch)
@@ -480,8 +519,8 @@ extern "C" int fb_replay_create(int n_envs, int ring_len, int capacity_per_env, 
     FB_CUDA_OK(cudaMalloc(&r->word_pos, 2 * sizeof(unsigned long long)));
     FB_CUDA_OK(cudaMemset(r->word_pos, 0, 2 * sizeof(unsigned long long)));
     r->mn = r->mx = nullptr; r->gmin = nullptr;
-    FB_CUDA_OK(cudaMalloc(&r->frame_tab, 512 * 5 * sizeof(long long)));
-    FB_CUDA_OK(cudaMemset(r->frame_tab, 0, 512 * 5 * sizeof(long long)));
+    FB_CUDA_OK(cudaMalloc(&r->frame_tab, 512 * 8 * sizeof(long long)));
+    FB_CUDA_OK(cudaMemset(r->frame_tab, 0, 512 * 8 * sizeof(long long)));
     FB_CUDA_OK(cudaMalloc(&r->counters, 2 * sizeof(unsigned int)));
     FB_CUDA_OK(cudaMemset(r->counters, 0, 2 * sizeof(unsigned int)));
     FB_CUDA_OK(cudaMalloc(&r->leaves, sizeof(int32_t) * r->scratch_n));
@@ -518,7 +557,7 @@ extern "C" int fb_replay_sample_uniform(fb_replay *r, long long t, int batch, ui
     long long n = (t - k_lo + 1) * r->N;
     if (t < 1 || n < batch) { fb_set_error("Sample larger than population or is negative"); return FB_ERR_INVALID; }   // random.sample's ValueError
     FB_REQUIRE(setsize <= 2u * kHashSize, "fb_replay_sample_uniform: setsize too large");
-    sample_uniform_kernel<<<1, kSampThreads, 0, (cudaStream_t)stream>>>((uint32_t)n, batch, setsize, seed, r->word_pos, idx_out_dev, FrameTabArgs{nullptr, 0, 0, 0, 0});
+    sample_uniform_kernel<<<1, kSampThreads, 0, (cudaStream_t)stream>>>((uint32_t)n, batch, setsize, seed, r->word_pos, idx_out_dev, FrameTabArgs{nullptr, 0, 0, 0, 0, 1});
     FB_CUDA_OK(cudaGetLastError());
     return FB_OK;
 }
@@ -530,39 +569,51 @@ extern "C" int fb_replay_gather(fb_replay *r, const uint8_t *ring_dev, const uin
     FB_REQUIRE(r && ring_dev && act_dev && rew_dev && term_dev && idx_dev && frames_out_dev && act_out_dev && rew_out_dev && term_out_dev && batch > 0,
                "fb_replay_gather: bad argument");
     GatherArgs g{ring_dev, r->N, r->L, act_dev, rew_dev, term_dev, t, r->C, prioritized_index, idx_dev, batch,
-                 frames_out_dev, act_out_dev, rew_out_dev, term_out_dev, env_out_dev, k_out_dev};
+                 frames_out_dev, act_out_dev, rew_out_dev, term_out_dev, env_out_dev, k_out_dev, 1, 0.0, nullptr, nullptr};
     gather_kernel<<<dim3(batch, 5), 128, 0, (cudaStream_t)stream>>>(g);
     FB_CUDA_OK(cudaGetLastError());
     return FB_OK;
 }
 
 static void launch_per_sample(fb_replay *r, int batch, double beta, uint64_t seed, int32_t *tree_idx, int32_t *data_idx, double *isw, double *prio,
-                              float *isw32, cudaStream_t st, FrameTabArgs ft = FrameTabArgs{nullptr, 0, 0, 0, 0}) {
+                              float *isw32, cudaStream_t st, FrameTabArgs ft = FrameTabArgs{nullptr, 0, 0, 0, 0, 1}) {
     per_sample_kernel<<<(batch + kSampleWarps - 1) / kSampleWarps, 32 * kSampleWarps, 0, st>>>(r->tree, r->gmin ? r->gmin : r->mn, r->cap, batch, beta, seed, r->word_pos + 1,
                                                                                                r->counters + 1, tree_idx, data_idx, isw, prio, isw32, ft);
 }
 
 // ---- sampling + gather as the head of a captured training step (fb_qnet_train_step_sampled) -------------------------
+// n_step == 0: the 1-step transitions; n_step >= 1: everything is decoded at t_eff = t - n + 1 (see the top of this file)
+static int horizon(const fb_step_sampling &p) { return p.n_step > 0 ? p.n_step : 1; }
+static long long decode_time(const fb_step_sampling &p) { return p.t - horizon(p) + 1; }
+int replay_frames_per_sample(const fb_step_sampling &p) { return frames_per_sample(horizon(p)); }
 static bool sampling_population(const fb_step_sampling &p, uint32_t *n_out) {
-    long long k_lo = p.t - p.replay->C + 1; if (k_lo < 1) k_lo = 1;
-    long long n = (p.t - k_lo + 1) * p.replay->N;
+    const long long t = decode_time(p);
+    long long k_lo = t - p.replay->C + 1; if (k_lo < 1) k_lo = 1;
+    long long n = (t - k_lo + 1) * p.replay->N;
     *n_out = (uint32_t)n;
-    return p.t >= 1 && n >= p.batch;
+    return t >= 1 && n >= p.batch;
 }
-static GatherArgs sampling_gather_args(const fb_step_sampling &p) {
+static GatherArgs sampling_gather_args(const fb_step_sampling &p, double gamma) {
     const fb_replay *r = p.replay;
-    return GatherArgs{p.ring_dev, r->N, r->L, p.act_dev, p.rew_dev, p.term_dev, p.t, r->C, p.prioritized ? 1 : 0, p.idx_out_dev, p.batch,
-                      p.frames_out_dev, p.act_out_dev, p.rew_out_dev, p.term_out_dev, p.env_out_dev, p.k_out_dev};
+    const bool nstep = p.n_step > 0;
+    return GatherArgs{p.ring_dev, r->N, r->L, p.act_dev, p.rew_dev, p.term_dev, decode_time(p), r->C, p.prioritized ? 1 : 0, p.idx_out_dev, p.batch,
+                      p.frames_out_dev, p.act_out_dev, p.rew_out_dev, p.term_out_dev, p.env_out_dev, p.k_out_dev,
+                      horizon(p), gamma, nstep ? p.ret_out_dev : nullptr, nstep ? p.disc_out_dev : nullptr};
 }
 static FrameTabArgs sampling_frame_tab(const fb_step_sampling &p, bool want) {
     const fb_replay *r = p.replay;
-    return FrameTabArgs{want ? r->frame_tab : nullptr, p.t, r->C, r->L, p.prioritized ? 1 : 0};
+    return FrameTabArgs{want ? r->frame_tab : nullptr, decode_time(p), r->C, r->L, p.prioritized ? 1 : 0, horizon(p)};
 }
 // the sampler alone; with_tab: it also leaves the ring offsets of the drawn frames in replay_frame_tab()
 int replay_launch_sample(const fb_step_sampling &p, bool with_tab, cudaStream_t st) {
     FB_REQUIRE(p.replay && p.ring_dev && p.act_dev && p.rew_dev && p.term_dev && p.idx_out_dev && p.frames_out_dev && p.act_out_dev &&
                p.rew_out_dev && p.term_out_dev && p.batch > 0 && p.batch <= 512, "step sampling: bad argument");
     fb_replay *r = p.replay;
+    if (p.n_step != 0) {
+        FB_REQUIRE(p.n_step >= 1 && p.n_step <= 16, "step sampling: n_step must be 0 (1-step) or 1..16");
+        FB_REQUIRE(p.ret_out_dev && p.disc_out_dev, "step sampling: n-step returns need ret_out_dev and disc_out_dev");
+        FB_REQUIRE(r->L >= r->C + p.n_step + 3, "step sampling: n-step returns need ring_len >= capacity_per_env + n_step + 3");
+    }
     if (p.prioritized) {
         FB_REQUIRE(r->tree && p.tree_idx_out_dev && p.is_weights_out_dev && p.is_weights_f32_out_dev && (p.per_mode == 0 || p.per_mode == 1) &&
                    p.batch <= r->scratch_n, "step sampling: prioritized replay arguments");
@@ -577,14 +628,14 @@ int replay_launch_sample(const fb_step_sampling &p, bool with_tab, cudaStream_t 
     FB_CUDA_OK(cudaGetLastError());
     return FB_OK;
 }
-int replay_launch_gather(const fb_step_sampling &p, cudaStream_t st) {
-    gather_kernel<<<dim3(p.batch, 5), 128, 0, st>>>(sampling_gather_args(p));
+int replay_launch_gather(const fb_step_sampling &p, double gamma, cudaStream_t st) {
+    gather_kernel<<<dim3(p.batch, replay_frames_per_sample(p)), 128, 0, st>>>(sampling_gather_args(p, gamma));
     FB_CUDA_OK(cudaGetLastError());
     return FB_OK;
 }
-int replay_launch_sample_gather(const fb_step_sampling &p, cudaStream_t st) {
+int replay_launch_sample_gather(const fb_step_sampling &p, double gamma, cudaStream_t st) {
     int rc = replay_launch_sample(p, false, st);
-    return rc ? rc : replay_launch_gather(p, st);
+    return rc ? rc : replay_launch_gather(p, gamma, st);
 }
 const long long *replay_frame_tab(const fb_replay *r) { return r->frame_tab; }
 int replay_launch_per_update(const fb_step_sampling &p, const float *abs_err_dev, cudaStream_t st) {
@@ -596,7 +647,8 @@ int replay_launch_per_update(const fb_step_sampling &p, const float *abs_err_dev
 }
 bool replay_is_sampler(const void *func) { return func == (const void *)sample_uniform_kernel || func == (const void *)per_sample_kernel; }
 bool replay_is_gather(const void *func) { return func == (const void *)gather_kernel; }
-int replay_patch_nodes(cudaGraphExec_t exec, cudaGraphNode_t sampler, cudaGraphNode_t gather, const fb_step_sampling &p, bool with_tab) {
+int replay_patch_nodes(cudaGraphExec_t exec, cudaGraphNode_t sampler, cudaGraphNode_t gather, const fb_step_sampling &p, double gamma,
+                       bool with_tab) {
     fb_replay *r = p.replay;
     cudaKernelNodeParams kp{};
     int batch = p.batch; uint64_t seed = p.seed; int32_t *idx = p.idx_out_dev;
@@ -616,9 +668,9 @@ int replay_patch_nodes(cudaGraphExec_t exec, cudaGraphNode_t sampler, cudaGraphN
         kp.func = (void *)sample_uniform_kernel; kp.gridDim = dim3(1); kp.blockDim = dim3(kSampThreads); kp.kernelParams = sargs;
         FB_CUDA_OK(cudaGraphExecKernelNodeSetParams(exec, sampler, &kp));
     }
-    GatherArgs g = sampling_gather_args(p);
+    GatherArgs g = sampling_gather_args(p, gamma);            // (t_eff, and with it the n-step window, moves with t)
     void *gargs[] = {&g};
-    kp.func = (void *)gather_kernel; kp.gridDim = dim3(p.batch, 5); kp.blockDim = dim3(128); kp.kernelParams = gargs;
+    kp.func = (void *)gather_kernel; kp.gridDim = dim3(p.batch, replay_frames_per_sample(p)); kp.blockDim = dim3(128); kp.kernelParams = gargs;
     FB_CUDA_OK(cudaGraphExecKernelNodeSetParams(exec, gather, &kp));
     return FB_OK;
 }

@@ -70,9 +70,10 @@ def main(argv=None):
     parser.add_argument("--replay-per-env", type=int, default=None)
     parser.add_argument("--report-every", type=int, default=1000)
     parser.add_argument("--seed", type=int, default=0)
+    parser.add_argument("--n-step", type=int, default=1, help="horizon of the TD target (1: the reference's one-step target)")
     a = parser.parse_args(argv)
     brain, _, stats = playFlappyBird(a.model, a.envs, a.steps, seed=a.seed, replay_memory_per_env=a.replay_per_env, report_every=a.report_every,
-                                     batch_size=a.batch, root_dir=a.root_dir, record=a.root_dir is not None)
+                                     batch_size=a.batch, root_dir=a.root_dir, record=a.root_dir is not None, n_step=a.n_step)
     if a.root_dir is not None:
         brain.save()
     if fdist.dist.is_initialized() and fdist.dist.get_rank() != 0:

@@ -21,6 +21,15 @@ _OFF_N = (C.c_int32 * 4)(6400, 12800, 19200, 25600)
 PRECISIONS = {"fp32": 0, "bf16": 1, "fp16": 2}
 
 
+def _sampled_offsets(frames: torch.Tensor):
+    """channel offsets of s and s' in a minibatch row u8[F][80][80] drawn by the replay: s = frames 0..3, s' = frames F-4..F-1
+    (F = 5: the 1-step row, s' = 1..4; F = 4 + min(n, 4) for n-step returns)"""
+    F = frames.shape[1]
+    if F == 5:
+        return _OFF_S, _OFF_N
+    return _OFF_S, (C.c_int32 * 4)(*[(F - 4 + c) * 6400 for c in range(4)])
+
+
 def truncated_normal_(t: torch.Tensor, std: float, generator=None):
     """tf.truncated_normal: N(0, std) resampled beyond two standard deviations (BrainDQN.py:122)."""
     torch.nn.init.trunc_normal_(t, mean=0.0, std=std, a=-2 * std, b=2 * std, generator=generator)
@@ -175,14 +184,17 @@ class QNetwork:
                       loss_sum: bool = False, global_batch: int | None = None, abs_err: torch.Tensor | None = None,
                       q_target: torch.Tensor | None = None, sampling=None) -> torch.Tensor:
         """frames u8[B][5][80][80]: s = frames 0..3, s' = frames 1..4 of each sample.  Fills self.grads, self.loss.
-        ``sampling``: as in train_step -- the minibatch is drawn by the first two kernels of the same graph."""
+        ``sampling``: as in train_step -- the minibatch is drawn by the first two kernels of the same graph (u8[B][F][80][80]
+        rows for n-step returns, whose targets then come from the replay's R / disc)."""
         B = frames.shape[0]
-        assert frames.shape[1:] == (5, 80, 80) and frames.dtype == torch.uint8 and frames.is_contiguous()
+        assert frames.shape[1:] == (5, 80, 80) or (sampling is not None and sampling.n_step > 0 and frames.shape[2:] == (80, 80))
+        assert frames.dtype == torch.uint8 and frames.is_contiguous()
         off_s, off_n = _OFF_S, _OFF_N
         ptr = lambda t: t.data_ptr() if t is not None else None
         self._sync_versions()
         if sampling is not None:
             assert frames.data_ptr() == sampling.frames_out_dev and B == sampling.batch and (is_weights is None) == (not sampling.prioritized)
+            off_s, off_n = _sampled_offsets(frames)
             _lib.check(self._L.fb_qnet_train_step_sampled(
                 self._h, C.addressof(sampling), VARIANTS[variant], self.params.data_ptr(), self.target.data_ptr(), off_s, off_n,
                 global_batch or B, float(gamma), int(loss_sum), self.grads.data_ptr(), self.loss.data_ptr(), ptr(abs_err), ptr(q_target),
@@ -205,12 +217,13 @@ class QNetwork:
 
         ``sampling`` (``ReplayMemory.step_sampling(batch)[0]``): the minibatch is drawn and gathered by the step's first two
         kernels -- ``random.sample`` and the list comprehensions of BrainDQN.py:197-201 ride in the same graph; ``frames`` /
-        ``actions`` / ``rewards`` / ``terminals`` must then be the replay's own minibatch buffers."""
+        ``actions`` / ``rewards`` / ``terminals`` must then be the replay's own minibatch buffers.  A memory with ``n_step`` > 1
+        hands out u8[B][F][80][80] rows and the step forms the n-step target from its R / disc."""
         in_step = self.exchange is None or self.exchange_in_step
         if sampling is not None and in_step:
             assert frames.data_ptr() == sampling.frames_out_dev and frames.shape[0] == sampling.batch
             assert (is_weights is None) == (not sampling.prioritized)
-            off_s, off_n = _OFF_S, _OFF_N
+            off_s, off_n = _sampled_offsets(frames)
             ptr = lambda t: t.data_ptr() if t is not None else None
             self._sync_versions()
             _lib.check(self._L.fb_qnet_train_step_sampled(
@@ -223,6 +236,7 @@ class QNetwork:
             return self.loss
         if sampling is not None:                 # not fusable here: draw the minibatch with its own two launches
             assert not sampling.prioritized, "with a peer exchange call PrioritizedMemory.sample / batch_update yourself"
+            assert sampling.n_step == 0, "n-step minibatches are drawn inside the training step only"
             _lib.check(self._L.fb_replay_sample_uniform(sampling.replay, sampling.t, sampling.batch, sampling.setsize, sampling.seed,
                                                         sampling.idx_out_dev, self._stream()), "fb_replay_sample_uniform")
             _lib.check(self._L.fb_replay_gather(sampling.replay, sampling.ring_dev, sampling.act_dev, sampling.rew_dev, sampling.term_dev,

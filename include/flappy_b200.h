@@ -345,6 +345,17 @@ typedef struct fb_step_sampling {
     int32_t *tree_idx_out_dev;
     double *is_weights_out_dev, *prio_out_dev;
     float *is_weights_f32_out_dev;
+    /* n-step returns.  n_step = 0 (a zero-initialised tail): the 1-step transitions above, unchanged.  1 <= n_step <= 16:
+     * transition k is (s_{k-1}, a_k, R_k, s_{k+n-1}, disc_k) with m the first i in 1..n whose term_{k+i-1} is set (else n),
+     * R_k = sum_{i<m} gamma^i r_{k+i} (float64, accumulated forward: R += g r; g *= gamma) and disc_k = 0 after a terminal,
+     * else gamma^n (that same product); the TD target is y = disc == 0 ? R : R + disc X, gamma being the step's `gamma`.
+     * A transition is drawn once its horizon is complete: the population / SumTree is that of t_eff = t - n_step + 1 (so
+     * the caller stores transition t - n + 1 into a prioritized memory at time t).  The frame ring must hold
+     * ring_len >= capacity_per_env + n_step + 3 frames (FB_ERR_INVALID otherwise).  frames_out_dev is then
+     * u8[batch][F][80][80], F = 4 + min(n, 4): s = frames 0..3, s' = frames min(n,4)..min(n,4)+3 (chan_off 0.. and
+     * min(n,4)*6400..; sample_stride F*6400); ret_out_dev / disc_out_dev f64[batch] receive R_k and disc_k (required). */
+    int n_step;
+    double *ret_out_dev, *disc_out_dev;
 } fb_step_sampling;
 /* fb_qnet_train_step with the minibatch drawn first (uniform or prioritized replay).  m_dev == v_dev == NULL: gradients only
  * (fb_qnet_loss_backward with the minibatch drawn first; the caller applies Adam, e.g. through fb_dist_adam).  FB_ERR_INVALID with "Sample larger than population
