@@ -132,6 +132,11 @@ _SIGNATURES = {
                                     _f32p, _f32p, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, _vp], C.c_int),
     "fb_qnet_adam": ([_vp, _f32p, _f32p, _f32p, _f32p, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, _vp], C.c_int),
     "fb_qnet_sync_target": ([_vp, _f32p, _f32p, _vp], C.c_int),
+    "fb_noisy_layout": ([_vp, _i32p], C.c_int),
+    "fb_noisy_draw": ([_vp, C.c_uint64, C.c_int, C.c_uint64, _f32p, _vp], C.c_int),
+    "fb_noisy_weights": ([_vp, _f32p, _f32p, _f32p, _f32p, _vp], C.c_int),
+    "fb_qnet_noisy_adam": ([_vp, _f32p, _f32p, _f32p, _f32p, _f32p, _f32p, _f32p, _f32p, C.c_float, C.c_float, C.c_float, C.c_float,
+                            C.c_float, _vp], C.c_int),
     "fb_debug_step_sampling_layout": ([_i32p, C.c_int], C.c_int),
     "fb_dist_debug_stamps": ([_vp, _vp], C.c_int),
     "fb_dist_create": ([C.c_int, C.c_int, C.c_longlong, C.POINTER(C.c_void_p)], C.c_int),

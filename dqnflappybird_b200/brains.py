@@ -23,6 +23,10 @@ BrainPrioritizedReplyDQN.py:243-251); the default runs the intended algorithm (m
 first terminal inside the window (replay.py, csrc/fb_replay.cu).  It needs the minibatch drawn inside the update
 (``fuse_sampling``), and for prioritized replay on several ranks the in-step gradient exchange.
 
+``noisy=True`` explores with NoisyNet layers (Fortunato et al. 2018): fc1 and the head run on mu + sigma * eps with factorised
+Gaussian noise drawn afresh for every update and every getAction (qnet.py, csrc/fb_noisy.cu).  The epsilon-greedy schedule is
+left as it is; pass ``initial_epsilon=0`` to explore by the noise alone.  On several ranks it takes the NCCL all-reduce path.
+
 All math runs in libflappy_b200.so; with torch.distributed initialised every rank trains on its own env /
 replay shard and the replicated learner sums the ranks' gradients inside the update's CUDA graph over NVLink
 peer memory (fb_dist.cu), or with an NCCL all-reduce before the Adam step when ``peer_exchange=False``.
@@ -67,7 +71,7 @@ class BrainDQN:
                  hidden: int = 512, lr: float = 1e-6, seed: int = 0, first_env_id: int = 0, updates_per_step: int = 1,
                  reference_quirks: bool = False, copy_target_at_init: bool = False, record: bool = False, max_act_batch: int = 4096,
                  precision: str = "fp16", peer_exchange: bool | None = None, root_dir: str | None = None, save_every: int = SAVE_EVERY,
-                 log_capacity: int = 1 << 20, n_step: int = 1):
+                 log_capacity: int = 1 << 20, n_step: int = 1, noisy: bool = False, noisy_sigma0: float = 0.5):
         if actionNum != 2:
             raise ValueError("the Flappy Bird hot path has two actions (FlappyBirdDQN.py:38)")
         self.actionNum, self.gameName = actionNum, gameName
@@ -82,6 +86,7 @@ class BrainDQN:
         self.fuse_sampling = True                  # uniform replay on one GPU: draw the minibatch inside the update's graph
         self.seed, self.first_env_id = seed, first_env_id
         self.n_step = int(n_step)
+        self.noisy = bool(noisy)
         # distributed: one process per GPU, replicated learner (SURVEY 8e)
         self.world = torch.distributed.get_world_size() if torch.distributed.is_available() and torch.distributed.is_initialized() else 1
         from .dist import local_batch as _local_batch
@@ -103,14 +108,18 @@ class BrainDQN:
         # init Q network (BrainDQN.py:60)
         dueling = self.dueling and not (reference_quirks and type(self).__name__ == "BrainDuelingDQN")
         self.net = QNetwork(self.device, hidden=hidden, dueling=dueling, max_batch=max(self.local_batch, min(N, max_act_batch)),
-                            seed=seed, lr=lr, copy_target_at_init=copy_target_at_init, precision=precision)
+                            seed=seed, lr=lr, copy_target_at_init=copy_target_at_init, precision=precision, noisy=self.noisy,
+                            sigma0=noisy_sigma0)
         if self.prioritized and reference_quirks:
             # what the shipped graph really minimises: ISWeights [B,1] x square(...) [B] broadcasts to [B,B], so every sample is
             # weighted by mean(ISWeights) (BrainPrioritizedReplyDQN.py:243-251); the default is the intended per-sample weight
             self.net.set_per_broadcast(True)
         # one process per GPU under NCCL: sum the gradients from NVLink peer memory inside the Adam kernel (fb_dist.cu)
+        if self.noisy and peer_exchange:
+            raise ValueError("noisy=True trains through loss_backward + all_reduce + the noisy Adam; the in-step peer exchange "
+                             "applies plain Adam and is not available with it")
         if peer_exchange is None:
-            peer_exchange = self.world > 1 and torch.distributed.get_backend() == "nccl"
+            peer_exchange = not self.noisy and self.world > 1 and torch.distributed.get_backend() == "nccl"
         if peer_exchange and self.world > 1:
             self.net.enable_peer_exchange()
         if self.n_step > 1 and self.prioritized and self.world > 1 and not self.net.exchange_in_step:

@@ -63,6 +63,16 @@ __device__ __forceinline__ float td_target(float x, float rf, uint8_t terminal, 
     return (float)(terminal ? r : r + gamma * (double)x);
 }
 
+// One tf.train.AdamOptimizer element (TF 1.12 ApplyAdam functor, as adam_kernel in fb_qnet.cu), alpha = lr sqrt(1 - beta2^t) /
+// (1 - beta1^t): m += (g - m) (1 - beta1); v += (g^2 - v) (1 - beta2); var -= (m alpha) / (sqrt(v) + eps).  Returns the new var.
+__device__ __forceinline__ float adam_math(float g, float pi, float &mi, float &vi, float alpha, float beta1, float beta2, float eps,
+                                           float grad_scale) {
+    float gi = g * grad_scale;
+    mi += (gi - mi) * (1.f - beta1);
+    vi += (gi * gi - vi) * (1.f - beta2);
+    return pi - (mi * alpha) / (sqrtf(vi) + eps);
+}
+
 // ---- handle shared by the strict-fp32 path (fb_qnet.cu) and the tcgen05 path (fb_qnet_tc.cu) ------------
 struct fb_dist;                 // multi-GPU gradient exchange (fb_dist.cu)
 struct TcState;                 // bf16 workspace, packed weights and TMA plans (fb_qnet_tc.cu)

@@ -446,15 +446,8 @@ __global__ void pack_weights_kernel(const float *params, QnetLayout L, PackedWei
     for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < L.bf1; i += gridDim.x * blockDim.x) scatter_packed(i, params[i], L, pw, fwd_only);
 }
 
-// tf.train.AdamOptimizer step (TF 1.12 ApplyAdam, as adam_kernel in fb_qnet.cu) that also refreshes the bf16 operand
+// tf.train.AdamOptimizer step (TF 1.12 ApplyAdam, adam_math in fb_qnet.cuh) that also refreshes the bf16 operand
 // copies of the parameters it has just written, so the next training step starts without a pack kernel
-__device__ __forceinline__ float adam_math(float g, float pi, float &mi, float &vi, float alpha, float beta1, float beta2, float eps,
-                                           float grad_scale) {
-    float gi = g * grad_scale;
-    mi += (gi - mi) * (1.f - beta1);
-    vi += (gi * gi - vi) * (1.f - beta2);
-    return pi - (mi * alpha) / (sqrtf(vi) + eps);
-}
 __device__ __forceinline__ void adam_one(int i, float g, float *__restrict__ p, float *__restrict__ m, float *__restrict__ v, float alpha,
                                          float beta1, float beta2, float eps, float grad_scale, const QnetLayout &L, const PackedWeights &pw) {
     float mi = m[i], vi = v[i];

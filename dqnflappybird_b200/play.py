@@ -71,9 +71,15 @@ def main(argv=None):
     parser.add_argument("--report-every", type=int, default=1000)
     parser.add_argument("--seed", type=int, default=0)
     parser.add_argument("--n-step", type=int, default=1, help="horizon of the TD target (1: the reference's one-step target)")
+    parser.add_argument("--noisy", action="store_true", help="NoisyNet exploration: factorised-Gaussian noisy fc1 and head layers")
+    parser.add_argument("--noisy-sigma0", type=float, default=0.5, help="initial noise scale: sigma = sigma0 / sqrt(fan-in)")
+    parser.add_argument("--initial-epsilon", type=float, default=None,
+                        help="start of the epsilon-greedy schedule (default: the reference's 0.03; 0 explores by noise alone)")
     a = parser.parse_args(argv)
     brain, _, stats = playFlappyBird(a.model, a.envs, a.steps, seed=a.seed, replay_memory_per_env=a.replay_per_env, report_every=a.report_every,
-                                     batch_size=a.batch, root_dir=a.root_dir, record=a.root_dir is not None, n_step=a.n_step)
+                                     batch_size=a.batch, root_dir=a.root_dir, record=a.root_dir is not None, n_step=a.n_step,
+                                     noisy=a.noisy, noisy_sigma0=a.noisy_sigma0,
+                                     **({} if a.initial_epsilon is None else {"initial_epsilon": a.initial_epsilon}))
     if a.root_dir is not None:
         brain.save()
     if fdist.dist.is_initialized() and fdist.dist.get_rank() != 0:

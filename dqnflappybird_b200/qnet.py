@@ -64,7 +64,11 @@ class FrameBatch:
 class QNetwork:
     def __init__(self, device="cuda:0", hidden: int = 512, dueling: bool = False, max_batch: int = 256, seed: int = 0,
                  lr: float = 1e-6, beta1: float = 0.9, beta2: float = 0.999, adam_eps: float = 1e-8,
-                 copy_target_at_init: bool = False, precision: str = "fp16"):
+                 copy_target_at_init: bool = False, precision: str = "fp16", noisy: bool = False, sigma0: float = 0.5):
+        """``noisy``: NoisyNet (Fortunato et al. 2018) with factorised Gaussian noise on fc1 and the head (csrc/fb_noisy.cu).
+        ``params`` / ``target`` are then mu (initialised exactly as without noise), ``sigma`` / ``target_sigma`` start at
+        sigma0 / sqrt(fan-in) on the noisy layers and 0 elsewhere, and training and acting run on the effective weights
+        mu + sigma * eps of a fresh draw; the noise stream is (``seed``, draw id), the same on every rank."""
         if not torch.cuda.is_available():
             raise _lib.FlappyError("QNetwork needs a CUDA device (B200); there is no CPU path")
         self.device = torch.device(device)
@@ -100,6 +104,64 @@ class QNetwork:
         self.adam_steps = 0
         self.exchange = None                    # dist.PeerGradExchange once enable_peer_exchange() was called
         self.exchange_in_step = False
+        self.noisy = bool(noisy)
+        if self.noisy:
+            self._init_noise(seed, float(sigma0))
+
+    # ---------------------------------------------------------------- noisy networks
+    def _init_noise(self, seed: int, sigma0: float):
+        lay = (C.c_int32 * 20)()
+        _lib.check(self._L.fb_noisy_layout(self._h, lay), "fb_noisy_layout")
+        # per noisy layer: parameter offsets of weight [p][q] and bias [q], and where f(eps_in) [p] / f(eps_out) [q] sit in a draw
+        self.noise_layout = [dict(w=lay[2 + 6 * k], b=lay[3 + 6 * k], p=lay[4 + 6 * k], q=lay[5 + 6 * k], f_in=lay[6 + 6 * k],
+                                  f_out=lay[7 + 6 * k]) for k in range(int(lay[0]))]
+        self.n_factors = int(lay[1])
+        self.noise_seed, self.sigma0 = int(seed), sigma0
+        z = lambda n: torch.zeros(n, dtype=torch.float32, device=self.device)
+        self.sigma, self.target_sigma, self.sigma_m, self.sigma_v = z(self.n_params), z(self.n_params), z(self.n_params), z(self.n_params)
+        # effective weights of the update's online / target draw and of the last acting draw, and the factor vectors they came from
+        self.weff, self.weff_target, self.weff_act = z(self.n_params), z(self.n_params), z(self.n_params)
+        self.noise_online, self.noise_target, self.noise_act = z(self.n_factors), z(self.n_factors), z(self.n_factors)
+        sig = torch.zeros(self.n_params, dtype=torch.float32)
+        for ly in self.noise_layout:                  # Fortunato's factorised rule: sigma0 / sqrt(fan-in), weights and bias alike
+            s0 = np.float32(sigma0 / np.sqrt(ly["p"]))
+            sig[ly["w"]:ly["w"] + ly["p"] * ly["q"]] = float(s0)
+            sig[ly["b"]:ly["b"] + ly["q"]] = float(s0)
+        self.sigma.copy_(sig); self.target_sigma.copy_(sig)
+        self.update_draws = 0                         # draw counters: update u (online and target role), acting call a
+        self.act_draws = 0
+
+    def draw_noise(self, role: str, counter: int, out: torch.Tensor | None = None) -> torch.Tensor:
+        """the factor vector of draw (role, counter), role in online / target / act (include/flappy_b200.h fb_noisy_draw)"""
+        out = out if out is not None else torch.empty(self.n_factors, dtype=torch.float32, device=self.device)
+        _lib.check(self._L.fb_noisy_draw(self._h, self.noise_seed, {"online": 0, "target": 1, "act": 2}[role], int(counter),
+                                         out.data_ptr(), self._stream()), "fb_noisy_draw")
+        return out
+
+    def noisy_weights(self, mu: torch.Tensor, sigma: torch.Tensor, factors: torch.Tensor, out: torch.Tensor) -> torch.Tensor:
+        """out = mu + sigma * eps on the noisy layers, mu elsewhere (fb_noisy_weights)"""
+        _lib.check(self._L.fb_noisy_weights(self._h, mu.data_ptr(), sigma.data_ptr(), factors.data_ptr(), out.data_ptr(), self._stream()),
+                   "fb_noisy_weights")
+        return out
+
+    def _act_weights(self, target: bool = False) -> torch.Tensor:
+        """effective weights of the next acting draw (consumes it)"""
+        self.draw_noise("act", self.act_draws, self.noise_act)
+        self.act_draws += 1
+        mu, sigma = (self.target, self.target_sigma) if target else (self.params, self.sigma)
+        return self.noisy_weights(mu, sigma, self.noise_act, self.weff_act)
+
+    def _train_weights(self, variant: str):
+        """(online, target) vectors the update runs on: the parameters, or for a noisy net the effective weights of update u's
+        online draw and -- for the Nature and Double targets -- its target draw (vanilla and Double evaluate Q(s') with the
+        online draw, no extra draw)"""
+        if not self.noisy:
+            return self.params, self.target
+        u = self.update_draws
+        self.noisy_weights(self.params, self.sigma, self.draw_noise("online", u, self.noise_online), self.weff)
+        if VARIANTS[variant] != 0:
+            self.noisy_weights(self.target, self.target_sigma, self.draw_noise("target", u, self.noise_target), self.weff_target)
+        return self.weff, self.weff_target
 
     def set_per_broadcast(self, on: bool):
         """PER loss exactly as the reference's graph evaluates it (BrainPrioritizedReplyDQN.py:243-251): the [B,1] ISWeights
@@ -110,7 +172,10 @@ class QNetwork:
         """Multi-GPU: keep the gradient vector in an NVLink-mapped exchange buffer and let adam_step() sum every rank's
         gradients from peer memory inside the Adam kernel (csrc/fb_dist.cu) instead of a separate all-reduce."""
         from .dist import PeerGradExchange
-        self.exchange = exchange if exchange is not None else PeerGradExchange(self.n_params, self.device)
+        if self.noisy:
+            raise ValueError("a noisy net takes the all-reduce path (loss_backward, all_reduce(grads), adam_step): the peer exchange "
+                             "applies plain Adam inside its own kernels")
+        self.exchange =exchange if exchange is not None else PeerGradExchange(self.n_params, self.device)
         self.grads = self.exchange.grads
         # tensor-core path: the exchange rides INSIDE the training step's graph (fb_dist.cu buckets) instead of after it
         self.exchange_in_step = self.precision != "fp32" and self.exchange.world > 1 and not getattr(self.exchange, "no_wait", False)
@@ -160,20 +225,25 @@ class QNetwork:
             self._seen_versions = v
 
     # ---------------------------------------------------------------- forward / act
-    def forward(self, fb: FrameBatch, target: bool = False, out: torch.Tensor | None = None) -> torch.Tensor:
-        """QValue.eval(feed_dict={stateInput: ...}) (BrainDQN.py:100): f32[B][2]."""
+    def forward(self, fb: FrameBatch, target: bool = False, out: torch.Tensor | None = None, noise: bool | None = None) -> torch.Tensor:
+        """QValue.eval(feed_dict={stateInput: ...}) (BrainDQN.py:100): f32[B][2].  A noisy net evaluates the effective weights
+        of the next acting draw (noise=False: mu)."""
         q = out if out is not None else torch.empty((fb.batch, 2), dtype=torch.float32, device=self.device)
         p = self.target if target else self.params
         self._sync_versions()
+        if self.noisy and noise is not False:
+            p = self._act_weights(target)
         _lib.check(self._L.fb_qnet_forward(self._h, p.data_ptr(), fb.ptr, fb.sample_stride, fb.chan_off, fb.batch,
                                            q.data_ptr(), self._stream()), "fb_qnet_forward")
         return q
 
     def act(self, fb: FrameBatch, epsilon: float, seed: int, first_env_id: int, rng_pos: torch.Tensor,
-            actions_out: torch.Tensor, q_out: torch.Tensor):
-        """getAction (BrainDQN.py:99-108) for every env of the batch."""
+            actions_out: torch.Tensor, q_out: torch.Tensor, noise: bool | None = None):
+        """getAction (BrainDQN.py:99-108) for every env of the batch.  A noisy net acts on the effective weights of the next
+        acting draw; the epsilon-greedy draws are unchanged.  noise=False acts on mu (evaluation)."""
         self._sync_versions()
-        _lib.check(self._L.fb_qnet_act(self._h, self.params.data_ptr(), fb.ptr, fb.sample_stride, fb.chan_off, fb.batch,
+        p = self._act_weights() if self.noisy and noise is not False else self.params
+        _lib.check(self._L.fb_qnet_act(self._h, p.data_ptr(), fb.ptr, fb.sample_stride, fb.chan_off, fb.batch,
                                        float(epsilon), seed, first_env_id, rng_pos.data_ptr(), q_out.data_ptr(),
                                        actions_out.data_ptr(), self._stream()), "fb_qnet_act")
         return actions_out
@@ -192,16 +262,17 @@ class QNetwork:
         off_s, off_n = _OFF_S, _OFF_N
         ptr = lambda t: t.data_ptr() if t is not None else None
         self._sync_versions()
+        p, tg = self._train_weights(variant)        # mu, or the effective weights of update u's draws
         if sampling is not None:
             assert frames.data_ptr() == sampling.frames_out_dev and B == sampling.batch and (is_weights is None) == (not sampling.prioritized)
             off_s, off_n = _sampled_offsets(frames)
             _lib.check(self._L.fb_qnet_train_step_sampled(
-                self._h, C.addressof(sampling), VARIANTS[variant], self.params.data_ptr(), self.target.data_ptr(), off_s, off_n,
+                self._h, C.addressof(sampling), VARIANTS[variant], p.data_ptr(), tg.data_ptr(), off_s, off_n,
                 global_batch or B, float(gamma), int(loss_sum), self.grads.data_ptr(), self.loss.data_ptr(), ptr(abs_err), ptr(q_target),
                 None, None, 0.0, 0.0, 0.0, 0.0, 1.0, 0.0, 0.0, self._stream()), "fb_qnet_train_step_sampled")
             return self.loss
         _lib.check(self._L.fb_qnet_loss_backward(
-            self._h, VARIANTS[variant], self.params.data_ptr(), self.target.data_ptr(), frames.data_ptr(), 5 * 6400,
+            self._h, VARIANTS[variant], p.data_ptr(), tg.data_ptr(), frames.data_ptr(), 5 * 6400,
             off_s, off_n, actions.data_ptr(), rewards.data_ptr(), terminals.data_ptr(), ptr(is_weights), B,
             global_batch or B, float(gamma), int(loss_sum), self.grads.data_ptr(), self.loss.data_ptr(), ptr(abs_err),
             ptr(q_target), self._stream()), "fb_qnet_loss_backward")
@@ -218,7 +289,14 @@ class QNetwork:
         ``sampling`` (``ReplayMemory.step_sampling(batch)[0]``): the minibatch is drawn and gathered by the step's first two
         kernels -- ``random.sample`` and the list comprehensions of BrainDQN.py:197-201 ride in the same graph; ``frames`` /
         ``actions`` / ``rewards`` / ``terminals`` must then be the replay's own minibatch buffers.  A memory with ``n_step`` > 1
-        hands out u8[B][F][80][80] rows and the step forms the n-step target from its R / disc."""
+        hands out u8[B][F][80][80] rows and the step forms the n-step target from its R / disc.
+
+        A noisy net: the gradient-only step on the effective weights of update u's draws, then the Adam over (mu, sigma)."""
+        if self.noisy:
+            self.loss_backward(variant, frames, actions, rewards, terminals, is_weights, gamma, loss_sum, global_batch, abs_err, q_target,
+                               sampling=sampling)
+            self.adam_step(grad_scale)
+            return self.loss
         in_step = self.exchange is None or self.exchange_in_step
         if sampling is not None and in_step:
             assert frames.data_ptr() == sampling.frames_out_dev and frames.shape[0] == sampling.batch
@@ -278,7 +356,14 @@ class QNetwork:
         """One tf.train.AdamOptimizer step on self.params with self.grads (TF-1 ApplyAdam)."""
         one = np.float32(1)
         alpha = np.float32(self.lr * np.sqrt(one - self.beta2_power) / (one - self.beta1_power))
-        if self.exchange is not None:           # sum over ranks + Adam in one kernel; then switch to the other buffer
+        if self.noisy:                          # mu with g, sigma with g * eps of update u's online draw; then draw u + 1
+            _lib.check(self._L.fb_qnet_noisy_adam(self._h, self.params.data_ptr(), self.sigma.data_ptr(), self.grads.data_ptr(),
+                                                  self.noise_online.data_ptr(), self.adam_m.data_ptr(), self.adam_v.data_ptr(),
+                                                  self.sigma_m.data_ptr(), self.sigma_v.data_ptr(), float(alpha), float(self.beta1),
+                                                  float(self.beta2), float(self.adam_eps), float(grad_scale), self._stream()),
+                       "fb_qnet_noisy_adam")
+            self.update_draws += 1
+        elif self.exchange is not None:         # sum over ranks + Adam in one kernel; then switch to the other buffer
             self.exchange.adam(self, alpha, grad_scale, wait=self.exchange.world > 1 and not getattr(self.exchange, "no_wait", False))
             self.grads = self.exchange.grads
         else:
@@ -291,16 +376,31 @@ class QNetwork:
         """sess.run(target_replace_op) (BrainDQNNature.py:107-111,151-152)."""
         _lib.check(self._L.fb_qnet_sync_target(self._h, self.target.data_ptr(), self.params.data_ptr(), self._stream()),
                    "fb_qnet_sync_target")
+        if self.noisy:
+            _lib.check(self._L.fb_qnet_sync_target(self._h, self.target_sigma.data_ptr(), self.sigma.data_ptr(), self._stream()),
+                       "fb_qnet_sync_target")
 
     # ---------------------------------------------------------------- checkpoint (row N2, weights + Adam slots + powers)
     def state_dict(self):
         return {"params": self.params.clone(), "target": self.target.clone(), "adam_m": self.adam_m.clone(),
                 "adam_v": self.adam_v.clone(), "beta1_power": float(self.beta1_power), "beta2_power": float(self.beta2_power),
-                "adam_steps": self.adam_steps, "hidden": self.hidden, "dueling": self.dueling}
+                "adam_steps": self.adam_steps, "hidden": self.hidden, "dueling": self.dueling, **self._noise_state()}
+
+    _NOISE_TENSORS = ("sigma", "target_sigma", "sigma_m", "sigma_v")
+
+    def _noise_state(self):
+        if not self.noisy:
+            return {}
+        return {"noisy": True, **{k: getattr(self, k).clone() for k in self._NOISE_TENSORS}, "update_draws": self.update_draws,
+                "act_draws": self.act_draws, "noise_seed": self.noise_seed, "sigma0": self.sigma0}
 
     def load_state_dict(self, sd):
         assert sd["hidden"] == self.hidden and sd["dueling"] == self.dueling
-        for k in ("params", "target", "adam_m", "adam_v"):
+        assert bool(sd.get("noisy", False)) == self.noisy, "plain and noisy checkpoints are not interchangeable"
+        for k in ("params", "target", "adam_m", "adam_v") + (self._NOISE_TENSORS if self.noisy else ()):
             getattr(self, k).copy_(sd[k])
         self.beta1_power, self.beta2_power = np.float32(sd["beta1_power"]), np.float32(sd["beta2_power"])
         self.adam_steps = int(sd["adam_steps"])
+        if self.noisy:
+            self.update_draws, self.act_draws = int(sd["update_draws"]), int(sd["act_draws"])
+            self.noise_seed, self.sigma0 = int(sd["noise_seed"]), float(sd["sigma0"])

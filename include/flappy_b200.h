@@ -239,6 +239,30 @@ int fb_qnet_train_step(fb_qnet *net, int variant, float *params_dev, const float
 /* target_replace_op (BrainDQNNature.py:107-111) */
 int fb_qnet_sync_target(fb_qnet *net, float *target_dev, const float *params_dev, void *stream);
 
+/* ---- noisy networks (Fortunato et al. 2018, factorised Gaussian noise; csrc/fb_noisy.cu).  The noisy layers are fc1 and the
+ * head (plain: W_fc2 / b_fc2; dueling: the V head and the A head, each its own layer); the convolutions stay deterministic.  A
+ * noisy net keeps mu (the usual parameter vector) and sigma (same layout, zero outside the noisy layers).  A draw fills the
+ * factor vector: per noisy layer, in layer order, f(eps_in)[p] then f(eps_out)[q], f(x) = sgn(x) sqrt|x| in fp32.  The layer
+ * runs on W[i][j] = mu[i][j] + sigma[i][j] * (f(eps_in[i]) * f(eps_out[j])), b[j] = mu_b[j] + sigma_b[j] * f(eps_out[j]) (fp32,
+ * each operation rounded once): the effective-weight vector has the parameter layout, and every forward / training call above
+ * takes it in place of the parameters.  The gradient they return is dL/dmu; dL/dsigma = dL/dW * eps.
+ *
+ * fb_noisy_layout: out20_host = {number of noisy layers (2 or 3), factor-vector length, then per layer (3 slots, -1 / 0 where
+ * absent): weight offset, bias offset, fan-in p, fan-out q, offset of f(eps_in), offset of f(eps_out)}. */
+int fb_noisy_layout(const fb_qnet *net, int32_t *out20_host);
+/* One draw into factors_dev.  Normal k comes from words 2k, 2k+1 (w0, w1) of Philox stream (seed, purpose 5,
+ * (counter << 2) | role) by Box-Muller in float64: u1 = (w0 + 1) 2^-32, u2 = w1 2^-32, z = sqrt(-2 ln u1) cos(2 pi u2), rounded
+ * to fp32.  role 0: online net of update `counter`; 1: target net of that update; 2: acting call `counter`.  The stream does
+ * not depend on the rank, so replicas draw the same noise without communicating. */
+int fb_noisy_draw(fb_qnet *net, uint64_t seed, int role, uint64_t counter, float *factors_dev, void *stream);
+/* weff_dev = mu + sigma * eps on the noisy layers, mu elsewhere; the operand copies made from weff_dev are marked stale */
+int fb_noisy_weights(fb_qnet *net, const float *mu_dev, const float *sigma_dev, const float *factors_dev, float *weff_dev, void *stream);
+/* One TF-1 Adam step over (mu, sigma) with one alpha: mu with grads_dev (dL/dW at W_eff) over every parameter, sigma with
+ * grads_dev * eps (eps recomputed from the draw's factors) over the noisy layers; the rule and operation order of fb_qnet_adam */
+int fb_qnet_noisy_adam(fb_qnet *net, float *mu_dev, float *sigma_dev, const float *grads_dev, const float *factors_dev, float *m_dev,
+                       float *v_dev, float *sigma_m_dev, float *sigma_v_dev, float alpha, float beta1, float beta2, float eps,
+                       float grad_scale, void *stream);
+
 /* ---- multi-GPU gradient exchange fused with Adam (the one exchange step of the path: the sum of the per-shard
  * gradients of the replicated learner, SURVEY 8e).  One process per GPU; each rank's gradient vector lives in an exchange
  * buffer the peers map through CUDA IPC; fb_dist_adam publishes this rank's step, waits for every rank's, sums the
