@@ -76,7 +76,7 @@ _u8p, _i32p, _f32p, _vp = C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p
 
 
 class StepSampling(C.Structure):
-    """fb_step_sampling (include/flappy_b200.h): the minibatch draw that rides at the head of fb_qnet_train_step_sampled"""
+    """fb_step_sampling (include/flappy_b200.h): the minibatch draw that rides at the head of fb_qnet_step"""
     _fields_ = [("replay", C.c_void_p), ("ring_dev", C.c_void_p), ("act_dev", C.c_void_p), ("rew_dev", C.c_void_p), ("term_dev", C.c_void_p),
                 ("t", C.c_longlong), ("batch", C.c_int), ("setsize", C.c_uint32), ("seed", C.c_uint64), ("idx_out_dev", C.c_void_p),
                 ("frames_out_dev", C.c_void_p), ("act_out_dev", C.c_void_p), ("rew_out_dev", C.c_void_p), ("term_out_dev", C.c_void_p),
@@ -84,6 +84,18 @@ class StepSampling(C.Structure):
                 ("prioritized", C.c_int), ("per_mode", C.c_int), ("beta", C.c_double), ("tree_idx_out_dev", C.c_void_p),
                 ("is_weights_out_dev", C.c_void_p), ("prio_out_dev", C.c_void_p), ("is_weights_f32_out_dev", C.c_void_p),
                 ("n_step", C.c_int), ("ret_out_dev", C.c_void_p), ("disc_out_dev", C.c_void_p)]
+
+
+class QnetStepArgs(C.Structure):
+    """fb_qnet_step_args (include/flappy_b200.h): one training step of the Q-network"""
+    _fields_ = [("variant", C.c_int), ("loss_sum", C.c_int), ("batch", C.c_int), ("global_batch", C.c_int), ("gamma", C.c_double),
+                ("params_dev", C.c_void_p), ("target_params_dev", C.c_void_p), ("sampling", C.c_void_p),
+                ("frames_dev", C.c_void_p), ("sample_stride", C.c_longlong), ("chan_off_s", C.c_int32 * 4), ("chan_off_next", C.c_int32 * 4),
+                ("actions_dev", C.c_void_p), ("rewards_dev", C.c_void_p), ("terminals_dev", C.c_void_p), ("is_weights_dev", C.c_void_p),
+                ("grads_dev", C.c_void_p), ("loss_out_dev", C.c_void_p), ("abs_err_out_dev", C.c_void_p), ("q_target_out_dev", C.c_void_p),
+                ("m_dev", C.c_void_p), ("v_dev", C.c_void_p), ("lr", C.c_float), ("beta1", C.c_float), ("beta2", C.c_float),
+                ("eps", C.c_float), ("grad_scale", C.c_float), ("beta1_power", C.c_float), ("beta2_power", C.c_float)]
+
 
 _SIGNATURES = {
     "fb_last_error": ([], C.c_char_p),
@@ -123,20 +135,15 @@ _SIGNATURES = {
     "fb_qnet_layout": ([_vp, _i32p], C.c_int),
     "fb_qnet_forward": ([_vp, _f32p, _u8p, C.c_longlong, _i32p, C.c_int, _f32p, _vp], C.c_int),
     "fb_qnet_act": ([_vp, _f32p, _u8p, C.c_longlong, _i32p, C.c_int, C.c_double, C.c_uint64, C.c_uint64, _vp, _f32p, _u8p, _vp], C.c_int),
-    "fb_qnet_loss_backward": ([_vp, C.c_int, _f32p, _f32p, _u8p, C.c_longlong, _i32p, _i32p, _u8p, _f32p, _u8p, _f32p,
-                               C.c_int, C.c_int, C.c_double, C.c_int, _f32p, _f32p, _f32p, _f32p, _vp], C.c_int),
-    "fb_qnet_train_step": ([_vp, C.c_int, _f32p, _f32p, _u8p, C.c_longlong, _i32p, _i32p, _u8p, _f32p, _u8p, _f32p,
-                            C.c_int, C.c_int, C.c_double, C.c_int, _f32p, _f32p, _f32p, _f32p, _f32p, _f32p, C.c_float, C.c_float,
-                            C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, _vp], C.c_int),
-    "fb_qnet_train_step_sampled": ([_vp, _vp, C.c_int, _f32p, _f32p, _i32p, _i32p, C.c_int, C.c_double, C.c_int, _f32p, _f32p, _f32p, _f32p,
-                                    _f32p, _f32p, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, _vp], C.c_int),
     "fb_qnet_adam": ([_vp, _f32p, _f32p, _f32p, _f32p, C.c_float, C.c_float, C.c_float, C.c_float, C.c_float, _vp], C.c_int),
+    "fb_qnet_step": ([_vp, _vp, _vp], C.c_int),
     "fb_qnet_sync_target": ([_vp, _f32p, _f32p, _vp], C.c_int),
     "fb_noisy_layout": ([_vp, _i32p], C.c_int),
     "fb_noisy_draw": ([_vp, C.c_uint64, C.c_int, C.c_uint64, _f32p, _vp], C.c_int),
     "fb_noisy_weights": ([_vp, _f32p, _f32p, _f32p, _f32p, _vp], C.c_int),
     "fb_qnet_noisy_adam": ([_vp, _f32p, _f32p, _f32p, _f32p, _f32p, _f32p, _f32p, _f32p, C.c_float, C.c_float, C.c_float, C.c_float,
                             C.c_float, _vp], C.c_int),
+    "fb_debug_struct_layout": ([C.c_int, _i32p, C.c_int], C.c_int),
     "fb_debug_step_sampling_layout": ([_i32p, C.c_int], C.c_int),
     "fb_dist_debug_stamps": ([_vp, _vp], C.c_int),
     "fb_dist_create": ([C.c_int, C.c_int, C.c_longlong, C.POINTER(C.c_void_p)], C.c_int),

@@ -69,28 +69,35 @@ extern "C" int fb_debug_host_mixed(const int32_t *state16) {
     return (make_draw_list(s).np_mixed & 16) ? 1 : 0;
 }
 
-// layout of fb_step_sampling as this library was compiled: sizeof, then the byte offset of every field in declaration
-// order -- the CPU test-suite checks the ctypes mirror (dqnflappybird_b200/_lib.py StepSampling) against it
-extern "C" int fb_debug_step_sampling_layout(int32_t *out, int capacity) {
-    const int32_t v[] = {(int32_t)sizeof(fb_step_sampling),
-                         (int32_t)offsetof(fb_step_sampling, replay), (int32_t)offsetof(fb_step_sampling, ring_dev),
-                         (int32_t)offsetof(fb_step_sampling, act_dev), (int32_t)offsetof(fb_step_sampling, rew_dev),
-                         (int32_t)offsetof(fb_step_sampling, term_dev), (int32_t)offsetof(fb_step_sampling, t),
-                         (int32_t)offsetof(fb_step_sampling, batch), (int32_t)offsetof(fb_step_sampling, setsize),
-                         (int32_t)offsetof(fb_step_sampling, seed), (int32_t)offsetof(fb_step_sampling, idx_out_dev),
-                         (int32_t)offsetof(fb_step_sampling, frames_out_dev), (int32_t)offsetof(fb_step_sampling, act_out_dev),
-                         (int32_t)offsetof(fb_step_sampling, rew_out_dev), (int32_t)offsetof(fb_step_sampling, term_out_dev),
-                         (int32_t)offsetof(fb_step_sampling, env_out_dev), (int32_t)offsetof(fb_step_sampling, k_out_dev),
-                         (int32_t)offsetof(fb_step_sampling, prioritized), (int32_t)offsetof(fb_step_sampling, per_mode),
-                         (int32_t)offsetof(fb_step_sampling, beta), (int32_t)offsetof(fb_step_sampling, tree_idx_out_dev),
-                         (int32_t)offsetof(fb_step_sampling, is_weights_out_dev), (int32_t)offsetof(fb_step_sampling, prio_out_dev),
-                         (int32_t)offsetof(fb_step_sampling, is_weights_f32_out_dev), (int32_t)offsetof(fb_step_sampling, n_step),
-                         (int32_t)offsetof(fb_step_sampling, ret_out_dev), (int32_t)offsetof(fb_step_sampling, disc_out_dev)};
-    const int n = (int)(sizeof(v) / sizeof(v[0]));
-    FB_REQUIRE(out != nullptr && capacity >= n, "fb_debug_step_sampling_layout: buffer too small");
+// layout of the C ABI's structs as this library was compiled: sizeof, then the byte offset of every field in declaration order
+// -- the CPU test-suite checks the ctypes mirrors (dqnflappybird_b200/_lib.py StepSampling, QnetStepArgs) against it
+#define FB_OFF(S, f) (int32_t) offsetof(S, f)
+extern "C" int fb_debug_struct_layout(int which, int32_t *out, int capacity) {
+    typedef fb_step_sampling S;
+    typedef fb_qnet_step_args A;
+    const int32_t sampling[] = {(int32_t)sizeof(S), FB_OFF(S, replay), FB_OFF(S, ring_dev), FB_OFF(S, act_dev), FB_OFF(S, rew_dev),
+                                FB_OFF(S, term_dev), FB_OFF(S, t), FB_OFF(S, batch), FB_OFF(S, setsize), FB_OFF(S, seed),
+                                FB_OFF(S, idx_out_dev), FB_OFF(S, frames_out_dev), FB_OFF(S, act_out_dev), FB_OFF(S, rew_out_dev),
+                                FB_OFF(S, term_out_dev), FB_OFF(S, env_out_dev), FB_OFF(S, k_out_dev), FB_OFF(S, prioritized),
+                                FB_OFF(S, per_mode), FB_OFF(S, beta), FB_OFF(S, tree_idx_out_dev), FB_OFF(S, is_weights_out_dev),
+                                FB_OFF(S, prio_out_dev), FB_OFF(S, is_weights_f32_out_dev), FB_OFF(S, n_step), FB_OFF(S, ret_out_dev),
+                                FB_OFF(S, disc_out_dev)};
+    const int32_t step[] = {(int32_t)sizeof(A), FB_OFF(A, variant), FB_OFF(A, loss_sum), FB_OFF(A, batch), FB_OFF(A, global_batch),
+                            FB_OFF(A, gamma), FB_OFF(A, params_dev), FB_OFF(A, target_params_dev), FB_OFF(A, sampling),
+                            FB_OFF(A, frames_dev), FB_OFF(A, sample_stride), FB_OFF(A, chan_off_s), FB_OFF(A, chan_off_next),
+                            FB_OFF(A, actions_dev), FB_OFF(A, rewards_dev), FB_OFF(A, terminals_dev), FB_OFF(A, is_weights_dev),
+                            FB_OFF(A, grads_dev), FB_OFF(A, loss_out_dev), FB_OFF(A, abs_err_out_dev), FB_OFF(A, q_target_out_dev),
+                            FB_OFF(A, m_dev), FB_OFF(A, v_dev), FB_OFF(A, lr), FB_OFF(A, beta1), FB_OFF(A, beta2), FB_OFF(A, eps),
+                            FB_OFF(A, grad_scale), FB_OFF(A, beta1_power), FB_OFF(A, beta2_power)};
+    FB_REQUIRE(which == 0 || which == 1, "fb_debug_struct_layout: which must be 0 (fb_step_sampling) or 1 (fb_qnet_step_args)");
+    const int32_t *v = which == 0 ? sampling : step;
+    const int n = which == 0 ? (int)(sizeof(sampling) / sizeof(sampling[0])) : (int)(sizeof(step) / sizeof(step[0]));
+    FB_REQUIRE(out != nullptr && capacity >= n, "fb_debug_struct_layout: buffer too small");
     for (int i = 0; i < n; i++) out[i] = v[i];
     return n;
 }
+#undef FB_OFF
+extern "C" int fb_debug_step_sampling_layout(int32_t *out, int capacity) { return fb_debug_struct_layout(0, out, capacity); }
 
 // ---- write-pattern probe (tools/write_bw_probe.py): how fast can the device absorb the env kernel's output pattern? ---------
 // n_chunks chunks of 6,400 bytes, chunk k at dst + k * stride_bytes.  mode 0: one warp per chunk, 16-byte streaming stores

@@ -11,6 +11,7 @@
 // ordered reduction) and fold the bias gradient in as an extra all-ones row of the A operand.
 // The tensor-core path (fb_qnet_tc.cu) replaces the big GEMMs and is checked against this one.
 #include <math.h>
+#include <string.h>
 
 #include <new>
 
@@ -433,8 +434,8 @@ extern "C" int fb_qnet_set_precision(fb_qnet *n, int precision) {
 
 extern "C" int fb_qnet_get_precision(const fb_qnet *n) { return n ? n->precision : -1; }
 
-// Several GPUs, tensor-core path: fb_qnet_train_step / _sampled then sum every rank's gradients inside their own graph (the
-// exchange's two buckets are kernels of the step, fb_dist.cu) and apply Adam to the sum; `grads_dev` must be the exchange's
+// Several GPUs, tensor-core path: fb_qnet_step with Adam then sums every rank's gradients inside its own graph (the
+// exchange's two buckets are kernels of the step, fb_dist.cu) and applies Adam to the sum; `grads_dev` must be the exchange's
 // current buffer (fb_dist_grads / fb_dist_parity) and the caller calls fb_dist_advance after each step.  NULL detaches.
 extern "C" int fb_qnet_attach_exchange(fb_qnet *n, fb_dist *d) {
     FB_REQUIRE(n != nullptr, "fb_qnet_attach_exchange: NULL argument");
@@ -469,10 +470,11 @@ extern "C" int fb_qnet_layout(const fb_qnet *n, int32_t *o) {
     return FB_OK;
 }
 
-static FrameView make_view(const uint8_t *frames, long long stride, const int32_t *chan_off) {
-    FrameView fv; fv.base = frames; fv.sample_stride = stride; fv.tab = nullptr; fv.tab_stride = 0;
+// field by field: a view inside a zero-filled QnetStep keeps its padding bytes zero
+static void set_view(FrameView &fv, const uint8_t *frames, long long stride, const int32_t *chan_off, const long long *tab = nullptr,
+                     int tab_stride = 0) {
+    fv.base = frames; fv.sample_stride = stride; fv.tab = tab; fv.tab_stride = tab_stride;
     for (int c = 0; c < 4; c++) fv.chan_off[c] = chan_off[c];
-    return fv;
 }
 
 extern "C" int fb_qnet_forward(fb_qnet *n, const float *params_dev, const uint8_t *frames_dev, long long sample_stride,
@@ -486,7 +488,8 @@ extern "C" int fb_qnet_forward(fb_qnet *n, const float *params_dev, const uint8_
     }
     for (int b0 = 0; b0 < batch; b0 += n->max_batch) {
         int B = min(n->max_batch, batch - b0);
-        FrameView fv = make_view(frames_dev + (size_t)b0 * sample_stride, sample_stride, chan_off);
+        FrameView fv;
+        set_view(fv, frames_dev + (size_t)b0 * sample_stride, sample_stride, chan_off);
         int rc = tc_precision(n->precision) ? tc_forward(n, slot, 0, params_dev, fv, B, q_out_dev + (size_t)b0 * 2, st)
                                                    : forward_chunk(n, params_dev, fv, B, q_out_dev + (size_t)b0 * 2, st);
         if (rc) return rc;
@@ -505,68 +508,37 @@ extern "C" int fb_qnet_act(fb_qnet *n, const float *params_dev, const uint8_t *f
     return FB_OK;
 }
 
-// fb_qnet_loss_backward; ret / disc (f64[batch] or nullptr): the n-step return and discount of each sample (td_target)
-static int loss_backward_impl(fb_qnet *n, int variant, const float *params_dev, const float *target_params_dev,
-                              const uint8_t *frames_dev, long long sample_stride, const int32_t *chan_off_s,
-                              const int32_t *chan_off_next, const uint8_t *actions_dev, const float *rewards_dev,
-                              const uint8_t *terminals_dev, const float *is_weights_dev, int batch, int global_batch,
-                              double gamma, int loss_sum, float *grads_dev, float *loss_out_dev, float *abs_err_out_dev,
-                              float *q_target_out_dev, const double *ret, const double *disc, void *stream) {
-    FB_REQUIRE(n && params_dev && frames_dev && chan_off_s && chan_off_next && actions_dev && rewards_dev && terminals_dev && grads_dev,
-               "fb_qnet_loss_backward: NULL argument");
-    FB_REQUIRE(batch > 0 && batch <= n->max_batch, "fb_qnet_loss_backward: batch exceeds max_batch");
-    FB_REQUIRE(variant >= 0 && variant <= 2, "fb_qnet_loss_backward: variant must be 0 (vanilla), 1 (nature) or 2 (double)");
-    FB_REQUIRE(variant == 0 || target_params_dev != nullptr, "fb_qnet_loss_backward: target parameters required");
-    cudaStream_t st = (cudaStream_t)stream;
+// TD target, loss and backward of the strict-fp32 path into a.grads
+static int loss_backward_impl(fb_qnet *n, const QnetStep &a, cudaStream_t st) {
     const QnetLayout &L = n->L;
-    const int B = batch;
-    if (global_batch <= 0) global_batch = batch;
-    FrameView fs = make_view(frames_dev, sample_stride, chan_off_s), fn = make_view(frames_dev, sample_stride, chan_off_next);
+    const int B = a.B;
     int rc;
-    if (tc_precision(n->precision)) {
-        TcTrainArgs ta{variant, params_dev, target_params_dev, fs, fn, actions_dev, rewards_dev, terminals_dev, is_weights_dev, B,
-                       global_batch, gamma, loss_sum, grads_dev, loss_out_dev ? loss_out_dev : n->loss_dev, abs_err_out_dev,
-                       q_target_out_dev};
-        ta.ret = ret; ta.disc = disc;
-        return tc_loss_backward(n, ta, st);
-    }
     // Q(s') with the net the variant names (and the online net too for Double), then Q(s) last so that its
     // activations are the ones left in the workspace for the backward pass.
-    if (variant == 2) { rc = forward_chunk(n, params_dev, fn, B, n->q_next_online, st); if (rc) return rc; }
-    rc = forward_chunk(n, variant == 0 ? params_dev : target_params_dev, fn, B, n->q_next, st); if (rc) return rc;
-    rc = forward_chunk(n, params_dev, fs, B, n->q, st); if (rc) return rc;
-    td_loss_kernel<<<1, 256, 0, st>>>(n->q, n->q_next, n->q_next_online, actions_dev, rewards_dev, terminals_dev, is_weights_dev,
-                                       B, global_batch, variant, gamma, loss_sum, n->dq, loss_out_dev ? loss_out_dev : n->loss_dev,
-                                       abs_err_out_dev, q_target_out_dev, n->per_broadcast, ret, disc);
+    if (a.variant == 2) { rc = forward_chunk(n, a.params, a.fn, B, n->q_next_online, st); if (rc) return rc; }
+    rc = forward_chunk(n, a.variant == 0 ? a.params : a.target, a.fn, B, n->q_next, st); if (rc) return rc;
+    rc = forward_chunk(n, a.params, a.fs, B, n->q, st); if (rc) return rc;
+    td_loss_kernel<<<1, 256, 0, st>>>(n->q, n->q_next, n->q_next_online, a.actions, a.rewards, a.terminals, a.isw, B, a.global_batch,
+                                       a.variant, a.gamma, a.loss_sum, n->dq, a.loss_out, a.abs_err, a.q_target, n->per_broadcast, a.ret,
+                                       a.disc);
     // ---- backward
-    head_backward_w_kernel<<<(L.hidden + 1 + 127) / 128, 128, 0, st>>>(n->h1, n->dq, L, B, grads_dev);
-    head_backward_h_kernel<<<(B * L.hidden + 255) / 256, 256, 0, st>>>(n->h1, n->dq, params_dev, L, B, n->dh1, nullptr);
+    head_backward_w_kernel<<<(L.hidden + 1 + 127) / 128, 128, 0, st>>>(n->h1, n->dq, L, B, a.grads);
+    head_backward_h_kernel<<<(B * L.hidden + 255) / 256, 256, 0, st>>>(n->h1, n->dq, a.params, L, B, n->dh1, nullptr);
     // fc1: dW = a3^T dh1 (+ bias row), da3 = dh1 Wf1^T masked by relu(a3)
-    wgrad<true>(n, kFlat, L.hidden, B, 64, LoadFc1T{n->a3}, n->dh1, grads_dev + L.wf1, st);
-    launch_gemm<64, false, true>(B, kFlat, L.hidden, 1, LoadPlain{n->dh1, L.hidden}, LoadTrans{params_dev + L.wf1, L.hidden},
+    wgrad<true>(n, kFlat, L.hidden, B, 64, LoadFc1T{n->a3}, n->dh1, a.grads + L.wf1, st);
+    launch_gemm<64, false, true>(B, kFlat, L.hidden, 1, LoadPlain{n->dh1, L.hidden}, LoadTrans{a.params + L.wf1, L.hidden},
                                  EpiMaskPos{n->dz3, n->a3, kFlat}, st);
     // conv3
-    wgrad<true>(n, kK3, kC3, B * 25, 512, LoadConv3T{n->a2}, n->dz3, grads_dev + L.w3, st);
-    launch_gemm<64, false, true>(B * 25, kC2, kK3, 1, LoadDgrad3{n->dz3}, LoadW3T{params_dev + L.w3}, EpiMaskPos{n->dz2, n->a2, kC2}, st);
+    wgrad<true>(n, kK3, kC3, B * 25, 512, LoadConv3T{n->a2}, n->dz3, a.grads + L.w3, st);
+    launch_gemm<64, false, true>(B * 25, kC2, kK3, 1, LoadDgrad3{n->dz3}, LoadW3T{a.params + L.w3}, EpiMaskPos{n->dz2, n->a2, kC2}, st);
     // conv2
-    wgrad<true>(n, kK2, kC2, B * 25, 512, LoadConv2T{n->p1}, n->dz2, grads_dev + L.w2, st);
-    launch_gemm<32, false, true>(B * 100, kC1, 4 * 4 * kC2, 1, LoadDgrad2{n->dz2}, LoadW2T{params_dev + L.w2}, EpiStore{n->dp1, kC1}, st);
+    wgrad<true>(n, kK2, kC2, B * 25, 512, LoadConv2T{n->p1}, n->dz2, a.grads + L.w2, st);
+    launch_gemm<32, false, true>(B * 100, kC1, 4 * 4 * kC2, 1, LoadDgrad2{n->dz2}, LoadW2T{a.params + L.w2}, EpiStore{n->dp1, kC1}, st);
     unpool_relu_kernel<<<(B * 3200 + 255) / 256, 256, 0, st>>>(n->z1, n->p1, n->dp1, n->dz1, B);
     // conv1 (no input gradient)
-    wgrad<false>(n, kK1, kC1, B * 400, 2048, LoadConv1T{fs}, n->dz1, grads_dev + L.w1, st);
+    wgrad<false>(n, kK1, kC1, B * 400, 2048, LoadConv1T{a.fs}, n->dz1, a.grads + L.w1, st);
     FB_CUDA_OK(cudaGetLastError());
     return FB_OK;
-}
-
-extern "C" int fb_qnet_loss_backward(fb_qnet *n, int variant, const float *params_dev, const float *target_params_dev,
-                                     const uint8_t *frames_dev, long long sample_stride, const int32_t *chan_off_s,
-                                     const int32_t *chan_off_next, const uint8_t *actions_dev, const float *rewards_dev,
-                                     const uint8_t *terminals_dev, const float *is_weights_dev, int batch, int global_batch,
-                                     double gamma, int loss_sum, float *grads_dev, float *loss_out_dev, float *abs_err_out_dev,
-                                     float *q_target_out_dev, void *stream) {
-    return loss_backward_impl(n, variant, params_dev, target_params_dev, frames_dev, sample_stride, chan_off_s, chan_off_next, actions_dev,
-                              rewards_dev, terminals_dev, is_weights_dev, batch, global_batch, gamma, loss_sum, grads_dev, loss_out_dev,
-                              abs_err_out_dev, q_target_out_dev, nullptr, nullptr, stream);
 }
 
 extern "C" int fb_qnet_adam(fb_qnet *n, float *params_dev, const float *grads_dev, float *m_dev, float *v_dev, float alpha,
@@ -581,97 +553,72 @@ extern "C" int fb_qnet_adam(fb_qnet *n, float *params_dev, const float *grads_de
     return FB_OK;
 }
 
-// session.run(trainStep) in one call (BrainDQN.py:204-207): fb_qnet_loss_backward followed by fb_qnet_adam with
-// alpha = lr sqrt(1 - beta2_power) / (1 - beta1_power).  On the tensor-core path the Adam update rides in the step's last
-// kernel and the whole step is one CUDA graph launch.
-extern "C" int fb_qnet_train_step(fb_qnet *n, int variant, float *params_dev, const float *target_params_dev, const uint8_t *frames_dev,
-                                  long long sample_stride, const int32_t *chan_off_s, const int32_t *chan_off_next,
-                                  const uint8_t *actions_dev, const float *rewards_dev, const uint8_t *terminals_dev,
-                                  const float *is_weights_dev, int batch, int global_batch, double gamma, int loss_sum, float *grads_dev,
-                                  float *loss_out_dev, float *abs_err_out_dev, float *q_target_out_dev, float *m_dev, float *v_dev, float lr,
-                                  float beta1, float beta2, float eps, float grad_scale, float beta1_power, float beta2_power, void *stream) {
-    FB_REQUIRE(n && params_dev && m_dev && v_dev && grads_dev, "fb_qnet_train_step: NULL argument");
-    if (tc_precision(n->precision) && n->tc != nullptr) {
-        FB_REQUIRE(frames_dev && chan_off_s && chan_off_next && actions_dev && rewards_dev && terminals_dev, "fb_qnet_train_step: NULL argument");
-        FB_REQUIRE(batch > 0 && batch <= n->max_batch, "fb_qnet_train_step: batch exceeds max_batch");
-        FB_REQUIRE(variant >= 0 && variant <= 2, "fb_qnet_train_step: variant must be 0 (vanilla), 1 (nature) or 2 (double)");
-        FB_REQUIRE(variant == 0 || target_params_dev != nullptr, "fb_qnet_train_step: target parameters required");
-        if (global_batch <= 0) global_batch = batch;
-        FrameView fs = make_view(frames_dev, sample_stride, chan_off_s), fn = make_view(frames_dev, sample_stride, chan_off_next);
-        TcTrainArgs ta{variant, params_dev, target_params_dev, fs, fn, actions_dev, rewards_dev, terminals_dev, is_weights_dev, batch,
-                       global_batch, gamma, loss_sum, grads_dev, loss_out_dev ? loss_out_dev : n->loss_dev, abs_err_out_dev,
-                       q_target_out_dev, AdamFuse{1, m_dev, v_dev, lr, beta1, beta2, eps, grad_scale}, n->xch};
-        return tc_train_step(n, ta, beta1_power, beta2_power, (cudaStream_t)stream);
+// _trainQNetwork up to session.run(trainStep) (BrainDQN.py:195-223): sampling, loss, backward and Adam as the arguments ask.
+// On the tensor-core path it is one CUDA graph launch (tc_step); here the same stages run one after the other.
+extern "C" int fb_qnet_step(fb_qnet *n, const fb_qnet_step_args *a, void *stream) {
+    FB_REQUIRE(n && a && a->params_dev && a->grads_dev, "fb_qnet_step: NULL argument");
+    FB_REQUIRE(a->variant >= 0 && a->variant <= 2, "fb_qnet_step: variant must be 0 (vanilla), 1 (nature) or 2 (double)");
+    FB_REQUIRE(a->variant == 0 || a->target_params_dev != nullptr, "fb_qnet_step: target parameters required");
+    FB_REQUIRE((a->m_dev != nullptr) == (a->v_dev != nullptr), "fb_qnet_step: m_dev and v_dev must both be set (Adam) or both be NULL");
+    const fb_step_sampling *sp = a->sampling;
+    if (sp) {
+        bool caller_minibatch = a->frames_dev || a->sample_stride || a->actions_dev || a->rewards_dev || a->terminals_dev || a->is_weights_dev;
+        for (int c = 0; c < 4; c++) caller_minibatch = caller_minibatch || a->chan_off_s[c] || a->chan_off_next[c];
+        FB_REQUIRE(!caller_minibatch, "fb_qnet_step: with `sampling` the step draws its minibatch: frames_dev .. is_weights_dev must be 0 / NULL");
+        FB_REQUIRE(sp->replay && (a->batch == 0 || a->batch == sp->batch), "fb_qnet_step: bad sampling descriptor or batch");
+        FB_REQUIRE(!sp->prioritized || a->abs_err_out_dev, "fb_qnet_step: prioritized replay needs abs_err_out_dev");
+    } else {
+        FB_REQUIRE(a->frames_dev && a->actions_dev && a->rewards_dev && a->terminals_dev, "fb_qnet_step: NULL argument");
     }
-    int rc = fb_qnet_loss_backward(n, variant, params_dev, target_params_dev, frames_dev, sample_stride, chan_off_s, chan_off_next, actions_dev,
-                                   rewards_dev, terminals_dev, is_weights_dev, batch, global_batch, gamma, loss_sum, grads_dev, loss_out_dev,
-                                   abs_err_out_dev, q_target_out_dev, stream);
-    if (rc) return rc;
-    const float alpha = lr * sqrtf(1.f - beta2_power) / (1.f - beta1_power);
-    return fb_qnet_adam(n, params_dev, grads_dev, m_dev, v_dev, alpha, beta1, beta2, eps, grad_scale, stream);
-}
+    const int batch = sp ? sp->batch : a->batch;
+    FB_REQUIRE(batch > 0 && batch <= n->max_batch, "fb_qnet_step: batch outside 1..max_batch");
+    const bool tc = tc_precision(n->precision);
+    cudaStream_t st = (cudaStream_t)stream;
 
-// The same with the minibatch drawn by the step's first two kernels (uniform replay): on the tensor-core path sampling,
-// gather, forward, backward and Adam are one CUDA graph launch.  With sp->n_step >= 1 the minibatch rows hold F frames and the
-// TD target is the n-step one (fb_step_sampling).
-extern "C" int fb_qnet_train_step_sampled(fb_qnet *n, const fb_step_sampling *sp, int variant, float *params_dev,
-                                          const float *target_params_dev, const int32_t *chan_off_s, const int32_t *chan_off_next,
-                                          int global_batch, double gamma, int loss_sum, float *grads_dev, float *loss_out_dev,
-                                          float *abs_err_out_dev, float *q_target_out_dev, float *m_dev, float *v_dev, float lr, float beta1,
-                                          float beta2, float eps, float grad_scale, float beta1_power, float beta2_power, void *stream) {
-    FB_REQUIRE(n && sp && sp->replay && params_dev && grads_dev && chan_off_s && chan_off_next && (m_dev != nullptr) == (v_dev != nullptr),
-               "fb_qnet_train_step_sampled: NULL argument");
-    const bool adam = m_dev != nullptr;            // without Adam slots: gradients only (the caller applies Adam, e.g. fb_dist_adam)
-    const int batch = sp->batch;
-    const int F = replay_frames_per_sample(*sp);   // frames per minibatch row: 5, or 4 + min(n, 4) with n-step returns
-    const double *ret = sp->n_step > 0 ? sp->ret_out_dev : nullptr, *disc = sp->n_step > 0 ? sp->disc_out_dev : nullptr;
-    if (tc_precision(n->precision) && n->tc != nullptr) {
-        FB_REQUIRE(batch > 0 && batch <= n->max_batch, "fb_qnet_train_step_sampled: batch exceeds max_batch");
-        FB_REQUIRE(variant >= 0 && variant <= 2, "fb_qnet_train_step_sampled: variant must be 0 (vanilla), 1 (nature) or 2 (double)");
-        FB_REQUIRE(variant == 0 || target_params_dev != nullptr, "fb_qnet_train_step_sampled: target parameters required");
-        if (global_batch <= 0) global_batch = batch;
-        FrameView fs = make_view(sp->frames_out_dev, F * 6400, chan_off_s), fn = make_view(sp->frames_out_dev, F * 6400, chan_off_next);
-        // channels that are whole frames of the minibatch buffer (the usual 0..3 / 1..4): the convolutions read them in place from
-        // the ring through the offsets the sampler leaves behind; the gather into frames_out_dev runs beside the forward passes
-        bool in_place = sp->ring_dev != nullptr;
-        for (int c = 0; c < 4; c++) in_place = in_place && chan_off_s[c] % 6400 == 0 && chan_off_s[c] / 6400 < F && chan_off_s[c] >= 0 &&
-                                               chan_off_next[c] % 6400 == 0 && chan_off_next[c] / 6400 < F && chan_off_next[c] >= 0;
-        if (in_place) {
-            fs.base = fn.base = sp->ring_dev; fs.sample_stride = fn.sample_stride = 0; fs.tab = fn.tab = replay_frame_tab(sp->replay);
-            fs.tab_stride = fn.tab_stride = F;
-            for (int c = 0; c < 4; c++) { fs.chan_off[c] = chan_off_s[c] / 6400; fn.chan_off[c] = chan_off_next[c] / 6400; }
-        }
-        FB_REQUIRE(!sp->prioritized || abs_err_out_dev != nullptr, "fb_qnet_train_step_sampled: prioritized replay needs abs_err_out_dev");
-        TcTrainArgs ta{variant, params_dev, target_params_dev, fs, fn, sp->act_out_dev, sp->rew_out_dev, sp->term_out_dev,
-                       sp->prioritized ? sp->is_weights_f32_out_dev : nullptr, batch,
-                       global_batch, gamma, loss_sum, grads_dev, loss_out_dev ? loss_out_dev : n->loss_dev, abs_err_out_dev,
-                       q_target_out_dev, AdamFuse{adam ? 1 : 0, m_dev, v_dev, lr, beta1, beta2, eps, grad_scale}, adam ? n->xch : nullptr, *sp,
-                       ret, disc};
-        return adam ? tc_train_step(n, ta, beta1_power, beta2_power, (cudaStream_t)stream) : tc_loss_backward(n, ta, (cudaStream_t)stream);
+    QnetStep s;
+    memset(&s, 0, sizeof(s));
+    s.variant = a->variant; s.params = a->params_dev; s.target = a->target_params_dev;
+    s.B = batch; s.global_batch = a->global_batch > 0 ? a->global_batch : batch; s.gamma = a->gamma; s.loss_sum = a->loss_sum;
+    s.grads = a->grads_dev; s.loss_out = a->loss_out_dev ? a->loss_out_dev : n->loss_dev; s.abs_err = a->abs_err_out_dev;
+    s.q_target = a->q_target_out_dev;
+    if (a->m_dev) {
+        s.ad.on = 1; s.ad.m = a->m_dev; s.ad.v = a->v_dev; s.ad.lr = a->lr; s.ad.beta1 = a->beta1; s.ad.beta2 = a->beta2;
+        s.ad.eps = a->eps; s.ad.grad_scale = a->grad_scale;
+        s.xch = n->xch;
     }
-    FB_REQUIRE(!sp->prioritized || abs_err_out_dev != nullptr, "fb_qnet_train_step_sampled: prioritized replay needs abs_err_out_dev");
-    int rc = replay_launch_sample_gather(*sp, gamma, (cudaStream_t)stream);
-    if (rc) return rc;
-    if (!adam)
-        rc = loss_backward_impl(n, variant, params_dev, target_params_dev, sp->frames_out_dev, F * 6400, chan_off_s, chan_off_next,
-                                sp->act_out_dev, sp->rew_out_dev, sp->term_out_dev, sp->prioritized ? sp->is_weights_f32_out_dev : nullptr,
-                                batch, global_batch, gamma, loss_sum, grads_dev, loss_out_dev, abs_err_out_dev, q_target_out_dev, ret, disc, stream);
-    else if (ret == nullptr)
-    rc = fb_qnet_train_step(n, variant, params_dev, target_params_dev, sp->frames_out_dev, 5 * 6400, chan_off_s, chan_off_next,
-                            sp->act_out_dev, sp->rew_out_dev, sp->term_out_dev, sp->prioritized ? sp->is_weights_f32_out_dev : nullptr, batch,
-                            global_batch, gamma, loss_sum, grads_dev, loss_out_dev, abs_err_out_dev, q_target_out_dev, m_dev, v_dev, lr, beta1,
-                            beta2, eps, grad_scale, beta1_power, beta2_power, stream);
-    else {                                         // fb_qnet_train_step's CUDA-core path with the n-step target
-        rc = loss_backward_impl(n, variant, params_dev, target_params_dev, sp->frames_out_dev, F * 6400, chan_off_s, chan_off_next,
-                                sp->act_out_dev, sp->rew_out_dev, sp->term_out_dev, sp->prioritized ? sp->is_weights_f32_out_dev : nullptr,
-                                batch, global_batch, gamma, loss_sum, grads_dev, loss_out_dev, abs_err_out_dev, q_target_out_dev, ret, disc, stream);
-        if (rc == FB_OK) {
-            const float alpha = lr * sqrtf(1.f - beta2_power) / (1.f - beta1_power);
-            rc = fb_qnet_adam(n, params_dev, grads_dev, m_dev, v_dev, alpha, beta1, beta2, eps, grad_scale, stream);
+    if (sp) {
+        s.pro = *sp;
+        s.actions = sp->act_out_dev; s.rewards = sp->rew_out_dev; s.terminals = sp->term_out_dev;
+        s.isw = sp->prioritized ? sp->is_weights_f32_out_dev : nullptr;
+        if (sp->n_step > 0) { s.ret = sp->ret_out_dev; s.disc = sp->disc_out_dev; }
+        // s = frames 0..3, s' = frames F-4..F-1 of each drawn row.  The tensor cores read them in place from the ring through the
+        // offsets the sampler leaves behind (frame numbers into that table; the gather runs beside the forward passes); the
+        // fp32 path reads the gathered rows (byte offsets)
+        const int F = replay_frames_per_sample(*sp), unit = tc ? 1 : FB_FRAME_BYTES;
+        int32_t off_s[4], off_n[4];
+        for (int c = 0; c < 4; c++) { off_s[c] = c * unit; off_n[c] = (F - 4 + c) * unit; }
+        if (tc) {
+            set_view(s.fs, sp->ring_dev, 0, off_s, replay_frame_tab(sp->replay), F);
+            set_view(s.fn, sp->ring_dev, 0, off_n, replay_frame_tab(sp->replay), F);
+        } else {
+            set_view(s.fs, sp->frames_out_dev, (long long)F * FB_FRAME_BYTES, off_s);
+            set_view(s.fn, sp->frames_out_dev, (long long)F * FB_FRAME_BYTES, off_n);
         }
+    } else {
+        s.actions = a->actions_dev; s.rewards = a->rewards_dev; s.terminals = a->terminals_dev; s.isw = a->is_weights_dev;
+        set_view(s.fs, a->frames_dev, a->sample_stride, a->chan_off_s);
+        set_view(s.fn, a->frames_dev, a->sample_stride, a->chan_off_next);
     }
-    if (rc) return rc;
-    return sp->prioritized ? replay_launch_per_update(*sp, abs_err_out_dev, (cudaStream_t)stream) : FB_OK;
+    if (tc) return tc_step(n, s, a->beta1_power, a->beta2_power, st);
+
+    int rc = sp ? replay_launch_sample_gather(*sp, s.gamma, st) : FB_OK;
+    if (rc == FB_OK) rc = loss_backward_impl(n, s, st);
+    if (rc == FB_OK && s.ad.on) {
+        const float alpha = a->lr * sqrtf(1.f - a->beta2_power) / (1.f - a->beta1_power);
+        rc = fb_qnet_adam(n, a->params_dev, a->grads_dev, a->m_dev, a->v_dev, alpha, a->beta1, a->beta2, a->eps, a->grad_scale, stream);
+    }
+    if (rc == FB_OK && sp && sp->prioritized) rc = replay_launch_per_update(*sp, s.abs_err, st);
+    return rc;
 }
 
 // target_replace_op (BrainDQNNature.py:107-111): hard copy of all variables

@@ -102,11 +102,12 @@ void qnet_launch_td_loss(const float *q_s, const float *q_next, const float *q_n
 void qnet_launch_head_backward(const float *h1, const float *dq, const float *params, const QnetLayout &L, int B, float *grads,
                                float *dh1_f32, __nv_bfloat16 *dh1_bf16, cudaStream_t st);
 
-// tcgen05 path entry points (fb_qnet_tc.cu); all return FB_OK or an error code with fb_set_error set
-// Adam fused into the last kernel of the training step (fb_qnet_train_step): alpha comes from the beta powers kept in
-// device memory, so a captured step replays without any per-step argument
+// One training step as fb_qnet_step validated it (fb_qnet.cu); both precisions run from it.  fb_qnet_step zero-fills it
+// before setting any field: a captured tensor-core step is keyed on its bytes, padding included (tc_step).
+// Adam: on the tensor-core path fused into the last kernel of the step, alpha from the beta powers kept in device memory, so a
+// captured step replays without any per-step argument
 struct AdamFuse { int on; float *m, *v; float lr, beta1, beta2, eps, grad_scale; };
-struct TcTrainArgs {
+struct QnetStep {
     int variant;
     const float *params, *target;
     FrameView fs, fn;                       // s and s' views of the minibatch frames
@@ -118,6 +119,7 @@ struct TcTrainArgs {
     fb_step_sampling pro;                   // pro.replay != nullptr: the minibatch is drawn by the step's first two kernels
     const double *ret, *disc;               // n-step return / discount per sample (pro.n_step >= 1), else nullptr: 1-step target
 };
+// tcgen05 path entry points (fb_qnet_tc.cu); all return FB_OK or an error code with fb_set_error set
 // fb_replay.cu: the two kernels of fb_replay_sample_uniform + fb_replay_gather on `st`; and the per-step patch of their
 // nodes in an instantiated graph (`t` -- and through it the n-step horizon t - n + 1 -- is the only argument that changes).
 // gamma: the step's discount, which the n-step gather folds into R and disc.
@@ -129,8 +131,7 @@ int replay_frames_per_sample(const fb_step_sampling &p);                        
 int replay_launch_per_update(const fb_step_sampling &p, const float *abs_err_dev, cudaStream_t st);     // Memory.batch_update, prioritized only
 bool replay_is_sampler(const void *func);        // sample_uniform_kernel or per_sample_kernel
 bool replay_is_gather(const void *func);
-int replay_patch_nodes(cudaGraphExec_t exec, cudaGraphNode_t sampler, cudaGraphNode_t gather, const fb_step_sampling &p, double gamma,
-                       bool with_tab);
+int replay_patch_nodes(cudaGraphExec_t exec, cudaGraphNode_t sampler, cudaGraphNode_t gather, const fb_step_sampling &p, double gamma);
 inline bool tc_precision(int precision) { return precision == FB_PRECISION_BF16 || precision == FB_PRECISION_FP16; }
 // fb_dist.cu: one bucket of the exchange + Adam as a kernel on `st` (bucket 0 = W_fc1, 1 = the rest), for the exchange buffer of
 // the current parity; the buffer the step's gradients must have been written to
@@ -146,7 +147,6 @@ int tc_slot_for(fb_qnet *n, const float *params_dev, int want_slot, cudaStream_t
 int tc_forward(fb_qnet *n, int slot, int ws, const float *params_dev, FrameView fv, int B, float *q_out, cudaStream_t st);
 int tc_forward_chunks(fb_qnet *n, int slot, const float *params_dev, const uint8_t *frames_dev, long long sample_stride,
                       const int32_t *chan_off, int batch, float *q_out_dev, cudaStream_t st);
-int tc_loss_backward(fb_qnet *n, const TcTrainArgs &a, cudaStream_t st);
-int tc_train_step(fb_qnet *n, const TcTrainArgs &a, float beta1_power, float beta2_power, cudaStream_t st);
+int tc_step(fb_qnet *n, const QnetStep &a, float beta1_power, float beta2_power, cudaStream_t st);
 int tc_adam(fb_qnet *n, float *params_dev, const float *grads_dev, float *m_dev, float *v_dev, float alpha, float beta1, float beta2,
             float eps, float grad_scale, cudaStream_t st);

@@ -520,7 +520,7 @@ __global__ void __launch_bounds__(256) colsum_kernel(ColsumJobs jobs) {
 // sum_b dh1.  Block = 32 hidden units x 8 row lanes; block gridDim.x-1 does the head bias.
 constexpr int kHeadRows = 256;                      // rows of the minibatch per head-backward CTA row group
 constexpr int kMaxHeadCtas = 160;                   // fused head kernel: at most one CTA (four samples at a time) per SM
-// Fused Adam (fb_qnet_train_step): one thread of this kernel -- early on the step's critical path, exactly once per step --
+// Fused Adam (fb_qnet_step with m_dev / v_dev): one thread of this kernel -- early on the step's critical path, exactly once per step --
 // turns the beta powers kept in device memory into this step's alpha = lr sqrt(1 - beta2^t) / (1 - beta1^t) (fp32, the
 // host formula) and advances them; the step's last kernel reads alpha.  Nothing about a step is a launch argument.
 struct AdamPow { int on; float *pow /* beta1^t, beta2^t */, *alpha; float lr, beta1, beta2; };
@@ -819,7 +819,7 @@ struct FinalizeArgs {
     float *loss_out;
     float inv_scale;                                // un-scales what came through the (scaled) gradient tensors
 };
-// With `ad.on` the same launch also applies Adam (fb_qnet_train_step): the CTA that has just summed 32 gradient elements
+// With `ad.on` the same launch also applies Adam (fb_qnet_step): the CTA that has just summed 32 gradient elements
 // updates those parameters (W_fc1, whose gradient the fc1 GEMM wrote in place, is updated earlier by adam_wf1_kernel).
 // alpha was left in device memory by the head kernel, so the whole update replays as one CUDA graph.
 // These kernels WRITE the bf16 operand copies: no early launch_dependents (see pack_weights_kernel).
@@ -1436,7 +1436,7 @@ struct TcPlan {                 // everything that depends on the batch size
     int s1, s2, s3, sf;                                              // split-K counts (conv weight gradients, fc1 forward)
 };
 struct GraphKey {               // a captured training step is replayed only for byte-identical arguments
-    TcTrainArgs a;
+    QnetStep a;
     int pack_online, pack_target;
 };
 struct GraphEntry {
@@ -1457,7 +1457,7 @@ struct TcState {
     float *bp1, *bp2, *bp3;
     float *hp, *hb;             // head-backward partials per row group
     float *loss_terms;          // per-sample loss terms
-    float *adam_pow;            // device: beta1^t, beta2^t of the fused Adam (fb_qnet_train_step), then this step's alpha
+    float *adam_pow;            // device: beta1^t, beta2^t of the fused Adam (fb_qnet_step), then this step's alpha
     float pow_host[2];          // what adam_pow will hold once everything enqueued so far has run
     float *pow_pinned;          // 16 x 2 staging slots for re-seeding adam_pow
     int pow_slot;
@@ -1842,7 +1842,7 @@ namespace {
 // (online forward on s -> TD loss -> data gradients -> conv1 weight gradient -> finalize) stays on `st`; the Q(s')
 // forward(s) and the other weight gradients run beside it on the auxiliary stream.  The same code is what a CUDA
 // graph captures.
-int train_step_launch(fb_qnet *n, const TcTrainArgs &a, int pack_online, int pack_target, cudaStream_t st) {
+int train_step_launch(fb_qnet *n, const QnetStep &a, int pack_online, int pack_target, cudaStream_t st) {
     TcState *t = n->tc;
     TcPlan *p;
     int rc = make_plan(n, a.B, &p);
@@ -1862,17 +1862,15 @@ int train_step_launch(fb_qnet *n, const TcTrainArgs &a, int pack_online, int pac
     // the minibatch itself.  The sampler leaves the ring offsets of the drawn frames behind (a.fs.tab): the convolutions read the
     // frames in place, and the gather into the caller-visible minibatch buffers (frames, actions, rewards, terminals -- the head
     // kernel needs the last three) runs on a side stream beside the forward passes: one dependent stage less (5.5 us)
-    const bool in_place = a.pro.replay != nullptr && a.fs.tab != nullptr;
-    t->step_samples = a.pro.replay != nullptr ? 1 : 0;            // (read by conv1_mode_at; reset below, after the step's conv1 launches)
+    const bool sampled = a.pro.replay != nullptr;
+    t->step_samples = sampled ? 1 : 0;                            // (read by conv1_mode_at; reset below, after the step's conv1 launches)
     const int e_gather = 12;
-    if (a.pro.replay != nullptr) {
-        rc = replay_launch_sample(a.pro, in_place, st); if (rc) return rc;
-        if (in_place) {
-            FB_CUDA_OK(cudaEventRecord(t->ev[e_gather], st));
-            FB_CUDA_OK(cudaStreamWaitEvent(t->aux4, t->ev[e_gather], 0));
-            rc = replay_launch_gather(a.pro, a.gamma, t->aux4); if (rc) return rc;
-            FB_CUDA_OK(cudaEventRecord(t->ev[e_gather], t->aux4));
-        } else { rc = replay_launch_gather(a.pro, a.gamma, st); if (rc) return rc; }
+    if (sampled) {
+        rc = replay_launch_sample(a.pro, true, st); if (rc) return rc;
+        FB_CUDA_OK(cudaEventRecord(t->ev[e_gather], st));
+        FB_CUDA_OK(cudaStreamWaitEvent(t->aux4, t->ev[e_gather], 0));
+        rc = replay_launch_gather(a.pro, a.gamma, t->aux4); if (rc) return rc;
+        FB_CUDA_OK(cudaEventRecord(t->ev[e_gather], t->aux4));
     }
     if (pack_online) { rc = tc_pack_weights(n, a.params, 0, st); if (rc) return rc; }
     FB_CUDA_OK(fork(st, sx));
@@ -1881,7 +1879,7 @@ int train_step_launch(fb_qnet *n, const TcTrainArgs &a, int pack_online, int pac
     if (a.variant == 2) { rc = tc_forward(n, 0, 1, a.params, a.fn, B, n->q_next_online, sx); if (rc) return rc; }
     rc = a.variant == 0 ? tc_forward(n, 0, 1, a.params, a.fn, B, n->q_next, sx) : tc_forward(n, 1, 1, a.target, a.fn, B, n->q_next, sx);
     if (rc) return rc;
-    if (in_place) FB_CUDA_OK(cudaStreamWaitEvent(sx, t->ev[e_gather], 0));    // the event below then also says: minibatch buffers complete
+    if (sampled) FB_CUDA_OK(cudaStreamWaitEvent(sx, t->ev[e_gather], 0));     // the event below then also says: minibatch buffers complete
     // ---- main: Q(s) with the online net; its activations stay in workspace 0 for the backward pass
     // the TD target, loss and dLoss/dQ come out of its head kernel, which first waits for Q(s') from the other stream
     FB_CUDA_OK(cudaEventRecord(t->ev[e], sx));
@@ -1905,7 +1903,7 @@ int train_step_launch(fb_qnet *n, const TcTrainArgs &a, int pack_online, int pac
     e++;
     // Memory.batch_update (BrainPrioritizedReplyDQN.py:316) needs only |TD error|, which the head kernel has just written: it runs on
     // a stream of its own beside the whole backward pass (measured: 26 us at the step's tail otherwise) and joins at the end
-    const bool per_on_side = a.pro.replay != nullptr && a.pro.prioritized;
+    const bool per_on_side = sampled && a.pro.prioritized;
     int e_head = -1;
     if (per_on_side) { e_head = e++; FB_CUDA_OK(cudaEventRecord(t->ev[e_head], st)); }       // launched below, after the fc1 gradient GEMMs
     // ---- backward.  The head's backward pass rode in the forward's last kernel when hidden = 512 (fc1_head_train_kernel);
@@ -2047,32 +2045,23 @@ extern "C" int fb_qnet_use_graphs(fb_qnet *n, int enable) {
     return FB_OK;
 }
 
-int tc_loss_backward(fb_qnet *n, const TcTrainArgs &a, cudaStream_t st) {
+// One training step (fb_qnet_step).  With Adam, beta*_power are the caller's (QNetwork keeps them like TF's beta1_power /
+// beta2_power variables); the device copy is re-seeded only when it does not already hold them (first step, load_state_dict, a
+// separate fb_qnet_adam in between).
+int tc_step(fb_qnet *n, const QnetStep &a, float beta1_power, float beta2_power, cudaStream_t st) {
     TcState *t = n->tc;
-    FB_REQUIRE(t != nullptr && a.B > 0 && a.B <= n->max_batch, "tc_loss_backward: bad argument");
-    GraphKey key;
-    memset(&key, 0, sizeof(key));                // padding bytes take part in the comparison
-    key.a.variant = a.variant; key.a.params = a.params; key.a.target = a.target;
-    key.a.fs.base = a.fs.base; key.a.fs.sample_stride = a.fs.sample_stride; key.a.fn.base = a.fn.base; key.a.fn.sample_stride = a.fn.sample_stride;
-    for (int c = 0; c < 4; c++) { key.a.fs.chan_off[c] = a.fs.chan_off[c]; key.a.fn.chan_off[c] = a.fn.chan_off[c]; }
-    key.a.fs.tab = a.fs.tab; key.a.fn.tab = a.fn.tab; key.a.fs.tab_stride = a.fs.tab_stride; key.a.fn.tab_stride = a.fn.tab_stride;
-    key.a.ret = a.ret; key.a.disc = a.disc;
-    key.a.actions = a.actions; key.a.rewards = a.rewards; key.a.terminals = a.terminals; key.a.isw = a.isw;
-    key.a.B = a.B; key.a.global_batch = a.global_batch; key.a.gamma = a.gamma; key.a.loss_sum = a.loss_sum;
-    key.a.grads = a.grads; key.a.loss_out = a.loss_out; key.a.abs_err = a.abs_err; key.a.q_target = a.q_target;
-    key.a.ad.on = a.ad.on; key.a.ad.m = a.ad.m; key.a.ad.v = a.ad.v; key.a.ad.lr = a.ad.lr; key.a.ad.beta1 = a.ad.beta1; key.a.ad.beta2 = a.ad.beta2;
-    key.a.ad.eps = a.ad.eps; key.a.ad.grad_scale = a.ad.grad_scale;
-    key.a.xch = a.xch;
-    {   // the sampling head: everything but `t`, which is patched into the two nodes before every launch
-        const fb_step_sampling &q = a.pro; fb_step_sampling &k = key.a.pro;
-        k.replay = q.replay; k.ring_dev = q.ring_dev; k.act_dev = q.act_dev; k.rew_dev = q.rew_dev; k.term_dev = q.term_dev;
-        k.batch = q.batch; k.setsize = q.setsize; k.seed = q.seed; k.idx_out_dev = q.idx_out_dev; k.frames_out_dev = q.frames_out_dev;
-        k.act_out_dev = q.act_out_dev; k.rew_out_dev = q.rew_out_dev; k.term_out_dev = q.term_out_dev; k.env_out_dev = q.env_out_dev;
-        k.k_out_dev = q.k_out_dev;
-        k.prioritized = q.prioritized; k.per_mode = q.per_mode; k.tree_idx_out_dev = q.tree_idx_out_dev;       // (beta is patched like t)
-        k.is_weights_out_dev = q.is_weights_out_dev; k.prio_out_dev = q.prio_out_dev; k.is_weights_f32_out_dev = q.is_weights_f32_out_dev;
-        k.n_step = q.n_step; k.ret_out_dev = q.ret_out_dev; k.disc_out_dev = q.disc_out_dev;     // n: frames per row, gather grid, horizon
+    if (a.ad.on) {
+        if (t->pow_host[0] != beta1_power || t->pow_host[1] != beta2_power) {
+            float *slot = t->pow_pinned + 2 * (t->pow_slot++ & 15);
+            slot[0] = beta1_power; slot[1] = beta2_power;
+            FB_CUDA_OK(cudaMemcpyAsync(t->adam_pow, slot, 2 * sizeof(float), cudaMemcpyHostToDevice, st));
+        }
+        t->pow_host[0] = t->pow_host[1] = -1.f;  // unknown unless the step below is enqueued in full
     }
+    GraphKey key;
+    memset(&key, 0, sizeof(key));
+    memcpy(&key.a, &a, sizeof(a));               // every argument, padding included (zero: fb_qnet_step zero-fills `a`) ...
+    key.a.pro.t = 0; key.a.pro.beta = 0.0;       // ... but the two that are patched into the sampler / gather nodes every step
     key.pack_online = n->packed_src[0] != a.params;
     key.pack_target = a.variant != 0 && n->packed_src[1] != a.target;
     int rc = FB_OK;
@@ -2086,7 +2075,7 @@ int tc_loss_backward(fb_qnet *n, const TcTrainArgs &a, cudaStream_t st) {
         }
     }
     if (ge && ge->exec) {
-        if (a.pro.replay != nullptr) { rc = replay_patch_nodes(ge->exec, ge->n_sampler, ge->n_gather, a.pro, a.gamma, a.fs.tab != nullptr); if (rc) return rc; }
+        if (a.pro.replay != nullptr) { rc = replay_patch_nodes(ge->exec, ge->n_sampler, ge->n_gather, a.pro, a.gamma); if (rc) return rc; }
         FB_CUDA_OK(cudaGraphLaunch(ge->exec, st));
     } else if (ge && ge->seen >= 1) {            // second identical call: capture (everything lazy was initialised by the first)
         cudaGraph_t graph = nullptr;
@@ -2123,23 +2112,7 @@ int tc_loss_backward(fb_qnet *n, const TcTrainArgs &a, cudaStream_t st) {
     n->packed_src[0] = a.params;            // (with a fused Adam the kernel has re-packed what it updated)
     if (a.variant != 0) n->packed_src[1] = a.target;
     if (a.ad.on && n->packed_src[1] == a.params) n->packed_src[1] = nullptr;
-    return FB_OK;
-}
-
-// loss_backward + Adam as one step.  beta*_power are the caller's (QNetwork keeps them like TF's beta1_power / beta2_power
-// variables); the device copy is re-seeded only when it does not already hold them (first step, load_state_dict, a separate
-// fb_qnet_adam in between).
-int tc_train_step(fb_qnet *n, const TcTrainArgs &a, float beta1_power, float beta2_power, cudaStream_t st) {
-    TcState *t = n->tc;
-    FB_REQUIRE(t != nullptr && a.ad.on && a.ad.m && a.ad.v, "tc_train_step: bad argument");
-    if (t->pow_host[0] != beta1_power || t->pow_host[1] != beta2_power) {
-        float *slot = t->pow_pinned + 2 * (t->pow_slot++ & 15);
-        slot[0] = beta1_power; slot[1] = beta2_power;
-        FB_CUDA_OK(cudaMemcpyAsync(t->adam_pow, slot, 2 * sizeof(float), cudaMemcpyHostToDevice, st));
-    }
-    int rc = tc_loss_backward(n, a, st);
-    if (rc) { t->pow_host[0] = t->pow_host[1] = -1.f; return rc; }
-    t->pow_host[0] = beta1_power * a.ad.beta1; t->pow_host[1] = beta2_power * a.ad.beta2;
+    if (a.ad.on) { t->pow_host[0] = beta1_power * a.ad.beta1; t->pow_host[1] = beta2_power * a.ad.beta2; }
     return FB_OK;
 }
 

@@ -581,7 +581,7 @@ static void launch_per_sample(fb_replay *r, int batch, double beta, uint64_t see
                                                                                                r->counters + 1, tree_idx, data_idx, isw, prio, isw32, ft);
 }
 
-// ---- sampling + gather as the head of a captured training step (fb_qnet_train_step_sampled) -------------------------
+// ---- sampling + gather as the head of a captured training step (fb_qnet_step with `sampling`) -------------------------
 // n_step == 0: the 1-step transitions; n_step >= 1: everything is decoded at t_eff = t - n + 1 (see the top of this file)
 static int horizon(const fb_step_sampling &p) { return p.n_step > 0 ? p.n_step : 1; }
 static long long decode_time(const fb_step_sampling &p) { return p.t - horizon(p) + 1; }
@@ -647,12 +647,12 @@ int replay_launch_per_update(const fb_step_sampling &p, const float *abs_err_dev
 }
 bool replay_is_sampler(const void *func) { return func == (const void *)sample_uniform_kernel || func == (const void *)per_sample_kernel; }
 bool replay_is_gather(const void *func) { return func == (const void *)gather_kernel; }
-int replay_patch_nodes(cudaGraphExec_t exec, cudaGraphNode_t sampler, cudaGraphNode_t gather, const fb_step_sampling &p, double gamma,
-                       bool with_tab) {
+// (a captured step always has its sampler leave the frame offsets behind: the tensor-core step reads the frames in place)
+int replay_patch_nodes(cudaGraphExec_t exec, cudaGraphNode_t sampler, cudaGraphNode_t gather, const fb_step_sampling &p, double gamma) {
     fb_replay *r = p.replay;
     cudaKernelNodeParams kp{};
     int batch = p.batch; uint64_t seed = p.seed; int32_t *idx = p.idx_out_dev;
-    FrameTabArgs ft = sampling_frame_tab(p, with_tab);
+    FrameTabArgs ft = sampling_frame_tab(p, true);
     if (p.prioritized) {
         const double *tree = r->tree, *mn = r->gmin ? r->gmin : r->mn; int cap = r->cap; double beta = p.beta; unsigned long long *word_pos = r->word_pos + 1;
         unsigned int *done = r->counters + 1;

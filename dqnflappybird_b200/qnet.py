@@ -15,19 +15,7 @@ import torch
 from . import _lib
 
 VARIANTS = {"vanilla": 0, "nature": 1, "double": 2}
-# byte offsets of the four frames of s and of s' inside one minibatch sample u8[5][80][80]
-_OFF_S = (C.c_int32 * 4)(0, 6400, 12800, 19200)
-_OFF_N = (C.c_int32 * 4)(6400, 12800, 19200, 25600)
 PRECISIONS = {"fp32": 0, "bf16": 1, "fp16": 2}
-
-
-def _sampled_offsets(frames: torch.Tensor):
-    """channel offsets of s and s' in a minibatch row u8[F][80][80] drawn by the replay: s = frames 0..3, s' = frames F-4..F-1
-    (F = 5: the 1-step row, s' = 1..4; F = 4 + min(n, 4) for n-step returns)"""
-    F = frames.shape[1]
-    if F == 5:
-        return _OFF_S, _OFF_N
-    return _OFF_S, (C.c_int32 * 4)(*[(F - 4 + c) * 6400 for c in range(4)])
 
 
 def truncated_normal_(t: torch.Tensor, std: float, generator=None):
@@ -249,6 +237,30 @@ class QNetwork:
         return actions_out
 
     # ---------------------------------------------------------------- training
+    def _step(self, variant, params, target, frames, actions, rewards, terminals, is_weights, gamma, loss_sum, global_batch, abs_err,
+              q_target, sampling, adam=False, grad_scale=1.0):
+        """fb_qnet_step on (params, target): loss and gradients of the caller's minibatch, or of the one ``sampling`` draws inside
+        the step; with ``adam`` the Adam update of self.params too"""
+        ptr = lambda t: t.data_ptr() if t is not None else None
+        a = _lib.QnetStepArgs(VARIANTS[variant], int(loss_sum), 0, global_batch or 0, float(gamma), params.data_ptr(), target.data_ptr())
+        if sampling is not None:
+            a.sampling = C.addressof(sampling)
+        else:                                   # u8[B][5][80][80]: s = frames 0..3, s' = frames 1..4 of each sample
+            assert frames.shape[1:] == (5, 80, 80) and frames.dtype == torch.uint8 and frames.is_contiguous()
+            a.batch, a.frames_dev, a.sample_stride = frames.shape[0], frames.data_ptr(), 5 * 6400
+            a.chan_off_s[:] = (0, 6400, 12800, 19200)
+            a.chan_off_next[:] = (6400, 12800, 19200, 25600)
+            a.actions_dev, a.rewards_dev, a.terminals_dev = actions.data_ptr(), rewards.data_ptr(), terminals.data_ptr()
+            a.is_weights_dev = ptr(is_weights)
+        a.grads_dev, a.loss_out_dev = self.grads.data_ptr(), self.loss.data_ptr()
+        a.abs_err_out_dev, a.q_target_out_dev = ptr(abs_err), ptr(q_target)
+        if adam:
+            a.m_dev, a.v_dev = self.adam_m.data_ptr(), self.adam_v.data_ptr()
+            a.lr, a.beta1, a.beta2, a.eps, a.grad_scale = self.lr, self.beta1, self.beta2, self.adam_eps, grad_scale
+            a.beta1_power, a.beta2_power = self.beta1_power, self.beta2_power
+        _lib.check(self._L.fb_qnet_step(self._h, C.byref(a), self._stream()), "fb_qnet_step")
+        return self.loss
+
     def loss_backward(self, variant: str, frames: torch.Tensor, actions: torch.Tensor, rewards: torch.Tensor,
                       terminals: torch.Tensor, is_weights: torch.Tensor | None = None, gamma: float = 0.99,
                       loss_sum: bool = False, global_batch: int | None = None, abs_err: torch.Tensor | None = None,
@@ -256,27 +268,10 @@ class QNetwork:
         """frames u8[B][5][80][80]: s = frames 0..3, s' = frames 1..4 of each sample.  Fills self.grads, self.loss.
         ``sampling``: as in train_step -- the minibatch is drawn by the first two kernels of the same graph (u8[B][F][80][80]
         rows for n-step returns, whose targets then come from the replay's R / disc)."""
-        B = frames.shape[0]
-        assert frames.shape[1:] == (5, 80, 80) or (sampling is not None and sampling.n_step > 0 and frames.shape[2:] == (80, 80))
-        assert frames.dtype == torch.uint8 and frames.is_contiguous()
-        off_s, off_n = _OFF_S, _OFF_N
-        ptr = lambda t: t.data_ptr() if t is not None else None
         self._sync_versions()
         p, tg = self._train_weights(variant)        # mu, or the effective weights of update u's draws
-        if sampling is not None:
-            assert frames.data_ptr() == sampling.frames_out_dev and B == sampling.batch and (is_weights is None) == (not sampling.prioritized)
-            off_s, off_n = _sampled_offsets(frames)
-            _lib.check(self._L.fb_qnet_train_step_sampled(
-                self._h, C.addressof(sampling), VARIANTS[variant], p.data_ptr(), tg.data_ptr(), off_s, off_n,
-                global_batch or B, float(gamma), int(loss_sum), self.grads.data_ptr(), self.loss.data_ptr(), ptr(abs_err), ptr(q_target),
-                None, None, 0.0, 0.0, 0.0, 0.0, 1.0, 0.0, 0.0, self._stream()), "fb_qnet_train_step_sampled")
-            return self.loss
-        _lib.check(self._L.fb_qnet_loss_backward(
-            self._h, VARIANTS[variant], p.data_ptr(), tg.data_ptr(), frames.data_ptr(), 5 * 6400,
-            off_s, off_n, actions.data_ptr(), rewards.data_ptr(), terminals.data_ptr(), ptr(is_weights), B,
-            global_batch or B, float(gamma), int(loss_sum), self.grads.data_ptr(), self.loss.data_ptr(), ptr(abs_err),
-            ptr(q_target), self._stream()), "fb_qnet_loss_backward")
-        return self.loss
+        return self._step(variant, p, tg, frames, actions, rewards, terminals, is_weights, gamma, loss_sum, global_batch, abs_err,
+                          q_target, sampling)
 
     def train_step(self, variant: str, frames: torch.Tensor, actions: torch.Tensor, rewards: torch.Tensor, terminals: torch.Tensor,
                    is_weights: torch.Tensor | None = None, gamma: float = 0.99, loss_sum: bool = False, global_batch: int | None = None,
@@ -284,7 +279,8 @@ class QNetwork:
                    sampling=None) -> torch.Tensor:
         """session.run(trainStep) (BrainDQN.py:204-207): loss_backward + adam_step as one library call, bit-identical to the
         two; on the tensor-core path one CUDA graph launch with Adam inside the step's last kernel.  With a peer exchange
-        (several GPUs) the sum over ranks lives in the Adam kernel, so the two calls are made separately.
+        (several GPUs) that is not carried inside the step the sum over ranks lives in the Adam kernel, so the two calls are
+        made separately.
 
         ``sampling`` (``ReplayMemory.step_sampling(batch)[0]``): the minibatch is drawn and gathered by the step's first two
         kernels -- ``random.sample`` and the list comprehensions of BrainDQN.py:197-201 ride in the same graph; ``frames`` /
@@ -292,51 +288,14 @@ class QNetwork:
         hands out u8[B][F][80][80] rows and the step forms the n-step target from its R / disc.
 
         A noisy net: the gradient-only step on the effective weights of update u's draws, then the Adam over (mu, sigma)."""
-        if self.noisy:
+        if self.noisy or (self.exchange is not None and not self.exchange_in_step):
             self.loss_backward(variant, frames, actions, rewards, terminals, is_weights, gamma, loss_sum, global_batch, abs_err, q_target,
                                sampling=sampling)
             self.adam_step(grad_scale)
             return self.loss
-        in_step = self.exchange is None or self.exchange_in_step
-        if sampling is not None and in_step:
-            assert frames.data_ptr() == sampling.frames_out_dev and frames.shape[0] == sampling.batch
-            assert (is_weights is None) == (not sampling.prioritized)
-            off_s, off_n = _sampled_offsets(frames)
-            ptr = lambda t: t.data_ptr() if t is not None else None
-            self._sync_versions()
-            _lib.check(self._L.fb_qnet_train_step_sampled(
-                self._h, C.addressof(sampling), VARIANTS[variant], self.params.data_ptr(), self.target.data_ptr(), off_s, off_n,
-                global_batch or sampling.batch, float(gamma), int(loss_sum), self.grads.data_ptr(), self.loss.data_ptr(), ptr(abs_err),
-                ptr(q_target), self.adam_m.data_ptr(), self.adam_v.data_ptr(), float(self.lr), float(self.beta1), float(self.beta2),
-                float(self.adam_eps), float(grad_scale), float(self.beta1_power), float(self.beta2_power), self._stream()),
-                "fb_qnet_train_step_sampled")
-            self._after_fused_step()
-            return self.loss
-        if sampling is not None:                 # not fusable here: draw the minibatch with its own two launches
-            assert not sampling.prioritized, "with a peer exchange call PrioritizedMemory.sample / batch_update yourself"
-            assert sampling.n_step == 0, "n-step minibatches are drawn inside the training step only"
-            _lib.check(self._L.fb_replay_sample_uniform(sampling.replay, sampling.t, sampling.batch, sampling.setsize, sampling.seed,
-                                                        sampling.idx_out_dev, self._stream()), "fb_replay_sample_uniform")
-            _lib.check(self._L.fb_replay_gather(sampling.replay, sampling.ring_dev, sampling.act_dev, sampling.rew_dev, sampling.term_dev,
-                                                sampling.t, 0, sampling.idx_out_dev, sampling.batch, sampling.frames_out_dev,
-                                                sampling.act_out_dev, sampling.rew_out_dev, sampling.term_out_dev, sampling.env_out_dev,
-                                                sampling.k_out_dev, self._stream()), "fb_replay_gather")
-        if self.exchange is not None and not self.exchange_in_step:
-            self.loss_backward(variant, frames, actions, rewards, terminals, is_weights, gamma, loss_sum, global_batch, abs_err, q_target)
-            self.adam_step(grad_scale)
-            return self.loss
-        B = frames.shape[0]
-        assert frames.shape[1:] == (5, 80, 80) and frames.dtype == torch.uint8 and frames.is_contiguous()
-        off_s, off_n = _OFF_S, _OFF_N
-        ptr = lambda t: t.data_ptr() if t is not None else None
         self._sync_versions()
-        _lib.check(self._L.fb_qnet_train_step(
-            self._h, VARIANTS[variant], self.params.data_ptr(), self.target.data_ptr(), frames.data_ptr(), 5 * 6400,
-            off_s, off_n, actions.data_ptr(), rewards.data_ptr(), terminals.data_ptr(), ptr(is_weights), B,
-            global_batch or B, float(gamma), int(loss_sum), self.grads.data_ptr(), self.loss.data_ptr(), ptr(abs_err),
-            ptr(q_target), self.adam_m.data_ptr(), self.adam_v.data_ptr(), float(self.lr), float(self.beta1), float(self.beta2),
-            float(self.adam_eps), float(grad_scale), float(self.beta1_power), float(self.beta2_power), self._stream()),
-            "fb_qnet_train_step")
+        self._step(variant, self.params, self.target, frames, actions, rewards, terminals, is_weights, gamma, loss_sum, global_batch,
+                   abs_err, q_target, sampling, adam=True, grad_scale=grad_scale)
         self._after_fused_step()
         return self.loss
 

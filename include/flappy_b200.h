@@ -177,11 +177,11 @@ int fb_debug_poison_packed(fb_qnet *net, int slot, void *stream);
 /* measurement hook (tools/write_bw_probe.py): n_chunks chunks of 6,400 bytes at dst + k * stride_bytes, written by one warp each
  * with 16-byte streaming stores (mode 0) or through shared memory + cp.async.bulk (mode 1); no computation */
 int fb_debug_write_probe(uint8_t *dst_dev, int n_chunks, long long stride_bytes, int mode, int ctas, void *stream);
-/* Tensor-core precisions (FB_PRECISION_BF16 / _FP16) only: replay fb_qnet_loss_backward as a CUDA graph once the same arguments were seen twice
+/* Tensor-core precisions (FB_PRECISION_BF16 / _FP16) only: replay fb_qnet_step as a CUDA graph once the same arguments were seen twice
  * (default on; the eager two-stream path is identical work). */
 int fb_qnet_use_graphs(fb_qnet *net, int enable);
 /* Tensor-core precisions only: how conv1 is run (also FB_TC_CONV1_MODE).  4 (default): 3 up to minibatch 512 when the step draws its own
- * minibatch (fb_qnet_train_step_sampled), 2 otherwise (measured).
+ * minibatch (fb_qnet_step with `sampling`), 2 otherwise (measured).
  * 3: the 2x2 max-pool is fused into conv1's epilogue and its input tile is ALWAYS built in the kernel straight from the u8 frames;
  * the 16-bit input matrix X2, which then only the conv1 weight gradient reads, is packed on a side stream beside the forwards.
  * 2: as 3 when no backward pass follows (acting, Q(s')); the training forward materialises X2 first and reads it by TMA.
@@ -207,34 +207,9 @@ int fb_qnet_act(fb_qnet *net, const float *params_dev, const uint8_t *frames_dev
                 const int32_t *chan_off_host4, int batch, double epsilon, uint64_t seed, uint64_t first_env_id,
                 uint32_t *rng_pos_dev, float *q_out_dev, uint8_t *actions_out_dev, void *stream);
 
-/* TD target + loss + backward into grads_dev (not applied).  variant 0 vanilla / 1 Nature target net /
- * 2 Double; the dueling head is a property of the net; is_weights_dev != NULL selects the PER loss.
- * s uses channels chan_off_s, s' uses chan_off_next of the same per-sample block.  loss_sum != 0:
- * sum of squares (BrainDQN.py:162), else mean over global_batch (BrainDQNNature.py:119) so that a
- * sum-allreduce of the gradients of `batch`-sized shards is the gradient of the global mean loss.
- * Outputs (any may be NULL): loss f32[1], abs_err f32[batch] (PER, :247), q_target f32[batch]. */
-int fb_qnet_loss_backward(fb_qnet *net, int variant, const float *params_dev, const float *target_params_dev,
-                          const uint8_t *frames_dev, long long sample_stride, const int32_t *chan_off_s_host4,
-                          const int32_t *chan_off_next_host4, const uint8_t *actions_dev, const float *rewards_dev,
-                          const uint8_t *terminals_dev, const float *is_weights_dev, int batch, int global_batch,
-                          double gamma, int loss_sum, float *grads_dev, float *loss_out_dev, float *abs_err_out_dev,
-                          float *q_target_out_dev, void *stream);
-
 /* One TF-1 ApplyAdam step over the flat vector; alpha = lr*sqrt(1-beta2^t)/(1-beta1^t) from the caller. */
 int fb_qnet_adam(fb_qnet *net, float *params_dev, const float *grads_dev, float *m_dev, float *v_dev, float alpha,
                  float beta1, float beta2, float eps, float grad_scale, void *stream);
-
-/* session.run(trainStep) (BrainDQN.py:204-207) as ONE call: fb_qnet_loss_backward + fb_qnet_adam, bit-identical to the two
- * calls.  beta1_power / beta2_power are the caller's beta^t (TF's beta1_power / beta2_power variables, before this step);
- * alpha = lr*sqrt(1-beta2_power)/(1-beta1_power) in fp32.  With FB_PRECISION_BF16 Adam runs inside the step's last kernel
- * from powers kept in device memory (re-seeded only when they differ from the caller's), so the whole update replays as one
- * CUDA graph launch; params_dev is updated in place, grads_dev / loss_out_dev are still written. */
-int fb_qnet_train_step(fb_qnet *net, int variant, float *params_dev, const float *target_params_dev, const uint8_t *frames_dev,
-                       long long sample_stride, const int32_t *chan_off_s_host4, const int32_t *chan_off_next_host4,
-                       const uint8_t *actions_dev, const float *rewards_dev, const uint8_t *terminals_dev,
-                       const float *is_weights_dev, int batch, int global_batch, double gamma, int loss_sum, float *grads_dev,
-                       float *loss_out_dev, float *abs_err_out_dev, float *q_target_out_dev, float *m_dev, float *v_dev, float lr,
-                       float beta1, float beta2, float eps, float grad_scale, float beta1_power, float beta2_power, void *stream);
 
 /* target_replace_op (BrainDQNNature.py:107-111) */
 int fb_qnet_sync_target(fb_qnet *net, float *target_dev, const float *params_dev, void *stream);
@@ -348,11 +323,12 @@ int fb_per_min_root(fb_replay *r, double *out_dev, void *stream);
 int fb_per_set_global_min(fb_replay *r, const double *global_min_dev);
 int fb_replay_rng_pos(fb_replay *r, uint64_t *pos_host2, int set, void *stream);
 
-/* The minibatch of fb_qnet_train_step drawn INSIDE the step: random.sample + the list comprehensions of BrainDQN.py:197-201
+/* The minibatch of fb_qnet_step drawn INSIDE the step: random.sample + the list comprehensions of BrainDQN.py:197-201
  * (fb_replay_sample_uniform + fb_replay_gather with these arguments) run as the first two kernels of the step, so that on
  * the tensor-core path sampling, gather, forward, backward and Adam are ONE CUDA graph launch; `t` is the only field that
- * changes from step to step and is patched into the two kernel nodes.  frames_out_dev etc. are the minibatch buffers the
- * step then reads (pass the same frames pointer as frames_dev of the step, sample_stride 5*6400, chan_off 0.. / 6400..). */
+ * changes from step to step and is patched into the two kernel nodes (a captured step is matched on the descriptor's bytes,
+ * padding included: zero-fill it before setting the fields).  frames_out_dev etc. are the minibatch buffers the gather fills
+ * (u8[batch][5][80][80]: s = frames 0..3, s' = frames 1..4). */
 typedef struct fb_step_sampling {
     fb_replay *replay;
     const uint8_t *ring_dev, *act_dev; const float *rew_dev; const uint8_t *term_dev;
@@ -376,26 +352,54 @@ typedef struct fb_step_sampling {
      * A transition is drawn once its horizon is complete: the population / SumTree is that of t_eff = t - n_step + 1 (so
      * the caller stores transition t - n + 1 into a prioritized memory at time t).  The frame ring must hold
      * ring_len >= capacity_per_env + n_step + 3 frames (FB_ERR_INVALID otherwise).  frames_out_dev is then
-     * u8[batch][F][80][80], F = 4 + min(n, 4): s = frames 0..3, s' = frames min(n,4)..min(n,4)+3 (chan_off 0.. and
-     * min(n,4)*6400..; sample_stride F*6400); ret_out_dev / disc_out_dev f64[batch] receive R_k and disc_k (required). */
+     * u8[batch][F][80][80], F = 4 + min(n, 4): s = frames 0..3, s' = frames F-4..F-1; ret_out_dev / disc_out_dev f64[batch]
+     * receive R_k and disc_k (required). */
     int n_step;
     double *ret_out_dev, *disc_out_dev;
 } fb_step_sampling;
-/* fb_qnet_train_step with the minibatch drawn first (uniform or prioritized replay).  m_dev == v_dev == NULL: gradients only
- * (fb_qnet_loss_backward with the minibatch drawn first; the caller applies Adam, e.g. through fb_dist_adam).  FB_ERR_INVALID with "Sample larger than population
- * or is negative" when the replay holds fewer than `batch` transitions (random.sample's ValueError). */
-int fb_qnet_train_step_sampled(fb_qnet *net, const fb_step_sampling *sampling, int variant, float *params_dev,
-                               const float *target_params_dev, const int32_t *chan_off_s_host4, const int32_t *chan_off_next_host4,
-                               int global_batch, double gamma, int loss_sum, float *grads_dev, float *loss_out_dev,
-                               float *abs_err_out_dev, float *q_target_out_dev, float *m_dev, float *v_dev, float lr, float beta1,
-                               float beta2, float eps, float grad_scale, float beta1_power, float beta2_power, void *stream);
+
+/* ---- one training step of the Q-network: _trainQNetwork (BrainDQN.py:195-223 and the variants' versions) up to and including
+ * session.run(trainStep) (:204-207).  TD target + loss + backward into grads_dev, then, when m_dev / v_dev are set, one TF-1
+ * Adam step bit-identical to fb_qnet_adam with alpha = lr*sqrt(1-beta2_power)/(1-beta1_power) in fp32; beta1_power /
+ * beta2_power are the caller's beta^t (TF's beta1_power / beta2_power variables, before this step).
+ *   variant       0 vanilla / 1 Nature target net / 2 Double (target_params_dev required for 1 and 2); the dueling head is a
+ *                 property of the net
+ *   loss_sum      != 0: sum of squares (BrainDQN.py:162), else the mean over global_batch (BrainDQNNature.py:119; <= 0: batch),
+ *                 so that a sum-allreduce of the gradients of `batch`-sized shards is the gradient of the global mean loss
+ *   sampling      NULL: the caller's minibatch -- `batch` samples, s = channels chan_off_s, s' = channels chan_off_next of the
+ *                 per-sample block at frames_dev + b*sample_stride, is_weights_dev != NULL selects the PER loss.
+ *                 Non-NULL: the step draws its minibatch first (fb_step_sampling; uniform or prioritized replay), batch is
+ *                 sampling->batch (`batch` 0 or equal), s = frames 0..3 and s' = frames F-4..F-1 of each drawn row, and the
+ *                 caller-minibatch fields (frames_dev .. is_weights_dev) must be 0 / NULL.  FB_ERR_INVALID with "Sample larger
+ *                 than population or is negative" when the replay holds fewer than `batch` transitions (random.sample's
+ *                 ValueError).
+ *   outputs       loss f32[1], abs_err f32[batch] (PER, :247; required with prioritized sampling), q_target f32[batch]; may
+ *                 be NULL otherwise
+ * On the tensor-core precisions Adam runs inside the step's last kernel from powers kept in device memory (re-seeded only when
+ * they differ from the caller's), so the whole step replays as one CUDA graph launch (fb_qnet_use_graphs); params_dev is
+ * updated in place, grads_dev / loss_out_dev are still written.  With an exchange attached (fb_qnet_attach_exchange) Adam
+ * applies the sum of every rank's gradients. */
+typedef struct fb_qnet_step_args {
+    int variant, loss_sum, batch, global_batch;
+    double gamma;
+    float *params_dev; const float *target_params_dev;
+    const fb_step_sampling *sampling;
+    const uint8_t *frames_dev; long long sample_stride; int32_t chan_off_s[4], chan_off_next[4];
+    const uint8_t *actions_dev; const float *rewards_dev; const uint8_t *terminals_dev; const float *is_weights_dev;
+    float *grads_dev, *loss_out_dev, *abs_err_out_dev, *q_target_out_dev;
+    float *m_dev, *v_dev;                           /* both NULL: gradients only; both set: Adam as well */
+    float lr, beta1, beta2, eps, grad_scale, beta1_power, beta2_power;
+} fb_qnet_step_args;
+int fb_qnet_step(fb_qnet *net, const fb_qnet_step_args *args, void *stream);
 
 
 /* ---- test hooks (host only, no device needed): the library's own physics / table / exact-pixel
  * code compiled for the host, so the CPU test-suite can pin it against the oracle. */
 int fb_debug_assets_load_host(const uint8_t *packed_host, size_t n);
-/* sizeof(fb_step_sampling) followed by the byte offset of each field, in declaration order; returns the count written */
-int fb_debug_step_sampling_layout(int32_t *out, int capacity);
+/* sizeof(S) followed by the byte offset of each field of S, in declaration order, for S = fb_step_sampling (which 0) or
+ * fb_qnet_step_args (which 1); returns the count written */
+int fb_debug_struct_layout(int which, int32_t *out, int capacity);
+int fb_debug_step_sampling_layout(int32_t *out, int capacity);     /* fb_debug_struct_layout(0, out, capacity) */
 int fb_debug_host_reset(int32_t *state16, const uint8_t *gaps, int gaps_len, uint64_t seed, uint64_t env_id);
 int fb_debug_host_step(int32_t *state16, int action, const uint8_t *gaps, int gaps_len, uint64_t seed,
                        uint64_t env_id, float *reward, uint8_t *terminal, int32_t *score);

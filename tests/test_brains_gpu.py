@@ -191,9 +191,10 @@ def test_driver_loop_single_env_and_bad_model(mods):
 
 @pytest.mark.parametrize("model", ["dqn", "ddqn", "duelingdqn", "prioritydqn"])
 def test_sampling_inside_the_step_is_identical_to_separate_launches(mods, model):
-    """fb_qnet_train_step_sampled: random.sample + gather as the first two kernels of the update's CUDA graph (their `t`
+    """fb_qnet_step with `sampling`: random.sample + gather as the first two kernels of the update's CUDA graph (their `t`
     patched into the graph nodes every step) -- same minibatches, same parameters, same stream positions as
-    fb_replay_sample_uniform + fb_replay_gather + fb_qnet_train_step, while the replay fills, wraps and the graph replays"""
+    fb_replay_sample_uniform + fb_replay_gather + fb_qnet_step on that minibatch, while the replay fills, wraps and the graph
+    replays"""
     game, brains = mods
     N = 48
     runs = []

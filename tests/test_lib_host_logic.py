@@ -158,14 +158,21 @@ def test_invalid_action_is_rejected(L):
     assert b"Multiple input actions" in L.fb_last_error()
 
 
-def test_step_sampling_struct_matches_the_c_layout():
-    """the ctypes mirror of fb_step_sampling (the descriptor handed to fb_qnet_train_step_sampled) against the compiled struct"""
-    import ctypes as C
-    from dqnflappybird_b200 import _lib
-    out = (C.c_int32 * 32)()
-    n = _lib.lib().fb_debug_step_sampling_layout(out, 32)
-    fields = _lib.StepSampling._fields_
+def _check_layout(mirror, out, n):
+    fields = mirror._fields_
     assert n == 1 + len(fields)
-    assert out[0] == C.sizeof(_lib.StepSampling)
+    assert out[0] == C.sizeof(mirror)
     for k, (name, _) in enumerate(fields):
-        assert out[1 + k] == getattr(_lib.StepSampling, name).offset, name
+        assert out[1 + k] == getattr(mirror, name).offset, name
+
+
+def test_step_sampling_struct_matches_the_c_layout():
+    """the ctypes mirror of fb_step_sampling (the sampling descriptor handed to fb_qnet_step) against the compiled struct"""
+    out = (C.c_int32 * 32)()
+    _check_layout(_lib.StepSampling, out, _lib.lib().fb_debug_step_sampling_layout(out, 32))
+
+
+def test_qnet_step_args_struct_matches_the_c_layout():
+    """the ctypes mirror of fb_qnet_step_args (the descriptor of fb_qnet_step) against the compiled struct"""
+    out = (C.c_int32 * 64)()
+    _check_layout(_lib.QnetStepArgs, out, _lib.lib().fb_debug_struct_layout(1, out, 64))

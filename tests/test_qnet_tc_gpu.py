@@ -263,8 +263,8 @@ def test_training_steps_track_the_strict_path(mods):
 @pytest.mark.parametrize("precision,variant,dueling", [("bf16", "nature", False), ("bf16", "double", True), ("bf16", "vanilla", False),
                                                        ("fp32", "nature", False)])
 def test_train_step_is_loss_backward_plus_adam(mods, precision, variant, dueling):
-    """fb_qnet_train_step (Adam inside the step's last kernel, alpha from beta powers in device memory, one CUDA graph) is
-    bit-identical to fb_qnet_loss_backward + fb_qnet_adam, over graph capture / replay and when the two forms are mixed"""
+    """fb_qnet_step with Adam (inside the step's last kernel, alpha from beta powers in device memory, one CUDA graph) is
+    bit-identical to the gradient-only fb_qnet_step + fb_qnet_adam, over graph capture / replay and when the two forms are mixed"""
     _lib, game, qnet = mods
     B = 64
     frames = _env_frames(game, B, 21)
@@ -512,3 +512,116 @@ def test_fp16_forward_and_training_step(mods):
     cos = (u0 @ u1 / (u0.norm() * u1.norm())).item()
     assert u1.abs().max().item() > 5e-6 and cos > 0.995, cos
     assert abs(nets[0].loss.item() - nets[1].loss.item()) <= 4e-3 * abs(nets[1].loss.item())
+
+
+def _memory(game, replay, N, C, B, steps, prioritized=False):
+    """a replay memory filled by `steps` random-action env steps: the same arguments give the same contents and the same draws"""
+    ring = torch.zeros((N, C + 4, 80, 80), dtype=torch.uint8, device="cuda")
+    mem = replay.PrioritizedMemory(ring, C, seed=7, max_batch=B) if prioritized else replay.ReplayMemory(ring, C, seed=7, max_batch=B)
+    gs = game.GameState(num_envs=N, seed=3, history=mem.L, ring=mem.ring)
+    gs.frame_step(torch.zeros(N, dtype=torch.uint8, device="cuda"))
+    for k in range(1, steps + 1):
+        a, r, t = mem.rows(k)
+        gs.step_random(1, 0.5, 21, a, r, t, None)
+        mem.appended(k)
+    return mem
+
+
+# one argument of the training step changed from BASE at a time: a captured graph that ignored it would be replayed for it
+BASE = dict(variant="nature", gamma=0.99, loss_sum=False, global_batch=None, outputs=True, grad_scale=1.0)
+CHANGES = [dict(gamma=0.9), dict(loss_sum=True), dict(global_batch=64), dict(variant="double"), dict(outputs=False),
+           dict(grad_scale=0.5)]
+
+
+@pytest.mark.parametrize("sampled", [False, True])
+def test_graph_replay_honours_every_argument(mods, sampled):
+    """fp16, graphs on: every configuration is called three times (eager, capture, replay), then once more each after all were
+    captured (replay), and after every call the net is bit-identical to a twin that never uses graphs -- the captured step is
+    keyed on all of its arguments, so a changed argument never replays a graph captured for another value"""
+    _lib, game, qnet = mods
+    from dqnflappybird_b200 import replay
+    B = 32
+    graph, eager = nets = [qnet.QNetwork(max_batch=B, seed=3, precision="fp16", lr=1e-4) for _ in range(2)]
+    _lib.check(_lib.lib().fb_qnet_use_graphs(eager._h, 0), "fb_qnet_use_graphs")
+    for n in nets:
+        n.params.mul_(3.0); n.target.mul_(3.0)
+    if sampled:
+        mems = [_memory(game, replay, 48, 20, B, 30) for _ in nets]
+    else:
+        frames = _env_frames(game, B, 21)
+        rng = np.random.default_rng(5)
+        a = torch.from_numpy(rng.integers(0, 2, B).astype(np.uint8)).cuda()
+        r = torch.from_numpy(rng.choice(np.array([0.1, 3.0, -3.0], np.float32), B)).cuda()
+        term = (r == -3.0).to(torch.uint8)
+    outs = [(torch.zeros(B, device="cuda"), torch.zeros(B, device="cuda")) for _ in nets]
+    p0 = graph.params.clone()
+    bits = lambda x: x.view(torch.int32)                               # bitwise, NaN included
+    configs = [BASE] + [{**BASE, **c} for c in CHANGES]
+    calls = [cfg for cfg in configs for _ in range(3)] + configs
+    for k, cfg in enumerate(calls):
+        for i, n in enumerate(nets):
+            sp = None
+            if sampled:
+                sp, mb = mems[i].step_sampling(B)
+                frames, a, r, term = mb.frames, mb.actions, mb.rewards, mb.terminals
+            abs_err, y = outs[i] if cfg["outputs"] else (None, None)
+            n.train_step(cfg["variant"], frames, a, r, term, None, cfg["gamma"], cfg["loss_sum"], cfg["global_batch"], abs_err, y,
+                         cfg["grad_scale"], sampling=sp)
+        for name in ("loss", "grads", "params", "adam_m", "adam_v"):
+            assert torch.equal(bits(getattr(graph, name)), bits(getattr(eager, name))), (k, cfg, name)
+        # (without outputs the buffers keep the last call's values: a replay that still wrote them would show here)
+        assert torch.equal(bits(outs[0][0]), bits(outs[1][0])) and torch.equal(bits(outs[0][1]), bits(outs[1][1])), (k, cfg)
+        if sampled:
+            assert torch.equal(mems[0]._idx[:B], mems[1]._idx[:B]), (k, cfg)
+    assert graph.adam_steps == len(calls) and torch.isfinite(graph.params).all() and not torch.equal(graph.params, p0)
+
+
+@pytest.mark.parametrize("precision", ["fp32", "fp16"])
+def test_step_rejects_bad_arguments(mods, precision):
+    """fb_qnet_step validates its descriptor once, for both precisions: FB_ERR_INVALID for a missing pointer, a batch outside
+    1..max_batch, a bad variant or a missing target, half of the Adam slots, prioritized replay without abs_err_out_dev, and
+    caller-minibatch fields set together with `sampling`"""
+    _lib, game, qnet = mods
+    from dqnflappybird_b200 import replay
+    L = _lib.lib()
+    B = 8
+    net = qnet.QNetwork(max_batch=B, precision=precision)
+    frames = torch.zeros((B, 5, 80, 80), dtype=torch.uint8, device="cuda")
+    a, r, t = torch.zeros(B, dtype=torch.uint8, device="cuda"), torch.zeros(B, device="cuda"), torch.zeros(B, dtype=torch.uint8, device="cuda")
+    abs_err = torch.zeros(B, device="cuda")
+
+    def step(sampling=None, **kw):
+        d = _lib.QnetStepArgs(variant=1, gamma=0.99, params_dev=net.params.data_ptr(), target_params_dev=net.target.data_ptr(),
+                              grads_dev=net.grads.data_ptr(), loss_out_dev=net.loss.data_ptr())
+        if sampling is None:
+            d.batch, d.frames_dev, d.sample_stride = B, frames.data_ptr(), 5 * 6400
+            d.chan_off_s[:] = (0, 6400, 12800, 19200)
+            d.chan_off_next[:] = (6400, 12800, 19200, 25600)
+            d.actions_dev, d.rewards_dev, d.terminals_dev = a.data_ptr(), r.data_ptr(), t.data_ptr()
+        else:
+            d.sampling = C.addressof(sampling)
+        for k, v in kw.items():
+            setattr(d, k, v)
+        rc = L.fb_qnet_step(net._h, C.byref(d), net._stream())
+        assert rc == 0 or b"fb_qnet_step" in L.fb_last_error(), L.fb_last_error()
+        return rc
+
+    assert step() == 0 and step(variant=0, target_params_dev=None) == 0
+    assert step(m_dev=net.adam_m.data_ptr(), v_dev=net.adam_v.data_ptr(), lr=1e-6, beta1=0.9, beta2=0.999, eps=1e-8, grad_scale=1.0,
+                beta1_power=0.9, beta2_power=0.999) == 0
+    for bad in (dict(params_dev=None), dict(grads_dev=None), dict(frames_dev=None), dict(actions_dev=None), dict(rewards_dev=None),
+                dict(terminals_dev=None), dict(batch=0), dict(batch=B + 1), dict(variant=3), dict(variant=-1),
+                dict(target_params_dev=None), dict(variant=2, target_params_dev=None), dict(m_dev=net.adam_m.data_ptr()),
+                dict(v_dev=net.adam_v.data_ptr())):
+        assert step(**bad) == -1, bad
+    mem = _memory(game, replay, 4, 8, B, 6)
+    sp, _ = mem.step_sampling(B)
+    assert step(sp) == 0 and step(sp, batch=B) == 0
+    for bad in (dict(frames_dev=frames.data_ptr()), dict(sample_stride=5 * 6400), dict(actions_dev=a.data_ptr()),
+                dict(rewards_dev=r.data_ptr()), dict(terminals_dev=t.data_ptr()), dict(is_weights_dev=r.data_ptr()),
+                dict(chan_off_next=(C.c_int32 * 4)(0, 0, 0, 6400)), dict(batch=B - 1)):
+        assert step(sp, **bad) == -1, bad
+    pmem = _memory(game, replay, 4, 8, B, 6, prioritized=True)
+    psp, _ = pmem.step_sampling(B)
+    assert step(psp) == -1 and step(psp, abs_err_out_dev=abs_err.data_ptr()) == 0
+    torch.cuda.synchronize()
