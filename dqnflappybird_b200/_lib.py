@@ -129,8 +129,6 @@ _SIGNATURES = {
     "fb_debug_poison_packed": ([_vp, C.c_int, _vp], C.c_int),
     "fb_debug_write_probe": ([_vp, C.c_int, C.c_longlong, C.c_int, C.c_int, _vp], C.c_int),
     "fb_qnet_use_graphs": ([_vp, C.c_int], C.c_int),
-    "fb_qnet_set_conv1_mode": ([_vp, C.c_int], C.c_int),
-    "fb_qnet_set_fused_backward": ([_vp, C.c_int], C.c_int),
     "fb_qnet_param_count": ([_vp], C.c_int),
     "fb_qnet_layout": ([_vp, _i32p], C.c_int),
     "fb_qnet_forward": ([_vp, _f32p, _u8p, C.c_longlong, _i32p, C.c_int, _f32p, _vp], C.c_int),
@@ -178,6 +176,7 @@ _SIGNATURES = {
     "fb_debug_host_mixed": ([_i32p], C.c_int),
     "fb_debug_tc_mma_rate": ([C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _vp, _vp], C.c_int),
     "fb_debug_tc_kernel": ([_vp, C.c_int, C.c_int, C.c_int, _f32p, _vp], C.c_int),
+    "fb_debug_tc_separate_kernels": ([_vp, C.c_int], C.c_int),
     "fb_debug_tc_slab": ([C.c_int, C.c_int, _vp, _vp, _f32p, _vp], C.c_int),
     "fb_debug_tc_gemm": ([C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _vp, _vp, _f32p, _vp, _vp], C.c_int),
 }

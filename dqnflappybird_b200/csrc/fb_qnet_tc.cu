@@ -21,7 +21,6 @@
 // head / TD loss / Adam in fp32 (shared with fb_qnet.cu).  Tolerances vs the float64 oracle: tests/test_qnet_tc_gpu.py.
 #include <cudaTypedefs.h>
 
-#include <stdlib.h>
 #include <string.h>
 
 #include <map>
@@ -238,19 +237,6 @@ __device__ __forceinline__ void load_bias16(const float *bs, int col, float (&b)
         b[4 * k] = t4.x; b[4 * k + 1] = t4.y; b[4 * k + 2] = t4.z; b[4 * k + 3] = t4.w;
     }
 }
-struct EpiConv1 {               // rows on the 21-grid -> Z1 [B*441][32] = relu(conv + b), zeros at invalid positions
-    bf16 *z1; const float *bias; int rows, f16;
-    __device__ void operator()(int row, int col, float (&v)[16], int, const float *bs) const {
-        float b[16];
-        load_bias16(bs, col, b);
-        if (row >= rows) return;
-        int p = row % kP1;
-        const float keep = ((p / kG1) < 20 && (p % kG1) < 20) ? 1.f : 0.f;
-#pragma unroll
-        for (int i = 0; i < 16; i++) v[i] = fmaxf(v[i] + b[i], 0.f) * keep;
-        store_bf16x16(z1 + (size_t)row * kC1 + col, v, f16);
-    }
-};
 struct EpiGrid7 {               // conv2: rows on the 7-grid -> A2 [B*49][64], zeros at invalid positions
     bf16 *out; const float *bias; int rows, f16;
     __device__ void operator()(int row, int col, float (&v)[16], int, const float *bs) const {
@@ -353,29 +339,6 @@ __global__ void pack_x2_kernel(FrameView fv, int B, bf16 *x2, int f16) {
 #pragma unroll
         for (int h = 0; h < 2; h++) w[s * 2 + h] = tc::pack2(px[s][2 * h], px[s][2 * h + 1], f16);
     *reinterpret_cast<uint4 *>(x2 + blk * 64 + r * 16 + sp * 8) = make_uint4(w[0], w[1], w[2], w[3]);
-}
-
-__device__ __forceinline__ uint4 bf16x8_max(uint4 a, uint4 b, int f16) {
-    return make_uint4(tc::max2(a.x, b.x, f16), tc::max2(a.y, b.y, f16), tc::max2(a.z, b.z, f16), tc::max2(a.w, b.w, f16));
-}
-
-// max_pool 2x2 (BrainDQN.py:128) + space-to-depth for conv2: Z1 (21-grid) -> P2 [B*49][128], channel j = r*64 + s*32 + c
-__global__ void pool_pack_kernel(const bf16 *z1, int B, bf16 *p2, int f16) {
-    tc::pdl_wait();
-    tc::pdl_launch();
-    size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= (size_t)B * 36 * 16) return;
-    int cg = (int)(t & 3), rs = (int)((t >> 2) & 3);
-    size_t blk = t >> 4;
-    int b = (int)(blk / 36), q = (int)(blk - (size_t)b * 36), bh = q / 6, bw = q - bh * 6;
-    int r = rs >> 1, s = rs & 1;
-    int ph = 2 * bh - 1 + r, pw = 2 * bw - 1 + s;
-    uint4 m = make_uint4(0, 0, 0, 0);
-    if ((unsigned)ph < 10u && (unsigned)pw < 10u) {
-        const uint4 *src = reinterpret_cast<const uint4 *>(z1 + ((size_t)b * kP1 + (2 * ph) * kG1 + 2 * pw) * kC1 + cg * 8);
-        m = bf16x8_max(bf16x8_max(__ldg(src), __ldg(src + 4), f16), bf16x8_max(__ldg(src + kG1 * 4), __ldg(src + kG1 * 4 + 4), f16), f16);
-    }
-    *reinterpret_cast<uint4 *>(p2 + ((size_t)b * kP2 + bh * kG2 + bw) * 128 + r * 64 + s * 32 + cg * 8) = m;
 }
 
 // eight channels of one pooling window: g = gradient of the pooled value, z[k] = the window's four activations (k = row-major
@@ -1431,7 +1394,7 @@ struct TcPlan {                 // everything that depends on the batch size
     CUtensorMap x2_w, p2_w, a2_w, a3_m;                              // weight-gradient A operands (workspace 0)
     CUtensorMap dz1_b, dz2_b, dz3_b, dh1_b;                          // weight-gradient B operands, 64 rows
     GemmParams fc1, fc1_d, fc1_w;
-    ConvParams conv1, conv2, conv3, conv3_d, conv2_d;
+    ConvParams conv2, conv3, conv3_d, conv2_d;
     WgradParams conv1_w, conv2_w, conv3_w;
     int s1, s2, s3, sf;                                              // split-K counts (conv weight gradients, fc1 forward)
 };
@@ -1449,6 +1412,9 @@ static void destroy_entry(GraphEntry &g) {
     if (g.graph) cudaGraphDestroy(g.graph);
     g.exec = nullptr; g.graph = nullptr;
 }
+// TcState::ev: a training step takes the running slots [0, kEvGather) in order, one per cross-stream edge; the named slots
+// after them have fixed uses (the replay gather and the early X2 conversion of a step, the two streams of chunked acting)
+constexpr int kEvGather = 12, kEvX2 = 13, kEvChunkIn = 14, kEvChunkOut = 15, kEvSlots = 16;
 struct TcState {
     FwdWs ws[2];                // 0: the online net on s (kept for backward); 1: the other forwards, concurrently
     bf16 *dh1, *dz3, *dz2, *dp2, *dz1;
@@ -1470,20 +1436,12 @@ struct TcState {
     cudaStream_t aux4;          // fifth stream: Memory.batch_update (prioritized replay) beside the whole backward pass
     cudaStream_t aux3;          // fourth stream (several GPUs): W_fc1's bucket of the gradient exchange, joined only at the step's end
     cudaStream_t cap;           // capture origin (the caller's stream may be the legacy default stream, which cannot capture)
-    cudaEvent_t ev[16];
+    cudaEvent_t ev[kEvSlots];
     std::vector<GraphEntry> graphs;
     int use_graph;
     int f16;                    // operand format of every 16-bit tensor of this net: 0 bf16, 1 fp16 (FB_PRECISION_FP16)
-    int fuse_fwd;               // 1 (default): conv2 + conv3 forward as one kernel (also FB_TC_FUSE_FWD)
-    int nopdl;                  // mask (FB_TC_NOPDL) of update kernels launched WITHOUT the early (programmatic) launch.  Default 1: the conv1
-                                // weight gradient -- launched early, its 147 CTAs sat on SMs waiting for the fused data-gradient kernel while
-                                // the conv3 weight gradient, which was ready, queued behind them (121 -> 114.5 us per update, measured).
-                                // 2: fused backward, 4 / 8: conv3 / conv2 weight gradient, 16: finalize -- all measured slower or equal
-    int fuse_bwd;               // 1 (default): conv3 / conv2 data gradients and the un-pool as one kernel (also FB_TC_FUSE_BWD)
-    int step_samples;           // set by train_step_launch around its forwards: the step draws its own minibatch (replay sampling inside)
-    int conv1_mode;             // 4 (default): 3 up to minibatch 512 when the step samples its own minibatch, else 2.  3: conv1 from the u8 frames in the training forward too, X2
-                                // (only the conv1 weight gradient reads it) packed beside the forwards; 2: pooled epilogue, slab from u8
-                                // when no backward follows; 1: slab always from X2; 0: separate pack_x2 / conv1 / pool_pack kernels
+    int separate_kernels;       // test hook (fb_debug_tc_separate_kernels): no fused conv2+conv3 forward / conv3-conv2 backward at any batch
+    FrameView probe_view;       // frames of this net's last forward (fb_debug_tc_kernel's conv1 probes re-read them)
 };
 
 namespace {
@@ -1536,8 +1494,6 @@ int make_plan(fb_qnet *n, int B, TcPlan **out) {
     MAP(dz1_b, t->dz1, P1, 32, 32, 64); MAP(dz2_b, t->dz2, P2, 64, 64, 64); MAP(dz3_b, t->dz3, P2, 64, 64, 64); MAP(dh1_b, t->dh1, B, H, 64, 64);
 #undef MAP
     // ---- forward: tap (dh,dw) of K-block kb = row offset inside the slab
-    p.conv1.n_tiles = (int)((P1 + 127) / 128); p.conv1.slab_row0 = 0;
-    for (int k = 0; k < 4; k++) { p.conv1.kb_rowoff[k] = (k >> 1) * kG1 + (k & 1); p.conv1.kb_half[k] = 0; }
     p.conv2.n_tiles = (int)((P2 + 127) / 128); p.conv2.slab_row0 = 0;
     for (int k = 0; k < 8; k++) { int tp = k >> 1; p.conv2.kb_rowoff[k] = (tp >> 1) * kG2 + (tp & 1); p.conv2.kb_half[k] = k & 1; }
     p.conv3.n_tiles = p.conv2.n_tiles; p.conv3.slab_row0 = -8;                  // pad ring = the row before / after: offset -8
@@ -1582,7 +1538,7 @@ int make_plan(fb_qnet *n, int B, TcPlan **out) {
     set_mnmajor(p.fc1_w, 128); p.fc1_w.p_total = B; p.fc1_w.klen = (B + 63) / 64 * 64;
     for (int mt = 0; mt < 13; mt++) for (int i = 0; i < 2; i++) { p.fc1_w.a2_rowoff[mt][i] = 0; p.fc1_w.a2_col[mt][i] = mt * 128 + i * 64; }
     FB_REQUIRE((size_t)p.s1 <= t->cap1 && (size_t)p.s2 <= t->cap2 && (size_t)p.s3 <= t->cap3, "tensor-core path: split-K workspace too small");
-    p.conv1.f16 = p.conv2.f16 = p.conv3.f16 = p.conv3_d.f16 = p.conv2_d.f16 = t->f16;
+    p.conv2.f16 = p.conv3.f16 = p.conv3_d.f16 = p.conv2_d.f16 = t->f16;
     p.conv1_w.f16 = p.conv2_w.f16 = p.conv3_w.f16 = t->f16;
     p.fc1.f16 = p.fc1_d.f16 = p.fc1_w.f16 = t->f16;
     auto res = t->plans.emplace(B, p);
@@ -1661,10 +1617,6 @@ int tc_state_create(fb_qnet *n) {
     }
     for (auto &e : t->ev) FB_CUDA_OK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     t->use_graph = 1;
-    { const char *e = getenv("FB_TC_FUSE_BWD"); t->fuse_bwd = (e && e[0] == '0') ? 0 : 1; }
-    { const char *e = getenv("FB_TC_FUSE_FWD"); t->fuse_fwd = (e && e[0] == '0') ? 0 : 1; }
-    { const char *e = getenv("FB_TC_CONV1_MODE"); t->conv1_mode = (e && e[0] >= '0' && e[0] <= '4') ? e[0] - '0' : 4; }
-    { const char *e = getenv("FB_TC_NOPDL"); t->nopdl = e ? atoi(e) : 1; }
     n->tc = t;
     return FB_OK;
 }
@@ -1745,24 +1697,18 @@ int tc_slot_for(fb_qnet *n, const float *params_dev, int want_slot, cudaStream_t
     return FB_OK;
 }
 
-// the conv1 path in effect at this minibatch: measured, mode 3 wins up to 512 samples (100.9 vs 102.9 us per update at 256) and
-// loses above (1,024: 235 vs 213 us; 4,096: 689 vs 635 us -- the u8 path is bound by shared memory, the X2 path by HBM)
-// (and only when the step draws its own minibatch: the replay gather ahead of the X2 conversion on their side stream keeps the
-// conversion's 3,528 CTAs out of the way of the two conv1 launches; on a caller-supplied minibatch 3 costs 105 vs 98 us)
-static inline int conv1_mode_at(const TcState *t, int B) {
-    return t->conv1_mode == 4 ? (B <= kFuseMaxBatch && t->step_samples ? 3 : 2) : t->conv1_mode;
-}
-static FrameView g_probe_view;                    // frames of the last forward (the fused conv1 probe re-reads them)
-// keep != 0: this forward's activations feed a backward pass (Z1 and, for the conv1 weight gradient, X2 are written)
-// td != nullptr: the TD target / loss is fused into the head kernel; `join` (if any) is waited for first -- it marks the end
-// of the Q(s') forward on the other stream
-static int tc_forward_impl(fb_qnet *n, int slot, int w, const float *params_dev, FrameView fv, int B, float *q_out, int keep, cudaStream_t st,
-                           const TdFuse *td = nullptr, cudaEvent_t join = nullptr, const AdamPow *ap = nullptr, float gscale = 1.f);
-int tc_forward(fb_qnet *n, int slot, int w, const float *params_dev, FrameView fv, int B, float *q_out, cudaStream_t st) {
-    return tc_forward_impl(n, slot, w, params_dev, fv, B, q_out, 0, st);
-}
-static int tc_forward_impl(fb_qnet *n, int slot, int w, const float *params_dev, FrameView fv, int B, float *q_out, int keep, cudaStream_t st,
-                           const TdFuse *td, cudaEvent_t join, const AdamPow *ap, float gscale) {
+// The training forward on s (train_step_launch): its activations feed the backward pass (Z1, A2, h1 and, for the conv1 weight
+// gradient, X2 are kept), and its head kernel also forms the TD target / loss -- after waiting for `join`, the end of the Q(s')
+// forward on the other stream.  nullptr: a forward with no backward pass (acting, Q(s')).
+struct TrainFwd {
+    TdFuse td;
+    cudaEvent_t join;
+    AdamPow ap;
+    float gscale;               // power of two carried by the gradient tensors (GradFmt)
+    bool x2_early;              // conv1 from the u8 frames, X2 packed early by the caller; else X2 is packed here and feeds conv1
+};
+static int run_forward(fb_qnet *n, int slot, int w, const float *params_dev, FrameView fv, int B, float *q_out, const TrainFwd *tr,
+                       cudaStream_t st) {
     TcState *t = n->tc;
     FB_REQUIRE(t != nullptr && B > 0 && B <= n->max_batch && (w == 0 || w == 1), "tc_forward: bad argument");
     TcPlan *p;
@@ -1772,25 +1718,19 @@ static int tc_forward_impl(fb_qnet *n, int slot, int w, const float *params_dev,
     const TcWeightMaps &wm = t->wm[slot];
     const FwdWs &f = t->ws[w];
     const int P1 = B * kP1, P2 = B * kP2;
-    g_probe_view = fv;
-    // conv1 with the 2x2 max-pool in its epilogue (Z1 is written only when a backward pass needs it; no pooling pass):
-    //   keep == 0 (acting, Q(s') forwards): slab built in the kernel straight from the u8 frames -- no X2 either;
-    //   keep != 0: X2 is materialised once (the conv1 weight gradient contracts over it by TMA) and feeds the slab.
-    // conv1_mode 0 restores the three separate kernels (pack_x2, conv1, pool_pack).
-    const int c1mode = conv1_mode_at(t, B);
-    if (c1mode == 0) {
+    const bool keep = tr != nullptr;
+    t->probe_view = fv;
+    // conv1 with the 2x2 max-pool in its epilogue (Z1 is written only when a backward pass needs it; no pooling pass), its slab
+    // built in the kernel straight from the u8 frames -- except in a training forward without x2_early: there X2 is materialised
+    // once (the conv1 weight gradient contracts over it by TMA) and feeds the slab
+    const Conv1FusedParams c1{fv, B, params_dev + L.b1, keep ? f.z1 : nullptr, f.p2, t->f16};
+    if (keep && !tr->x2_early) {
         FB_CUDA_OK(tc::launch_pdl(pack_x2_kernel, dim3((unsigned)(((size_t)P1 * 8 + 255) / 256)), dim3(256), 0, st, fv, B, f.x2, t->f16));
-        FB_CUDA_OK((launch_tc_conv<32, kSlab1, 1, 4, 6, 1>(p->x2_s[w], wm.w1p, p->conv1, t->n_sms, EpiConv1{f.z1, params_dev + L.b1, P1, t->f16}, st)));
-        FB_CUDA_OK(tc::launch_pdl(pool_pack_kernel, dim3((unsigned)(((size_t)B * 36 * 16 + 255) / 256)), dim3(256), 0, st, f.z1, B, f.p2, t->f16));
-    } else if ((keep && c1mode != 3) || c1mode == 1) {
-        FB_CUDA_OK(tc::launch_pdl(pack_x2_kernel, dim3((unsigned)(((size_t)P1 * 8 + 255) / 256)), dim3(256), 0, st, fv, B, f.x2, t->f16));
-        FB_CUDA_OK((launch_tc_conv1_fused<6, true>(p->x2_s[w], wm.w1p, Conv1FusedParams{fv, B, params_dev + L.b1, keep ? f.z1 : nullptr, f.p2, t->f16},
-                                                  t->n_sms, st)));
+        FB_CUDA_OK((launch_tc_conv1_fused<6, true>(p->x2_s[w], wm.w1p, c1, t->n_sms, st)));
     } else {
-        // (mode 3 with keep: Z1 is written here too; X2, which only the conv1 weight gradient reads, is packed off the critical path)
-        FB_CUDA_OK((launch_tc_conv1_fused<4, false>(p->x2_s[w], wm.w1p, Conv1FusedParams{fv, B, params_dev + L.b1, keep ? f.z1 : nullptr, f.p2, t->f16}, t->n_sms, st)));
+        FB_CUDA_OK((launch_tc_conv1_fused<4, false>(p->x2_s[w], wm.w1p, c1, t->n_sms, st)));
     }
-    if (t->fuse_fwd && B <= kFuseMaxBatch) {
+    if (B <= kFuseMaxBatch && !t->separate_kernels) {
         FB_CUDA_OK((launch_tc_fwd23<2>(p->p2_s[w], wm.w2p, wm.w3p, Fwd23Params{(B + 1) / 2, B, params_dev + L.b2, params_dev + L.b3, keep ? f.a2 : nullptr, f.a3, t->f16},
                                        t->n_sms, st)));
     } else {
@@ -1799,19 +1739,22 @@ static int tc_forward_impl(fb_qnet *n, int slot, int w, const float *params_dev,
     }
     FB_CUDA_OK((launch_tc_gemm<128, 2>(p->a3_k[w], wm.wf1n, p->fc1, dim3((B + 127) / 128, L.hidden / 128, p->sf),
                                        EpiStoreF32{f.parth, B, L.hidden, (size_t)n->max_batch * L.hidden}, st)));
-    if (join) FB_CUDA_OK(cudaStreamWaitEvent(st, join, 0));
-    TdFuse none{};
-    if (td != nullptr && ap != nullptr && fused_head_ok(L))      // training step: head forward + TD loss + head backward in one kernel
+    if (keep) FB_CUDA_OK(cudaStreamWaitEvent(st, tr->join, 0));
+    if (keep && fused_head_ok(L))              // training step: head forward + TD loss + head backward in one kernel
         FB_CUDA_OK(tc::launch_pdl(fc1_head_train_kernel<16>, dim3(head_ctas(t, B)), dim3(128), 0, st, f.parth, p->sf,
-                                  (size_t)n->max_batch * L.hidden, params_dev, L, B, q_out, *td, HeadBwd{t->dh1, t->hp, t->hb, GradFmt{t->f16, gscale}}, *ap));
-    else if (td == nullptr && fused_head_ok(L)) {
+                                  (size_t)n->max_batch * L.hidden, params_dev, L, B, q_out, tr->td, HeadBwd{t->dh1, t->hp, t->hb, GradFmt{t->f16, tr->gscale}},
+                                  tr->ap));
+    else if (!keep && fused_head_ok(L)) {
         const int ctas = (B + 3) / 4 < 4 * t->n_sms ? (B + 3) / 4 : 4 * t->n_sms;
         FB_CUDA_OK(tc::launch_pdl(fc1_head_warp_kernel<16>, dim3(ctas), dim3(128), 0, st, f.parth, p->sf, (size_t)n->max_batch * L.hidden,
-                                  params_dev, L, B, keep ? f.h1 : nullptr, q_out));
+                                  params_dev, L, B, (float *)nullptr, q_out));
     } else
         FB_CUDA_OK(tc::launch_pdl(fc1_head_kernel, dim3(B), dim3(128), 0, st, f.parth, p->sf, (size_t)n->max_batch * L.hidden, params_dev, L, B,
-                                  keep ? f.h1 : nullptr, q_out, td ? *td : none));
+                                  keep ? f.h1 : nullptr, q_out, keep ? tr->td : TdFuse{}));
     return FB_OK;
+}
+int tc_forward(fb_qnet *n, int slot, int w, const float *params_dev, FrameView fv, int B, float *q_out, cudaStream_t st) {
+    return run_forward(n, slot, w, params_dev, fv, B, q_out, nullptr, st);
 }
 
 // Acting over more samples than one workspace holds: chunks alternate between the two forward workspaces and the two
@@ -1822,7 +1765,7 @@ int tc_forward_chunks(fb_qnet *n, int slot, const float *params_dev, const uint8
     FB_REQUIRE(t != nullptr, "tc_forward_chunks: no tensor-core state");
     const int nchunks = (batch + n->max_batch - 1) / n->max_batch;
     const bool two = nchunks > 1;
-    if (two) { FB_CUDA_OK(cudaEventRecord(t->ev[14], st)); FB_CUDA_OK(cudaStreamWaitEvent(t->aux, t->ev[14], 0)); }
+    if (two) { FB_CUDA_OK(cudaEventRecord(t->ev[kEvChunkIn], st)); FB_CUDA_OK(cudaStreamWaitEvent(t->aux, t->ev[kEvChunkIn], 0)); }
     int c = 0;
     for (int b0 = 0; b0 < batch; b0 += n->max_batch, c++) {
         const int B = min(n->max_batch, batch - b0), w = two ? (c & 1) : 0;
@@ -1832,7 +1775,7 @@ int tc_forward_chunks(fb_qnet *n, int slot, const float *params_dev, const uint8
         int rc = tc_forward(n, slot, w, params_dev, fv, B, q_out_dev + (size_t)b0 * 2, w ? t->aux : st);
         if (rc) return rc;
     }
-    if (two) { FB_CUDA_OK(cudaEventRecord(t->ev[15], t->aux)); FB_CUDA_OK(cudaStreamWaitEvent(st, t->ev[15], 0)); }
+    if (two) { FB_CUDA_OK(cudaEventRecord(t->ev[kEvChunkOut], t->aux)); FB_CUDA_OK(cudaStreamWaitEvent(st, t->ev[kEvChunkOut], 0)); }
     return FB_OK;
 }
 
@@ -1852,83 +1795,96 @@ int train_step_launch(fb_qnet *n, const QnetStep &a, int pack_online, int pack_t
     const FwdWs &f = t->ws[0];
     const int B = a.B, H = L.hidden, P1 = B * kP1, P2 = B * kP2;
     cudaStream_t sx = t->aux;
-    int e = 0;
-    auto fork = [&](cudaStream_t from, cudaStream_t to) -> cudaError_t {       // `to` waits for everything issued on `from`
-        cudaError_t r = cudaEventRecord(t->ev[e], from);
-        if (r == cudaSuccess) r = cudaStreamWaitEvent(to, t->ev[e], 0);
-        e++;
-        return r;
+    int e = 0;                                  // next running event slot
+    auto record = [&](cudaStream_t on, cudaEvent_t *ev) -> int {            // the next running slot, recorded on `on`
+        FB_REQUIRE(e < kEvGather, "train_step_launch: out of running event slots (the next one is the replay gather's)");
+        *ev = t->ev[e++];
+        FB_CUDA_OK(cudaEventRecord(*ev, on));
+        return FB_OK;
+    };
+    auto fork = [&](cudaStream_t from, cudaStream_t to, cudaEvent_t *ev_out = nullptr) -> int {   // `to` waits for everything issued on `from`
+        cudaEvent_t ev;
+        int r = record(from, &ev);
+        if (r) return r;
+        FB_CUDA_OK(cudaStreamWaitEvent(to, ev, 0));
+        if (ev_out) *ev_out = ev;
+        return FB_OK;
     };
     // the minibatch itself.  The sampler leaves the ring offsets of the drawn frames behind (a.fs.tab): the convolutions read the
     // frames in place, and the gather into the caller-visible minibatch buffers (frames, actions, rewards, terminals -- the head
     // kernel needs the last three) runs on a side stream beside the forward passes: one dependent stage less (5.5 us)
     const bool sampled = a.pro.replay != nullptr;
-    t->step_samples = sampled ? 1 : 0;                            // (read by conv1_mode_at; reset below, after the step's conv1 launches)
-    const int e_gather = 12;
     if (sampled) {
         rc = replay_launch_sample(a.pro, true, st); if (rc) return rc;
-        FB_CUDA_OK(cudaEventRecord(t->ev[e_gather], st));
-        FB_CUDA_OK(cudaStreamWaitEvent(t->aux4, t->ev[e_gather], 0));
+        FB_CUDA_OK(cudaEventRecord(t->ev[kEvGather], st));
+        FB_CUDA_OK(cudaStreamWaitEvent(t->aux4, t->ev[kEvGather], 0));
         rc = replay_launch_gather(a.pro, a.gamma, t->aux4); if (rc) return rc;
-        FB_CUDA_OK(cudaEventRecord(t->ev[e_gather], t->aux4));
+        FB_CUDA_OK(cudaEventRecord(t->ev[kEvGather], t->aux4));
     }
     if (pack_online) { rc = tc_pack_weights(n, a.params, 0, st); if (rc) return rc; }
-    FB_CUDA_OK(fork(st, sx));
+    if ((rc = fork(st, sx))) return rc;
     // ---- aux: Q(s') with the net the variant names (and the online net too for Double)
     if (a.variant != 0 && pack_target) { rc = tc_pack_weights(n, a.target, 1, sx); if (rc) return rc; }
     if (a.variant == 2) { rc = tc_forward(n, 0, 1, a.params, a.fn, B, n->q_next_online, sx); if (rc) return rc; }
     rc = a.variant == 0 ? tc_forward(n, 0, 1, a.params, a.fn, B, n->q_next, sx) : tc_forward(n, 1, 1, a.target, a.fn, B, n->q_next, sx);
     if (rc) return rc;
-    if (sampled) FB_CUDA_OK(cudaStreamWaitEvent(sx, t->ev[e_gather], 0));     // the event below then also says: minibatch buffers complete
+    if (sampled) FB_CUDA_OK(cudaStreamWaitEvent(sx, t->ev[kEvGather], 0));     // the event below then also says: minibatch buffers complete
     // ---- main: Q(s) with the online net; its activations stay in workspace 0 for the backward pass
     // the TD target, loss and dLoss/dQ come out of its head kernel, which first waits for Q(s') from the other stream
-    FB_CUDA_OK(cudaEventRecord(t->ev[e], sx));
-    const int e_x2 = 13;
-    const int c1mode = conv1_mode_at(t, B);
-    if (c1mode == 3) {                         // X2 of s for the conv1 weight gradient: early, on the stream of the replay gather
-        FB_CUDA_OK(cudaEventRecord(t->ev[e_x2], st));          // (st has seen the sampler; nothing else of this step yet)
-        FB_CUDA_OK(cudaStreamWaitEvent(t->aux4, t->ev[e_x2], 0));
+    cudaEvent_t q_next_done;
+    if ((rc = record(sx, &q_next_done))) return rc;
+    // Q(s)'s conv1 from the u8 frames too, X2 packed early on the stream of the replay gather -- up to minibatch 512 when the step
+    // draws its own minibatch.  Measured: it wins there (100.9 vs 102.9 us per update at 256) and loses above (1,024: 235 vs
+    // 213 us; 4,096: 689 vs 635 us -- the u8 path is bound by shared memory, the X2 path by HBM); on a caller-supplied minibatch
+    // no gather runs ahead of the X2 conversion to keep its 3,528 CTAs out of the way of the two conv1 launches (105 vs 98 us)
+    const bool x2_early = sampled && B <= kFuseMaxBatch;
+    if (x2_early) {                            // X2 of s for the conv1 weight gradient: early, on the stream of the replay gather
+        FB_CUDA_OK(cudaEventRecord(t->ev[kEvX2], st));         // (st has seen the sampler; nothing else of this step yet)
+        FB_CUDA_OK(cudaStreamWaitEvent(t->aux4, t->ev[kEvX2], 0));
         pack_x2_kernel<<<dim3((unsigned)(((size_t)P1 * 8 + 255) / 256)), dim3(256), 0, t->aux4>>>(a.fs, B, f.x2, t->f16);
         FB_CUDA_OK(cudaGetLastError());
-        FB_CUDA_OK(cudaEventRecord(t->ev[e_x2], t->aux4));
+        FB_CUDA_OK(cudaEventRecord(t->ev[kEvX2], t->aux4));
     }
-    TdFuse td{1, a.variant, a.loss_sum, a.global_batch, n->per_broadcast, a.gamma, n->q_next, n->q_next_online, a.rewards, a.isw, a.actions,
-              a.terminals, n->dq, a.abs_err, a.q_target, t->loss_terms, a.ret, a.disc};
-    const AdamPow apow{a.ad.on, t->adam_pow, t->adam_pow + 2, a.ad.lr, a.ad.beta1, a.ad.beta2};
+    TrainFwd tr{};
+    tr.td = TdFuse{1, a.variant, a.loss_sum, a.global_batch, n->per_broadcast, a.gamma, n->q_next, n->q_next_online, a.rewards, a.isw, a.actions,
+                   a.terminals, n->dq, a.abs_err, a.q_target, t->loss_terms, a.ret, a.disc};
+    tr.join = q_next_done;
+    tr.ap = AdamPow{a.ad.on, t->adam_pow, t->adam_pow + 2, a.ad.lr, a.ad.beta1, a.ad.beta2};
     // fp16 operands: gradient tensors carry a power-of-two factor that keeps them in fp16's normal range (dq ~ err / batch for the
     // mean losses); it is removed exactly where weight / bias gradients are finalised.  bf16: 1.
     float gscale = 1.f;
     if (t->f16) { gscale = 8.f; if (!a.loss_sum) { int gb = a.global_batch > 0 ? a.global_batch : B; while (gscale < 8.f * (float)gb) gscale *= 2.f; } }
-    rc = tc_forward_impl(n, 0, 0, a.params, a.fs, B, n->q, 1, st, &td, t->ev[e], &apow, gscale); if (rc) return rc;
-    e++;
+    tr.gscale = gscale;
+    tr.x2_early = x2_early;
+    rc = run_forward(n, 0, 0, a.params, a.fs, B, n->q, &tr, st); if (rc) return rc;
     // Memory.batch_update (BrainPrioritizedReplyDQN.py:316) needs only |TD error|, which the head kernel has just written: it runs on
     // a stream of its own beside the whole backward pass (measured: 26 us at the step's tail otherwise) and joins at the end
     const bool per_on_side = sampled && a.pro.prioritized;
-    int e_head = -1;
-    if (per_on_side) { e_head = e++; FB_CUDA_OK(cudaEventRecord(t->ev[e_head], st)); }       // launched below, after the fc1 gradient GEMMs
+    cudaEvent_t head_done = nullptr;
+    if (per_on_side && (rc = record(st, &head_done))) return rc;        // launched below, after the fc1 gradient GEMMs
     // ---- backward.  The head's backward pass rode in the forward's last kernel when hidden = 512 (fc1_head_train_kernel);
     // otherwise: fp32 gradients of the head variables and the fc1 bias straight into partials, dh1 as bf16
     const bool fused_head = fused_head_ok(L);
     const int G = fused_head ? head_ctas(t, B) : (B + kHeadRows - 1) / kHeadRows;
     if (!fused_head)
         FB_CUDA_OK(tc::launch_pdl(head_backward_tc_kernel, dim3(H / 32 + 1, G), dim3(256), 0, st, f.h1, n->dq, a.params, L, B, t->hp, t->hb,
-                                  t->loss_terms, t->dh1, apow, GradFmt{t->f16, gscale}));
+                                  t->loss_terms, t->dh1, tr.ap, GradFmt{t->f16, gscale}));
     cudaStream_t sy = t->aux2;                  // third stream: bias column sums and the early Adam on W_fc1, all off the critical path
-    FB_CUDA_OK(fork(st, sx));
+    if ((rc = fork(st, sx))) return rc;
     // fc1: dW = a3^T dh1 (aux, written in place), dz3 = (dh1 Wf1^T) * relu'(a3)
     FB_CUDA_OK((launch_tc_gemm<128, 1>(p->a3_m, p->dh1_b, p->fc1_w, dim3(13, H / 128, 1), EpiStoreF32{a.grads + L.wf1, kFlat, H, 0, 1.f / gscale}, sx)));
-    const int e_fc1w = e++;
-    FB_CUDA_OK(cudaEventRecord(t->ev[e_fc1w], sx));                    // W_fc1's gradient is final
+    cudaEvent_t fc1w_done;
+    if ((rc = record(sx, &fc1w_done))) return rc;                      // W_fc1's gradient is final
     FB_CUDA_OK((launch_tc_gemm<64, 0>(p->dh1_k, wm.wf1n, p->fc1_d, dim3((B + 127) / 128, kFlat / 64, 1), EpiFc1Dgrad{t->dz3, f.a3, B, t->f16}, st)));
-    FB_CUDA_OK(fork(st, sx));
-    const int e_fc1d = e - 1;
+    cudaEvent_t fc1d_done;
+    if ((rc = fork(st, sx, &fc1d_done))) return rc;
     if (per_on_side) {
         // (captured AFTER the two fc1 GEMMs: its one 1,024-thread CTA fits only on the SMs the fused backward kernel leaves free,
         // and a kernel that cannot be placed held back the launches captured behind it -- the fc1 weight gradient started 5 us late)
-        FB_CUDA_OK(cudaStreamWaitEvent(t->aux4, t->ev[e_head], 0));
+        FB_CUDA_OK(cudaStreamWaitEvent(t->aux4, head_done, 0));
         rc = replay_launch_per_update(a.pro, a.abs_err, t->aux4); if (rc) return rc;
     }
-    FB_CUDA_OK(cudaStreamWaitEvent(sy, t->ev[e_fc1d], 0));              // sy: after the fc1 data gradient (dz3 complete, wf1n no longer read)
+    FB_CUDA_OK(cudaStreamWaitEvent(sy, fc1d_done, 0));              // sy: after the fc1 data gradient (dz3 complete, wf1n no longer read)
     const int c1 = (P1 + kChunk1 - 1) / kChunk1, c23 = (P2 + kChunk23 - 1) / kChunk23;
     auto colsum_on = [&](const bf16 *x, float *part, int rows, int N, int chunk_rows, int chunks) -> cudaError_t {
         ColsumJobs cj{};
@@ -1940,15 +1896,14 @@ int train_step_launch(fb_qnet *n, const QnetStep &a, int pack_online, int pack_t
     FB_CUDA_OK(colsum_on(t->dz3, t->bp3, P2, 64, kChunk23, c23));
     FB_REQUIRE(a.xch == nullptr || !a.ad.on || a.grads == dist_current_grads(a.xch), "training step with an exchange: gradients must go to its current buffer");
     AdamDev ad{a.ad.on && a.xch == nullptr, const_cast<float *>(a.params), a.ad.m, a.ad.v, a.ad.beta1, a.ad.beta2, a.ad.eps, a.ad.grad_scale, t->adam_pow + 2};
-    tc::pdl_next_launch_plain(t->nopdl & 4);
     FB_CUDA_OK((launch_tc_wgrad<64, 5, kSlabW3, 1, 6>(p->a2_w, p->dz3_b, p->conv3_w, p->s3, EpiStoreF32{t->part3, 640, 64, (size_t)640 * 64}, sx)));
     if (a.ad.on) {
         // Adam on W_fc1 (91 % of the parameters) on a stream of its own, as soon as its gradient is final (fc1 weight-gradient GEMM,
         // sx) and its bf16 / fp16 copy has been read for the last time (fc1 data-gradient GEMM): beside everything that is left of
         // the step -- nothing downstream reads W_fc1 or its gradient again; it joins at the step's end.  On several GPUs the same
         // slot holds W_fc1's bucket of the gradient exchange (sum over NVLink peer memory + Adam).
-        FB_CUDA_OK(cudaStreamWaitEvent(t->aux3, t->ev[e_fc1d], 0));
-        FB_CUDA_OK(cudaStreamWaitEvent(t->aux3, t->ev[e_fc1w], 0));
+        FB_CUDA_OK(cudaStreamWaitEvent(t->aux3, fc1d_done, 0));
+        FB_CUDA_OK(cudaStreamWaitEvent(t->aux3, fc1w_done, 0));
         if (a.xch != nullptr) {
             rc = dist_launch_bucket(a.xch, n, 0, const_cast<float *>(a.params), a.ad.m, a.ad.v, t->adam_pow + 2, a.ad.beta1, a.ad.beta2, a.ad.eps,
                                     a.ad.grad_scale, t->aux3);
@@ -1958,46 +1913,48 @@ int train_step_launch(fb_qnet *n, const QnetStep &a, int pack_online, int pack_t
             FB_CUDA_OK(cudaGetLastError());
         }
     }
-    if (t->fuse_bwd && B <= kFuseMaxBatch) {
+    if (B <= kFuseMaxBatch && !t->separate_kernels) {
         // conv3 data gradient + ReLU mask + conv2 data gradient + un-pool in one kernel (tc_bwd23_kernel)
-        tc::pdl_next_launch_plain(t->nopdl & 2);
         FB_CUDA_OK((launch_tc_bwd23<2>(p->dz3_s, wm.w3d, wm.w2d, Bwd23Params{(B + 1) / 2, B, f.a2, t->dz2, f.z1, t->dz1, t->f16}, t->n_sms, st)));
-        FB_CUDA_OK(fork(st, sx));
-        FB_CUDA_OK(cudaStreamWaitEvent(sy, t->ev[e - 1], 0));          // sx, sy: dz2 and dz1 complete
+        cudaEvent_t dgrad_done;
+        if ((rc = fork(st, sx, &dgrad_done))) return rc;
+        FB_CUDA_OK(cudaStreamWaitEvent(sy, dgrad_done, 0));             // sx, sy: dz2 and dz1 complete
         FB_CUDA_OK(colsum_on(t->dz1, t->bp1, P1, 32, kChunk1, c1));
         FB_CUDA_OK(colsum_on(t->dz2, t->bp2, P2, 64, kChunk23, c23));
-        tc::pdl_next_launch_plain(t->nopdl & 8);
         FB_CUDA_OK((launch_tc_wgrad<64, 4, kSlabW2, 2, 4>(p->p2_w, p->dz2_b, p->conv2_w, p->s2, EpiStoreF32{t->part2, 512, 64, (size_t)512 * 64}, sx)));
     } else {
         FB_CUDA_OK((launch_tc_conv<64, kSlab3, 1, 9, 4, 1>(p->dz3_s, wm.w3d, p->conv3_d, t->n_sms, EpiConv3Dgrad{t->dz2, f.a2, P2, t->f16}, st)));
-        FB_CUDA_OK(fork(st, sx));
-        FB_CUDA_OK(cudaStreamWaitEvent(sy, t->ev[e - 1], 0));          // sy: after the conv3 data gradient (dz2 complete)
+        cudaEvent_t dgrad_done;
+        if ((rc = fork(st, sx, &dgrad_done))) return rc;
+        FB_CUDA_OK(cudaStreamWaitEvent(sy, dgrad_done, 0));             // sy: after the conv3 data gradient (dz2 complete)
         FB_CUDA_OK(colsum_on(t->dz2, t->bp2, P2, 64, kChunk23, c23));
         FB_CUDA_OK((launch_tc_wgrad<64, 4, kSlabW2, 2, 4>(p->p2_w, p->dz2_b, p->conv2_w, p->s2, EpiStoreF32{t->part2, 512, 64, (size_t)512 * 64}, sx)));
         FB_CUDA_OK((launch_tc_conv<128, kSlab2, 1, 4, 4, 1>(p->dz2_s, wm.w2d, p->conv2_d, t->n_sms, EpiStoreBf16{t->dp2, P2, 128, t->f16}, st)));
         FB_CUDA_OK(tc::launch_pdl(unpool_relu_kernel_tc, dim3((unsigned)(((size_t)B * 400 + 255) / 256)), dim3(256), 0, st, f.z1, t->dp2, B, t->dz1, t->f16));
-        FB_CUDA_OK(fork(st, sy));                                       // sy: after the un-pool (dz1 complete)
+        if ((rc = fork(st, sy))) return rc;                             // sy: after the un-pool (dz1 complete)
         FB_CUDA_OK(colsum_on(t->dz1, t->bp1, P1, 32, kChunk1, c1));
     }
     // conv1 weight gradient (no input gradient there); the bias gradients = column sums of the dZ tensors ran beside it
-    t->step_samples = 0;
-    if (c1mode == 3) FB_CUDA_OK(cudaStreamWaitEvent(st, t->ev[e_x2], 0));
-    tc::pdl_next_launch_plain((t->nopdl & 1) && B <= kFuseMaxBatch);      // (large minibatches fill the GPU by themselves: early launch pays there)
+    if (x2_early) FB_CUDA_OK(cudaStreamWaitEvent(st, t->ev[kEvX2], 0));
+    // launched plainly up to minibatch 512: launched early, its 147 CTAs sat on SMs waiting for the fused data-gradient kernel while
+    // the conv3 weight gradient, which was ready, queued behind them (121 -> 114.5 us per update, measured; the fused backward, the
+    // other weight gradients and finalize launched plainly measured slower or equal).  Large minibatches fill the GPU by
+    // themselves: early launch pays there.
+    tc::pdl_next_launch_plain(B <= kFuseMaxBatch);
     FB_CUDA_OK((launch_tc_wgrad<32, 2, kSlabW1, 1, 6>(p->x2_w, p->dz1_b, p->conv1_w, p->s1, EpiStoreF32{t->part1, 256, 32, (size_t)256 * 32}, st)));
-    FB_CUDA_OK(fork(sx, st));
-    FB_CUDA_OK(fork(sy, st));
+    if ((rc = fork(sx, st))) return rc;
+    if ((rc = fork(sy, st))) return rc;
     FinalizeArgs fa{t->part1, t->part2, t->part3, p->s1, p->s2, p->s3, t->bp1, t->bp2, t->bp3, c1, c23, c23, t->hp, t->hb, G, a.loss_out, 1.f / gscale};
     const int n_compact = L.wf1 + (L.total - L.bf1);
     const int nb_fin = (n_compact + 31) / 32;
-    tc::pdl_next_launch_plain(t->nopdl & 16);
     FB_CUDA_OK(tc::launch_pdl(finalize_grads_kernel, dim3(nb_fin), dim3(32 * kFinWarps), 0, st, fa, L, a.grads, ad, t->pw[0]));
     if (a.ad.on && a.xch != nullptr) {          // the rest of the vector (79,522 parameters): the only exchange left at the tail
         rc = dist_launch_bucket(a.xch, n, 1, const_cast<float *>(a.params), a.ad.m, a.ad.v, t->adam_pow + 2, a.ad.beta1, a.ad.beta2, a.ad.eps,
                                 a.ad.grad_scale, st);
         if (rc) return rc;
     }
-    if (a.ad.on) FB_CUDA_OK(fork(t->aux3, st));  // W_fc1's Adam / exchange bucket joins here, at the very end
-    if (per_on_side) FB_CUDA_OK(fork(t->aux4, st));          // Memory.batch_update (started right after the head) joins here
+    if (a.ad.on && (rc = fork(t->aux3, st))) return rc;          // W_fc1's Adam / exchange bucket joins here, at the very end
+    if (per_on_side && (rc = fork(t->aux4, st))) return rc;      // Memory.batch_update (started right after the head) joins here
     return FB_OK;
 }
 
@@ -2024,25 +1981,18 @@ int tc_drop_graphs(fb_qnet *n) {
     return FB_OK;
 }
 
-extern "C" int fb_qnet_set_conv1_mode(fb_qnet *n, int mode) {
-    FB_REQUIRE(n != nullptr && n->tc != nullptr && mode >= 0 && mode <= 4, "fb_qnet_set_conv1_mode: needs a tensor-core precision and mode 0..4");
-    n->tc->conv1_mode = mode;
-    for (auto &g : n->tc->graphs) destroy_entry(g);
-    n->tc->graphs.clear();
-    return FB_OK;
-}
-
-extern "C" int fb_qnet_set_fused_backward(fb_qnet *n, int on) {
-    FB_REQUIRE(n != nullptr && n->tc != nullptr, "fb_qnet_set_fused_backward: needs FB_PRECISION_BF16");
-    n->tc->fuse_bwd = (on & 1) ? 1 : 0;
-    n->tc->fuse_fwd = (on & 2) || on == 1 ? 1 : 0;
+// test hook: the separate conv2 / conv3 forward kernels and the separate conv3 data gradient / conv2 data gradient / un-pool
+// kernels at every minibatch, where the fused ones would run -- the reference the fused kernels are held to bit for bit
+extern "C" int fb_debug_tc_separate_kernels(fb_qnet *n, int on) {
+    FB_REQUIRE(n != nullptr && n->tc != nullptr, "fb_debug_tc_separate_kernels: needs a tensor-core precision");
+    n->tc->separate_kernels = on ? 1 : 0;
     return tc_drop_graphs(n);
 }
 
 extern "C" int fb_qnet_use_graphs(fb_qnet *n, int enable) {
     FB_REQUIRE(n != nullptr, "fb_qnet_use_graphs: NULL argument");
     if (n->tc) n->tc->use_graph = enable ? 1 : 0;
-    return FB_OK;
+    return tc_drop_graphs(n);
 }
 
 // One training step (fb_qnet_step).  With Adam, beta*_power are the caller's (QNetwork keeps them like TF's beta1_power /
@@ -2118,10 +2068,14 @@ int tc_step(fb_qnet *n, const QnetStep &a, float beta1_power, float beta2_power,
 
 // ------------------------------------------------------------------------------------------------ kernel probe
 // Re-launches ONE GEMM kernel of the path `reps` times on whatever the workspaces hold (after a forward / training
-// step at the same batch), so that bench.py and ncu can time it in isolation.  which: 0 conv1 forward, 1 conv2
-// forward, 2 conv3 forward, 3 fc1 forward, 4 conv1 weight gradient, 5 conv3 data gradient, 6 fc1 data gradient.
+// step at the same batch), so that bench.py and ncu can time it in isolation.  which: 1 conv2 forward, 2 conv3 forward,
+// 3 fc1 forward, 4 conv1 weight gradient, 5 conv3 data gradient, 6 fc1 data gradient; 7..11 the fused conv1 on the frames of
+// this net's last forward: from the u8 frames without / with Z1 (7 / 8), from X2 without / with Z1 (9 / 10), from X2 without
+// pooling (11).  0 was conv1 as a kernel of its own, which the library no longer has.
 extern "C" int fb_debug_tc_kernel(fb_qnet *n, int which, int B, int reps, const float *params_dev, void *stream) {
     FB_REQUIRE(n && n->tc && params_dev && B > 0 && B <= n->max_batch && reps > 0, "fb_debug_tc_kernel: bad argument");
+    FB_REQUIRE(which != 0, "fb_debug_tc_kernel: kernel 0, the separate conv1 forward kernel, is retired (7..11 time the fused conv1)");
+    FB_REQUIRE(which >= 1 && which <= 11, "fb_debug_tc_kernel: which must be 1..11");
     TcState *t = n->tc;
     TcPlan *p;
     int rc = make_plan(n, B, &p);
@@ -2130,10 +2084,9 @@ extern "C" int fb_debug_tc_kernel(fb_qnet *n, int which, int B, int reps, const 
     const QnetLayout &L = n->L;
     const TcWeightMaps &wm = t->wm[0];
     const FwdWs &f = t->ws[0];
-    const int H = L.hidden, P1 = B * kP1, P2 = B * kP2;
+    const int H = L.hidden, P2 = B * kP2;
     for (int r = 0; r < reps; r++) {
         switch (which) {
-            case 0: FB_CUDA_OK((launch_tc_conv<32, kSlab1, 1, 4, 6, 1>(p->x2_s[0], wm.w1p, p->conv1, t->n_sms, EpiConv1{f.z1, params_dev + L.b1, P1, t->f16}, st))); break;
             case 1: FB_CUDA_OK((launch_tc_conv<64, kSlab2, 2, 8, 3, 1>(p->p2_s[0], wm.w2p, p->conv2, t->n_sms, EpiGrid7{f.a2, params_dev + L.b2, P2, t->f16}, st))); break;
             case 2: FB_CUDA_OK((launch_tc_conv<64, kSlab3, 1, 9, 4, 1>(p->a2_s[0], wm.w3p, p->conv3, t->n_sms, EpiConv3{f.a3, params_dev + L.b3, P2, t->f16}, st))); break;
             case 3: FB_CUDA_OK((launch_tc_gemm<128, 2>(p->a3_k[0], wm.wf1n, p->fc1, dim3((B + 127) / 128, H / 128, p->sf),
@@ -2141,12 +2094,11 @@ extern "C" int fb_debug_tc_kernel(fb_qnet *n, int which, int B, int reps, const 
             case 4: FB_CUDA_OK((launch_tc_wgrad<32, 2, kSlabW1, 1, 6>(p->x2_w, p->dz1_b, p->conv1_w, p->s1, EpiStoreF32{t->part1, 256, 32, (size_t)256 * 32}, st))); break;
             case 5: FB_CUDA_OK((launch_tc_conv<64, kSlab3, 1, 9, 4, 1>(p->dz3_s, wm.w3d, p->conv3_d, t->n_sms, EpiConv3Dgrad{t->dz2, f.a2, P2, t->f16}, st))); break;
             case 6: FB_CUDA_OK((launch_tc_gemm<64, 0>(p->dh1_k, wm.wf1n, p->fc1_d, dim3((B + 127) / 128, kFlat / 64, 1), EpiFc1Dgrad{t->dz3, f.a3, B, t->f16}, st))); break;
-            case 7: FB_CUDA_OK((launch_tc_conv1_fused<4, false>(p->x2_s[0], wm.w1p, Conv1FusedParams{g_probe_view, B, params_dev + L.b1, nullptr, f.p2, t->f16}, t->n_sms, st))); break;
-            case 8: FB_CUDA_OK((launch_tc_conv1_fused<4, false>(p->x2_s[0], wm.w1p, Conv1FusedParams{g_probe_view, B, params_dev + L.b1, f.z1, f.p2, t->f16}, t->n_sms, st))); break;
-            case 9: FB_CUDA_OK((launch_tc_conv1_fused<6, true>(p->x2_s[0], wm.w1p, Conv1FusedParams{g_probe_view, B, params_dev + L.b1, nullptr, f.p2, t->f16}, t->n_sms, st))); break;
-            case 10: FB_CUDA_OK((launch_tc_conv1_fused<6, true>(p->x2_s[0], wm.w1p, Conv1FusedParams{g_probe_view, B, params_dev + L.b1, f.z1, f.p2, t->f16}, t->n_sms, st))); break;
-            case 11: FB_CUDA_OK((launch_tc_conv1_fused<6, true>(p->x2_s[0], wm.w1p, Conv1FusedParams{g_probe_view, B, params_dev + L.b1, nullptr, nullptr, t->f16}, t->n_sms, st))); break;
-            default: FB_REQUIRE(false, "fb_debug_tc_kernel: which must be 0..11");
+            case 7: FB_CUDA_OK((launch_tc_conv1_fused<4, false>(p->x2_s[0], wm.w1p, Conv1FusedParams{t->probe_view, B, params_dev + L.b1, nullptr, f.p2, t->f16}, t->n_sms, st))); break;
+            case 8: FB_CUDA_OK((launch_tc_conv1_fused<4, false>(p->x2_s[0], wm.w1p, Conv1FusedParams{t->probe_view, B, params_dev + L.b1, f.z1, f.p2, t->f16}, t->n_sms, st))); break;
+            case 9: FB_CUDA_OK((launch_tc_conv1_fused<6, true>(p->x2_s[0], wm.w1p, Conv1FusedParams{t->probe_view, B, params_dev + L.b1, nullptr, f.p2, t->f16}, t->n_sms, st))); break;
+            case 10: FB_CUDA_OK((launch_tc_conv1_fused<6, true>(p->x2_s[0], wm.w1p, Conv1FusedParams{t->probe_view, B, params_dev + L.b1, f.z1, f.p2, t->f16}, t->n_sms, st))); break;
+            case 11: FB_CUDA_OK((launch_tc_conv1_fused<6, true>(p->x2_s[0], wm.w1p, Conv1FusedParams{t->probe_view, B, params_dev + L.b1, nullptr, nullptr, t->f16}, t->n_sms, st))); break;
         }
     }
     return FB_OK;

@@ -178,21 +178,8 @@ int fb_debug_poison_packed(fb_qnet *net, int slot, void *stream);
  * with 16-byte streaming stores (mode 0) or through shared memory + cp.async.bulk (mode 1); no computation */
 int fb_debug_write_probe(uint8_t *dst_dev, int n_chunks, long long stride_bytes, int mode, int ctas, void *stream);
 /* Tensor-core precisions (FB_PRECISION_BF16 / _FP16) only: replay fb_qnet_step as a CUDA graph once the same arguments were seen twice
- * (default on; the eager two-stream path is identical work). */
+ * (default on; the eager two-stream path is identical work).  Every call drops the graphs captured so far. */
 int fb_qnet_use_graphs(fb_qnet *net, int enable);
-/* Tensor-core precisions only: how conv1 is run (also FB_TC_CONV1_MODE).  4 (default): 3 up to minibatch 512 when the step draws its own
- * minibatch (fb_qnet_step with `sampling`), 2 otherwise (measured).
- * 3: the 2x2 max-pool is fused into conv1's epilogue and its input tile is ALWAYS built in the kernel straight from the u8 frames;
- * the 16-bit input matrix X2, which then only the conv1 weight gradient reads, is packed on a side stream beside the forwards.
- * 2: as 3 when no backward pass follows (acting, Q(s')); the training forward materialises X2 first and reads it by TMA.
- * 1: pooled epilogue, input always via the materialised matrix; 0: three separate kernels (conversion, conv1, pooling).
- * Results are bit-identical in all modes. */
-int fb_qnet_set_conv1_mode(fb_qnet *net, int mode);
-/* Tensor-core precisions only.  Which fused kernels the update uses at minibatch <= 512 (also FB_TC_FUSE_FWD / FB_TC_FUSE_BWD):
- * 0: none (conv2, conv3, conv3 data gradient, conv2 data gradient, un-pool are separate kernels); 2: the forward pair only
- * (conv2 + conv3 as one kernel); 1 or 3 (default): forward pair and backward triple (conv3 data gradient, its ReLU mask, conv2
- * data gradient and the un-pool as ONE kernel whose intermediate never leaves the SM).  Results are bit-identical. */
-int fb_qnet_set_fused_backward(fb_qnet *net, int on);
 int fb_qnet_param_count(const fb_qnet *net);
 int fb_qnet_layout(const fb_qnet *net, int32_t *out16_host);
 
@@ -412,8 +399,14 @@ int fb_debug_tc_gemm(int mode, int bn, int M, int N, int K, const void *a_bf16_d
 /* measurement hook: SM cycles for `iters` back-to-back tcgen05.mma (M 128, K 16, bf16) of width n from one thread */
 int fb_debug_tc_mma_rate(int n, int mn_major, int naccs, int iters, int same_operands, long long *cycles_dev, void *stream);
 /* measurement hook: re-launch one GEMM kernel of the tensor-core path `reps` times on the current workspace contents
- * (which: 0 conv1 fwd, 1 conv2 fwd, 2 conv3 fwd, 3 fc1 fwd, 4 conv1 wgrad, 5 conv3 dgrad, 6 fc1 dgrad) */
+ * (which: 1 conv2 fwd, 2 conv3 fwd, 3 fc1 fwd, 4 conv1 wgrad, 5 conv3 dgrad, 6 fc1 dgrad; 7..11 the fused conv1 on the frames of the
+ * net's last forward: from the u8 frames without / with Z1 (7 / 8), from X2 without / with Z1 (9 / 10), from X2 without pooling (11).
+ * 0, conv1 as a kernel of its own, is retired: FB_ERR_INVALID) */
 int fb_debug_tc_kernel(fb_qnet *net, int which, int batch, int reps, const float *params_dev, void *stream);
+/* test hook, tensor-core precisions only: on != 0 runs the separate conv2 / conv3 forward kernels and the separate conv3 data
+ * gradient / conv2 data gradient / un-pool kernels at every minibatch (at minibatch <= 512 the fused kernels run otherwise; the
+ * results are bit-identical).  Drops the net's captured graphs. */
+int fb_debug_tc_separate_kernels(fb_qnet *net, int on);
 /* device test hook: D[128][64] = A[shift..shift+128)[64] Bt[64][64]^T with A [256][64] loaded once as a swizzled slab and
  * the MMA descriptor started shift rows into it (the property the one-slab-many-taps convolution relies on). */
 int fb_debug_tc_slab(int shift, int base_offset, const void *a_bf16_dev, const void *b_bf16_dev, float *d_dev, void *stream);

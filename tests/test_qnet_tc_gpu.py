@@ -128,28 +128,26 @@ def test_forward_matches_oracle_bf16(mods, dueling):
     assert np.abs(q - q32).max() <= 2e-2 * np.abs(q32).max()
 
 
-def test_conv1_modes_are_bit_identical(mods):
-    """conv1 as three kernels (mode 0), with the max-pool in its epilogue (1), built straight from the u8 frames when no
-    backward follows (2, default), and from the u8 frames in the training forward too, X2 packed beside it for the weight
-    gradient (3): the same arithmetic on different data paths -- identical Q-values and gradients"""
+def test_conv1_paths_are_bit_identical(mods):
+    """conv1 of the training forward on s has two data paths: built from the u8 frames, with X2 (which then only the conv1 weight
+    gradient reads) packed beside it -- when the step draws its own minibatch, up to minibatch 512 -- or from X2 materialised
+    first and read by TMA -- on a minibatch the caller passes.  The same arithmetic on different data paths: a step that draws its
+    minibatch and a twin net's step on that same minibatch, passed by the caller, give identical gradients and loss, bit for bit
+    (bf16, an odd minibatch)"""
     _lib, game, qnet = mods
+    from dqnflappybird_b200 import replay
     B = 70
-    frames = _env_frames(game, B, 9)
-    nets = [qnet.QNetwork(max_batch=128, seed=2, precision="bf16") for _ in range(5)]      # modes 0..3 and 4 = the default choice by minibatch
-    for mode, n in enumerate(nets):
+    mem = _memory(game, replay, 48, 20, B, 30)
+    nets = [qnet.QNetwork(max_batch=128, seed=2, precision="bf16") for _ in range(2)]
+    for n in nets:
         n.params.mul_(4.0); n.target.mul_(4.0)
-        _lib.check(_lib.lib().fb_qnet_set_conv1_mode(n._h, mode), "fb_qnet_set_conv1_mode")
-    q = [n.forward(qnet.FrameBatch.from_stack(frames, 1)) for n in nets]
-    assert all(torch.equal(q[0], x) for x in q[1:])
-    rng = np.random.default_rng(3)
-    a = torch.from_numpy(rng.integers(0, 2, B).astype(np.uint8)).cuda()
-    r = torch.from_numpy(rng.choice(np.array([0.1, 3.0, -3.0], np.float32), B)).cuda()
-    term = (r == -3.0).to(torch.uint8)
-    for _ in range(3):                              # eager, eager, graph replay
-        for n in nets:
-            n.loss_backward("double", frames, a, r, term)
-        for n in nets[1:]:
-            assert torch.equal(nets[0].grads, n.grads) and nets[0].loss.item() == n.loss.item()
+    for rep in range(3):                            # eager, eager, graph replay
+        sp, mb = mem.step_sampling(B)
+        nets[0].loss_backward("double", mb.frames, mb.actions, mb.rewards, mb.terminals, sampling=sp)     # conv1 from the u8 frames
+        nets[1].loss_backward("double", mb.frames, mb.actions, mb.rewards, mb.terminals)                  # conv1 from X2
+        assert torch.isfinite(nets[0].grads).all()
+        assert torch.equal(nets[0].grads, nets[1].grads) and nets[0].loss.item() == nets[1].loss.item(), rep
+    assert nets[0].grads.abs().max().item() > 0
 
 
 def test_forward_from_ring_view_bf16(mods):
@@ -402,19 +400,21 @@ def test_loss_and_gradients_other_hidden_width_bf16(mods):
         assert np.linalg.norm(g[o:o + sz] - g_ref[o:o + sz]) <= 1.5e-2 * np.linalg.norm(g_ref[o:o + sz]), name
 
 
+@pytest.mark.parametrize("precision", ["bf16", "fp16"])
 @pytest.mark.parametrize("B,variant,dueling", [(33, "nature", False), (70, "double", True), (300, "nature", False), (700, "vanilla", False)])
-def test_fused_backward_is_bit_identical(mods, B, variant, dueling):
+def test_fused_backward_is_bit_identical(mods, B, variant, dueling, precision):
     """tc_bwd23_kernel (conv3 data gradient + ReLU mask + conv2 data gradient + un-pool in one kernel, dZ2 handed from the
     first GEMM's epilogue to the second through a hand-swizzled shared-memory slab) against the three separate kernels:
-    identical gradients, bit for bit.  Odd minibatch (last tile = one sample), one tile per CTA, and several tiles per CTA
-    (the slab ring and both accumulators are reused: 350 tiles on 148 CTAs)."""
+    identical gradients, bit for bit, in both 16-bit operand formats (fp16: gradient tensors scaled by a power of two).  Odd
+    minibatch (last tile = one sample), one tile per CTA, and several tiles per CTA (the slab ring and both accumulators are
+    reused: 350 tiles on 148 CTAs)."""
     _lib, game, qnet = mods
     frames = _env_frames(game, B, 23)
-    nets = [qnet.QNetwork(max_batch=B, seed=2, dueling=dueling, precision="bf16") for _ in range(2)]
+    nets = [qnet.QNetwork(max_batch=B, seed=2, dueling=dueling, precision=precision) for _ in range(2)]
     for n in nets:
         n.params.mul_(4.0); n.target.mul_(4.0)
-    _lib.check(_lib.lib().fb_qnet_set_fused_backward(nets[1]._h, 0), "fb_qnet_set_fused_backward")
-    # (switch 0 also turns off the forward twin, tc_fwd23_kernel: conv2 + conv3 as one kernel)
+    _lib.check(_lib.lib().fb_debug_tc_separate_kernels(nets[1]._h, 1), "fb_debug_tc_separate_kernels")
+    # (the hook also turns off the forward twin, tc_fwd23_kernel: conv2 + conv3 as one kernel)
     q = [n.forward(qnet.FrameBatch.from_stack(frames, 1)) for n in nets]
     assert torch.isfinite(q[0]).all() and torch.equal(q[0], q[1])
     rng = np.random.default_rng(3)

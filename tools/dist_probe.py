@@ -39,7 +39,8 @@ def main():
              ("no exchange work at all", 15)]
     for name, mask in cases:
         _lib.check(L.fb_dist_debug_mask(x._h, mask), "fb_dist_debug_mask")
-        _lib.check(L.fb_qnet_set_fused_backward(net._h, 3), "drop graphs")          # re-capture with the new mask
+        for on in (0, 1):                                                           # drop the graphs: re-capture with the new mask
+            _lib.check(L.fb_qnet_use_graphs(net._h, on), "fb_qnet_use_graphs")
         dist.barrier()
         for _ in range(20):
             net.train_step("nature", frames, a, r, term, global_batch=B * world)
