@@ -26,7 +26,7 @@ struct NoisyLayers {
     int factors;                          // length of the factor vector
 };
 
-NoisyLayers noisy_layers(const QnetLayout &L) {
+NoisyLayers noisy_layers(const NetLayout &L) {
     NoisyLayers N{};
     const int H = L.hidden;
     auto add = [&](int w, int b, int p, int q) {
@@ -36,8 +36,9 @@ NoisyLayers noisy_layers(const QnetLayout &L) {
         N.factors += p + q;
     };
     add(L.wf1, L.bf1, kFlat, H);
-    if (!L.dueling) add(L.wf2, L.bf2, H, kActions);
-    else { add(L.wv, L.bv, H, 1); add(L.wa, L.ba, H, kActions); }
+    const int nv = L.atoms ? L.atoms : 1, na = L.atoms ? kActions * L.atoms : kActions;      // C51: fan-out N and 2N
+    if (!L.dueling) add(L.wf2, L.bf2, H, na);
+    else { add(L.wv, L.bv, H, nv); add(L.wa, L.ba, H, na); }
     return N;
 }
 

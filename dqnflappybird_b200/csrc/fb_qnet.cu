@@ -369,8 +369,10 @@ static void wgrad(fb_qnet *n, int M, int N, int K, int kchunk, AL al, const floa
     splitk_reduce_kernel<<<(unsigned)((mn + 255) / 256), 256, 0, st>>>(n->partial, splits, mn, gout);
 }
 
-static int forward_chunk(fb_qnet *n, const float *params, FrameView fv, int B, float *q_out, cudaStream_t st) {
-    const QnetLayout &L = n->L;
+// probs / logp (C51 net only, may be nullptr): p and log p of every action's atoms, [B][2][N]
+static int forward_chunk(fb_qnet *n, const float *params, FrameView fv, int B, float *q_out, cudaStream_t st, float *probs = nullptr,
+                         float *logp = nullptr) {
+    const NetLayout &L = n->L;
     launch_gemm<32, false, false>(B * 400, kC1, kK1, 1, LoadConv1{fv}, LoadPlain{params + L.w1, kC1},
                                   EpiBiasRelu{n->z1, params + L.b1, kC1}, st);
     maxpool_kernel<<<(B * 3200 + 255) / 256, 256, 0, st>>>(n->z1, n->p1, B);
@@ -380,16 +382,16 @@ static int forward_chunk(fb_qnet *n, const float *params, FrameView fv, int B, f
                                   EpiBiasRelu{n->a3, params + L.b3, kC3}, st);
     launch_gemm<64, false, false>(B, L.hidden, kFlat, 1, LoadPlain{n->a3, kFlat}, LoadPlain{params + L.wf1, L.hidden},
                                   EpiBiasRelu{n->h1, params + L.bf1, L.hidden}, st);
+    if (L.atoms) return c51_launch_head_forward(nullptr, 0, 0, n->h1, params, L, B, nullptr, probs, logp, q_out, st);
     head_forward_kernel<<<(B + 3) / 4, 128, 0, st>>>(n->h1, params, L, B, q_out);
     FB_CUDA_OK(cudaGetLastError());
     return FB_OK;
 }
 
-extern "C" int fb_qnet_create(int hidden, int dueling, int max_batch, fb_qnet **out) {
-    FB_REQUIRE(out != nullptr && hidden > 0 && hidden % 4 == 0 && max_batch > 0, "fb_qnet_create: bad argument");
+static int create_net(int hidden, int dueling, int max_batch, int atoms, double v_min, double v_max, fb_qnet **out) {
     fb_qnet *n = new (std::nothrow) fb_qnet();
     FB_REQUIRE(n != nullptr, "fb_qnet_create: out of host memory");
-    n->L = qnet_layout(hidden, dueling ? 1 : 0);
+    n->L = NetLayout{qnet_layout(hidden, dueling ? 1 : 0, atoms), atoms, v_min, v_max};
     n->max_batch = max_batch;
     n->precision = FB_PRECISION_FP32;
     n->tc = nullptr;
@@ -410,14 +412,37 @@ extern "C" int fb_qnet_create(int hidden, int dueling, int max_batch, fb_qnet **
     n->partial_floats = need;
     FB_CUDA_OK(alloc(&n->partial, need));
     FB_CUDA_OK(alloc(&n->loss_dev, 4));
+    if (atoms) {
+        const size_t G = (B + kC51Rows - 1) / kC51Rows;
+        FB_CUDA_OK(alloc(&n->c51_ps, B * 2 * atoms)); FB_CUDA_OK(alloc(&n->c51_logps, B * 2 * atoms)); FB_CUDA_OK(alloc(&n->c51_pn, B * 2 * atoms));
+        FB_CUDA_OK(alloc(&n->c51_dl, B * c51_cols(n->L))); FB_CUDA_OK(alloc(&n->c51_terms, B));
+        FB_CUDA_OK(alloc(&n->c51_hp, G * c51_partial_stride(n->L))); FB_CUDA_OK(alloc(&n->c51_hb, G * 4));
+    }
     *out = n;
     return FB_OK;
+}
+
+extern "C" int fb_qnet_create(int hidden, int dueling, int max_batch, fb_qnet **out) {
+    FB_REQUIRE(out != nullptr && hidden > 0 && hidden % 4 == 0 && max_batch > 0, "fb_qnet_create: bad argument");
+    return create_net(hidden, dueling, max_batch, 0, 0.0, 0.0, out);
+}
+
+// The distributional (C51) head: atoms outputs per action over the support v_min .. v_max (fb_c51.cu)
+extern "C" int fb_qnet_create_c51(int hidden, int dueling, int max_batch, int atoms, double v_min, double v_max, fb_qnet **out) {
+    FB_REQUIRE(out != nullptr && hidden > 0 && hidden % 32 == 0 && hidden <= 2048 && max_batch > 0,
+               "fb_qnet_create_c51: bad argument (hidden must be a multiple of 32, at most 2048)");
+    FB_REQUIRE(atoms >= 2 && atoms <= kC51MaxAtoms, "fb_qnet_create_c51: atoms must be 2..64");
+    FB_REQUIRE(isfinite(v_min) && isfinite(v_max) && v_min < v_max, "fb_qnet_create_c51: the support needs finite v_min < v_max");
+    int rc = c51_prepare();
+    if (rc) return rc;
+    return create_net(hidden, dueling, max_batch, atoms, v_min, v_max, out);
 }
 
 extern "C" int fb_qnet_destroy(fb_qnet *n) {
     if (!n) return FB_OK;
     tc_state_destroy(n);
-    float *ps[] = {n->z1, n->p1, n->a2, n->a3, n->h1, n->q, n->q_next, n->q_next_online, n->dq, n->dh1, n->dz3, n->dz2, n->dp1, n->dz1, n->partial, n->loss_dev};
+    float *ps[] = {n->z1, n->p1, n->a2, n->a3, n->h1, n->q, n->q_next, n->q_next_online, n->dq, n->dh1, n->dz3, n->dz2, n->dp1, n->dz1, n->partial, n->loss_dev,
+                   n->c51_ps, n->c51_logps, n->c51_pn, n->c51_dl, n->c51_terms, n->c51_hp, n->c51_hb};
     for (float *p : ps) cudaFree(p);
     delete n;
     return FB_OK;
@@ -439,6 +464,7 @@ extern "C" int fb_qnet_get_precision(const fb_qnet *n) { return n ? n->precision
 // current buffer (fb_dist_grads / fb_dist_parity) and the caller calls fb_dist_advance after each step.  NULL detaches.
 extern "C" int fb_qnet_attach_exchange(fb_qnet *n, fb_dist *d) {
     FB_REQUIRE(n != nullptr, "fb_qnet_attach_exchange: NULL argument");
+    FB_REQUIRE(d == nullptr || n->L.atoms == 0, "fb_qnet_attach_exchange: a C51 net takes the all-reduce path (no in-step exchange)");
     n->xch = d;
     return tc_drop_graphs(n);
 }
@@ -477,24 +503,36 @@ static void set_view(FrameView &fv, const uint8_t *frames, long long stride, con
     for (int c = 0; c < 4; c++) fv.chan_off[c] = chan_off[c];
 }
 
-extern "C" int fb_qnet_forward(fb_qnet *n, const float *params_dev, const uint8_t *frames_dev, long long sample_stride,
-                               const int32_t *chan_off, int batch, float *q_out_dev, void *stream) {
-    FB_REQUIRE(n && params_dev && frames_dev && chan_off && q_out_dev && batch > 0, "fb_qnet_forward: bad argument");
-    cudaStream_t st = (cudaStream_t)stream;
+static int forward_impl(fb_qnet *n, const float *params_dev, const uint8_t *frames_dev, long long sample_stride, const int32_t *chan_off,
+                        int batch, float *probs_out_dev, float *q_out_dev, cudaStream_t st) {
     int slot = 0;
     if (tc_precision(n->precision)) {
         int rc = tc_slot_for(n, params_dev, -1, st, &slot); if (rc) return rc;
-        return tc_forward_chunks(n, slot, params_dev, frames_dev, sample_stride, chan_off, batch, q_out_dev, st);
+        return tc_forward_chunks(n, slot, params_dev, frames_dev, sample_stride, chan_off, batch, q_out_dev, st, probs_out_dev);
     }
     for (int b0 = 0; b0 < batch; b0 += n->max_batch) {
         int B = min(n->max_batch, batch - b0);
         FrameView fv;
         set_view(fv, frames_dev + (size_t)b0 * sample_stride, sample_stride, chan_off);
-        int rc = tc_precision(n->precision) ? tc_forward(n, slot, 0, params_dev, fv, B, q_out_dev + (size_t)b0 * 2, st)
-                                                   : forward_chunk(n, params_dev, fv, B, q_out_dev + (size_t)b0 * 2, st);
+        int rc = forward_chunk(n, params_dev, fv, B, q_out_dev + (size_t)b0 * 2, st,
+                               probs_out_dev ? probs_out_dev + (size_t)b0 * 2 * n->L.atoms : nullptr);
         if (rc) return rc;
     }
     return FB_OK;
+}
+
+extern "C" int fb_qnet_forward(fb_qnet *n, const float *params_dev, const uint8_t *frames_dev, long long sample_stride,
+                               const int32_t *chan_off, int batch, float *q_out_dev, void *stream) {
+    FB_REQUIRE(n && params_dev && frames_dev && chan_off && q_out_dev && batch > 0, "fb_qnet_forward: bad argument");
+    return forward_impl(n, params_dev, frames_dev, sample_stride, chan_off, batch, nullptr, q_out_dev, (cudaStream_t)stream);
+}
+
+// C51 net: the per-action distributions probs_out [batch][2][atoms] and their expectations q_out [batch][2]
+extern "C" int fb_qnet_forward_dist(fb_qnet *n, const float *params_dev, const uint8_t *frames_dev, long long sample_stride,
+                                    const int32_t *chan_off, int batch, float *probs_out_dev, float *q_out_dev, void *stream) {
+    FB_REQUIRE(n && params_dev && frames_dev && chan_off && probs_out_dev && q_out_dev && batch > 0, "fb_qnet_forward_dist: bad argument");
+    FB_REQUIRE(n->L.atoms > 0, "fb_qnet_forward_dist: the net has the expected-value head (create it with fb_qnet_create_c51)");
+    return forward_impl(n, params_dev, frames_dev, sample_stride, chan_off, batch, probs_out_dev, q_out_dev, (cudaStream_t)stream);
 }
 
 extern "C" int fb_qnet_act(fb_qnet *n, const float *params_dev, const uint8_t *frames_dev, long long sample_stride,
@@ -510,20 +548,29 @@ extern "C" int fb_qnet_act(fb_qnet *n, const float *params_dev, const uint8_t *f
 
 // TD target, loss and backward of the strict-fp32 path into a.grads
 static int loss_backward_impl(fb_qnet *n, const QnetStep &a, cudaStream_t st) {
-    const QnetLayout &L = n->L;
+    const NetLayout &L = n->L;
     const int B = a.B;
     int rc;
     // Q(s') with the net the variant names (and the online net too for Double), then Q(s) last so that its
     // activations are the ones left in the workspace for the backward pass.
     if (a.variant == 2) { rc = forward_chunk(n, a.params, a.fn, B, n->q_next_online, st); if (rc) return rc; }
-    rc = forward_chunk(n, a.variant == 0 ? a.params : a.target, a.fn, B, n->q_next, st); if (rc) return rc;
-    rc = forward_chunk(n, a.params, a.fs, B, n->q, st); if (rc) return rc;
-    td_loss_kernel<<<1, 256, 0, st>>>(n->q, n->q_next, n->q_next_online, a.actions, a.rewards, a.terminals, a.isw, B, a.global_batch,
-                                       a.variant, a.gamma, a.loss_sum, n->dq, a.loss_out, a.abs_err, a.q_target, n->per_broadcast, a.ret,
-                                       a.disc);
-    // ---- backward
-    head_backward_w_kernel<<<(L.hidden + 1 + 127) / 128, 128, 0, st>>>(n->h1, n->dq, L, B, a.grads);
-    head_backward_h_kernel<<<(B * L.hidden + 255) / 256, 256, 0, st>>>(n->h1, n->dq, a.params, L, B, n->dh1, nullptr);
+    rc = forward_chunk(n, a.variant == 0 ? a.params : a.target, a.fn, B, n->q_next, st, n->c51_pn); if (rc) return rc;
+    rc = forward_chunk(n, a.params, a.fs, B, n->q, st, n->c51_ps, n->c51_logps); if (rc) return rc;
+    if (L.atoms) {              // C51: projection + cross-entropy, then the head's backward pass (fb_c51.cu)
+        rc = c51_launch_loss(L, B, a.variant, a.loss_sum, a.global_batch, a.gamma, n->c51_ps, n->c51_logps, n->c51_pn, n->q_next, n->q_next_online,
+                             a.actions, a.rewards, a.terminals, a.isw, a.ret, a.disc, n->c51_dl, n->c51_terms, a.abs_err, a.q_target, st);
+        if (rc == FB_OK)
+            rc = c51_launch_head_backward(L, B, n->h1, n->c51_dl, a.params, n->c51_terms, a.grads, a.loss_out, n->dh1, nullptr, nullptr, nullptr, 0,
+                                          1.f, AdamPow{}, st);
+        if (rc) return rc;
+    } else {
+        td_loss_kernel<<<1, 256, 0, st>>>(n->q, n->q_next, n->q_next_online, a.actions, a.rewards, a.terminals, a.isw, B, a.global_batch,
+                                           a.variant, a.gamma, a.loss_sum, n->dq, a.loss_out, a.abs_err, a.q_target, n->per_broadcast, a.ret,
+                                           a.disc);
+        // ---- backward
+        head_backward_w_kernel<<<(L.hidden + 1 + 127) / 128, 128, 0, st>>>(n->h1, n->dq, L, B, a.grads);
+        head_backward_h_kernel<<<(B * L.hidden + 255) / 256, 256, 0, st>>>(n->h1, n->dq, a.params, L, B, n->dh1, nullptr);
+    }
     // fc1: dW = a3^T dh1 (+ bias row), da3 = dh1 Wf1^T masked by relu(a3)
     wgrad<true>(n, kFlat, L.hidden, B, 64, LoadFc1T{n->a3}, n->dh1, a.grads + L.wf1, st);
     launch_gemm<64, false, true>(B, kFlat, L.hidden, 1, LoadPlain{n->dh1, L.hidden}, LoadTrans{a.params + L.wf1, L.hidden},
@@ -570,6 +617,7 @@ extern "C" int fb_qnet_step(fb_qnet *n, const fb_qnet_step_args *a, void *stream
     } else {
         FB_REQUIRE(a->frames_dev && a->actions_dev && a->rewards_dev && a->terminals_dev, "fb_qnet_step: NULL argument");
     }
+    FB_REQUIRE(n->L.atoms == 0 || !n->per_broadcast, "fb_qnet_step: the reference's broadcast PER loss (fb_qnet_set_per_broadcast) has no C51 form");
     const int batch = sp ? sp->batch : a->batch;
     FB_REQUIRE(batch > 0 && batch <= n->max_batch, "fb_qnet_step: batch outside 1..max_batch");
     const bool tc = tc_precision(n->precision);

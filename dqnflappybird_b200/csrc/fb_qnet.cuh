@@ -19,21 +19,30 @@ constexpr int kK1 = 8 * 8 * 4, kK2 = 4 * 4 * 32, kK3 = 3 * 3 * 64;
 struct QnetLayout {             // offsets (in floats) into the flat parameter vector, TF variable creation order
     int hidden, dueling;
     int w1, b1, w2, b2, w3, b3, wf1, bf1;
-    int wf2, bf2;               // plain head [H,2], [2]
-    int wv, bv, wa, ba;         // dueling heads [H,1],[1],[H,2],[2]
+    int wf2, bf2;               // plain head [H,2], [2]             (C51: [H,2N], [2N], column a N + i)
+    int wv, bv, wa, ba;         // dueling heads [H,1],[1],[H,2],[2]  (C51: [H,N],[N],[H,2N],[2N])
     int total;
 };
+// The net's layout with its head: atoms 0 is the expected-value head, 2..64 the distributional (C51) head over N = atoms
+// (fb_c51.cu) with the support z_i = (float)(v_min + i dz), dz = (v_max - v_min) / (N - 1) in float64.  Kept apart from
+// QnetLayout, which the trunk and expected-value head kernels take by value, so that their parameters and code stay as they are.
+struct NetLayout : QnetLayout {
+    int atoms;
+    double v_min, v_max;
+};
 
-inline QnetLayout qnet_layout(int hidden, int dueling) {
+// the offsets; atoms > 0 sizes the C51 head
+inline QnetLayout qnet_layout(int hidden, int dueling, int atoms = 0) {
     QnetLayout L{};
     L.hidden = hidden; L.dueling = dueling;
+    const int nv = atoms ? atoms : 1, na = atoms ? kActions * atoms : kActions;     // outputs of the V head, of the A (or plain) head
     int o = 0;
     L.w1 = o; o += kK1 * kC1; L.b1 = o; o += kC1;
     L.w2 = o; o += kK2 * kC2; L.b2 = o; o += kC2;
     L.w3 = o; o += kK3 * kC3; L.b3 = o; o += kC3;
     L.wf1 = o; o += kFlat * hidden; L.bf1 = o; o += hidden;
-    if (!dueling) { L.wf2 = o; o += hidden * kActions; L.bf2 = o; o += kActions; L.wv = L.bv = L.wa = L.ba = -1; }
-    else { L.wv = o; o += hidden; L.bv = o; o += 1; L.wa = o; o += hidden * kActions; L.ba = o; o += kActions; L.wf2 = L.bf2 = -1; }
+    if (!dueling) { L.wf2 = o; o += hidden * na; L.bf2 = o; o += na; L.wv = L.bv = L.wa = L.ba = -1; }
+    else { L.wv = o; o += hidden * nv; L.bv = o; o += nv; L.wa = o; o += hidden * na; L.ba = o; o += na; L.wf2 = L.bf2 = -1; }
     L.total = o;
     return L;
 }
@@ -73,11 +82,64 @@ __device__ __forceinline__ float adam_math(float g, float pi, float &mi, float &
     return pi - (mi * alpha) / (sqrtf(vi) + eps);
 }
 
+// Fused Adam (fb_qnet_step with m_dev / v_dev): one thread of the step's head kernel -- early on the step's critical path, exactly
+// once per step -- turns the beta powers kept in device memory into this step's alpha = lr sqrt(1 - beta2^t) / (1 - beta1^t)
+// (fp32, the host formula) and advances them; the step's last kernel reads alpha.  Nothing about a step is a launch argument.
+struct AdamPow { int on; float *pow /* beta1^t, beta2^t */, *alpha; float lr, beta1, beta2; };
+__device__ __forceinline__ void adam_pow_advance(const AdamPow &ap) {
+    const float b1p = ap.pow[0], b2p = ap.pow[1];
+    *ap.alpha = ap.lr * sqrtf(1.f - b2p) / (1.f - b1p);
+    ap.pow[0] = b1p * ap.beta1; ap.pow[1] = b2p * ap.beta2;
+}
+
+// ---- distributional (C51) head, L.atoms > 0 (fb_c51.cu).  Column space of the head's outputs: plain c = a N + i (W_fc2 /
+// b_fc2); dueling c < N the V head's atom c, c = N + a N + i the A head's (a, i).  Per-sample loss gradients are kept in that
+// space ([B][c51_cols]); the backward pass writes per row group partials [G][(H + 1) cols + H]: weight (j, c) at j cols + c,
+// head bias c at H cols + c, fc1 bias j at (H + 1) cols + j.
+constexpr int kC51MaxAtoms = 64;
+constexpr int kC51Rows = 16;                // minibatch rows per head-backward row group (tensor-core path)
+__host__ __device__ inline int c51_cols(const NetLayout &L) { return (L.dueling ? 3 : 2) * L.atoms; }
+__host__ __device__ inline size_t c51_partial_stride(const NetLayout &L) { return (size_t)(L.hidden + 1) * c51_cols(L) + L.hidden; }
+// flat parameter index of head weight (j, c), or of head bias c for j == hidden
+__host__ __device__ inline int c51_flat(const NetLayout &L, int j, int c) {
+    const int N = L.atoms, H = L.hidden;
+    if (!L.dueling) return j < H ? L.wf2 + j * 2 * N + c : L.bf2 + c;
+    if (c < N) return j < H ? L.wv + j * N + c : L.bv + c;
+    return j < H ? L.wa + j * 2 * N + (c - N) : L.ba + (c - N);
+}
+// the inverse for a flat index inside the head
+__host__ __device__ inline void c51_column(const NetLayout &L, int i, int *j, int *c) {
+    const int N = L.atoms, H = L.hidden;
+    if (!L.dueling) {
+        if (i < L.bf2) { const int e = i - L.wf2; *j = e / (2 * N); *c = e % (2 * N); } else { *j = H; *c = i - L.bf2; }
+    } else if (i < L.bv) { const int e = i - L.wv; *j = e / N; *c = e % N; }
+    else if (i < L.wa) { *j = H; *c = i - L.bv; }
+    else if (i < L.ba) { const int e = i - L.wa; *j = e / (2 * N); *c = N + e % (2 * N); }
+    else { *j = H; *c = N + i - L.ba; }
+}
+int c51_prepare();              // kernel attributes (once per process, at create)
+// head forward, one warp per sample: h1 from fc1's split-K partials (part != nullptr: sum in order + bias + ReLU, kept in h1_out
+// when that is set) or read from h1_in; probs / logp [B][2][N] when set; q [B][2]
+int c51_launch_head_forward(const float *part, int splits, size_t split_stride, const float *h1_in, const float *params, const NetLayout &L,
+                            int B, float *h1_out, float *probs, float *logp, float *q, cudaStream_t st);
+// target projection, cross-entropy, dLoss/dlogits (column space) and the per-sample outputs.  pn: p of the Q(s') forward
+// whose argmax (or, for Double, q_next_online's) picks a*
+int c51_launch_loss(const NetLayout &L, int B, int variant, int loss_sum, int global_batch, double gamma, const float *ps, const float *logps,
+                    const float *pn, const float *q_next, const float *q_next_online, const uint8_t *actions, const float *rewards,
+                    const uint8_t *terminals, const float *isw, const double *ret, const double *disc, float *dl, float *terms, float *abs_err,
+                    float *q_target, cudaStream_t st);
+// head backward.  grads != nullptr (fp32 path): one row group, head weights / biases written into grads, dh1 fp32 into dh1_f32, the
+// loss (terms in order) into loss_out.  Else: row groups of kC51Rows, partials into hp and the loss partial into hb[g * 4 + 2], dh1
+// times gscale rounded to the 16-bit format (f16) into dh1_16, the fc1 bias partial from the rounded values; ap: the fused Adam's alpha
+int c51_launch_head_backward(const NetLayout &L, int B, const float *h1, const float *dl, const float *params, const float *terms, float *grads,
+                             float *loss_out, float *dh1_f32, float *hp, float *hb, void *dh1_16, int f16, float gscale, const AdamPow &ap,
+                             cudaStream_t st);
+
 // ---- handle shared by the strict-fp32 path (fb_qnet.cu) and the tcgen05 path (fb_qnet_tc.cu) ------------
 struct fb_dist;                 // multi-GPU gradient exchange (fb_dist.cu)
 struct TcState;                 // bf16 workspace, packed weights and TMA plans (fb_qnet_tc.cu)
 struct fb_qnet {
-    QnetLayout L;
+    NetLayout L;
     int max_batch;
     int precision;              // FB_PRECISION_FP32 (CUDA-core FMA), FB_PRECISION_BF16 or FB_PRECISION_FP16 (tcgen05, fp32 accumulate)
     // fp32 activations of the online net on s (kept for backward) and scratch for the other forwards
@@ -90,6 +152,9 @@ struct fb_qnet {
     fb_dist *xch;                 // attached exchange: the training step sums every rank's gradients inside its own graph (or NULL)
     int per_broadcast;            // PER loss as the reference's graph really computes it: every sample weighted by mean(ISWeights)
     const float *packed_src[2];   // parameter vectors the bf16 operand copies (slot 0 online, 1 target) were made from
+    // C51 head (L.atoms > 0), allocated at create for max_batch: p and log p of the training forward on s, p of the Q(s')
+    // forward [B][2][N]; dLoss/dlogits [B][c51_cols]; loss terms [B]; head-backward partials [G][c51_partial_stride], [G][4]
+    float *c51_ps, *c51_logps, *c51_pn, *c51_dl, *c51_terms, *c51_hp, *c51_hb;
 };
 
 // small CUDA-core stages both paths share (defined in fb_qnet.cu)
@@ -144,9 +209,10 @@ int tc_drop_graphs(fb_qnet *n);                 // captured steps embed the net'
 void tc_state_destroy(fb_qnet *n);
 int tc_pack_weights(fb_qnet *n, const float *params_dev, int slot /* 0 online, 1 target */, cudaStream_t st);
 int tc_slot_for(fb_qnet *n, const float *params_dev, int want_slot, cudaStream_t st, int *slot_out);
-int tc_forward(fb_qnet *n, int slot, int ws, const float *params_dev, FrameView fv, int B, float *q_out, cudaStream_t st);
+// probs (C51 net, may be nullptr): p [B][2][N] beside Q
+int tc_forward(fb_qnet *n, int slot, int ws, const float *params_dev, FrameView fv, int B, float *q_out, cudaStream_t st, float *probs = nullptr);
 int tc_forward_chunks(fb_qnet *n, int slot, const float *params_dev, const uint8_t *frames_dev, long long sample_stride,
-                      const int32_t *chan_off, int batch, float *q_out_dev, cudaStream_t st);
+                      const int32_t *chan_off, int batch, float *q_out_dev, cudaStream_t st, float *probs_dev = nullptr);
 int tc_step(fb_qnet *n, const QnetStep &a, float beta1_power, float beta2_power, cudaStream_t st);
 int tc_adam(fb_qnet *n, float *params_dev, const float *grads_dev, float *m_dev, float *v_dev, float alpha, float beta1, float beta2,
             float eps, float grad_scale, cudaStream_t st);

@@ -483,10 +483,7 @@ __global__ void __launch_bounds__(256) colsum_kernel(ColsumJobs jobs) {
 // sum_b dh1.  Block = 32 hidden units x 8 row lanes; block gridDim.x-1 does the head bias.
 constexpr int kHeadRows = 256;                      // rows of the minibatch per head-backward CTA row group
 constexpr int kMaxHeadCtas = 160;                   // fused head kernel: at most one CTA (four samples at a time) per SM
-// Fused Adam (fb_qnet_step with m_dev / v_dev): one thread of this kernel -- early on the step's critical path, exactly once per step --
-// turns the beta powers kept in device memory into this step's alpha = lr sqrt(1 - beta2^t) / (1 - beta1^t) (fp32, the
-// host formula) and advances them; the step's last kernel reads alpha.  Nothing about a step is a launch argument.
-struct AdamPow { int on; float *pow /* beta1^t, beta2^t */, *alpha; float lr, beta1, beta2; };
+// Fused Adam: AdamPow (fb_qnet.cuh) -- one thread of this kernel, early on the step's critical path, forms this step's alpha.
 // operand format of the gradient tensors and the power of two they are scaled by (1 for bf16; fp16's exponent range is narrow:
 // dh1 and everything downstream of it carry the factor, the weight / bias gradients are un-scaled where they are finalised)
 struct GradFmt { int f16; float scale; };
@@ -810,8 +807,11 @@ __global__ void __launch_bounds__(256) adam_wf1_kernel(QnetLayout L, const float
         *reinterpret_cast<uint2 *>(pw.wf1n + 4 * i4) = make_uint2(pk[0], pk[1]);
     }
 }
+// kC51: the head region reads c51_head_backward_kernel's partials (fb_c51.cu); a separate instantiation, so that the expected-value
+// head's code is exactly what it was
+template <bool kC51>
 __global__ void __launch_bounds__(32 * kFinWarps) finalize_grads_kernel(const FinalizeArgs a, QnetLayout L, float *__restrict__ grads, const AdamDev ad,
-                                                                       const PackedWeights pw) {
+                                                                       const PackedWeights pw, const NetLayout Lc /* kC51: the head */) {
     __shared__ float red[kFinWarps][32];
     const int lane = threadIdx.x & 31, g = threadIdx.x >> 5, H = L.hidden;
     const int k = blockIdx.x * 32 + lane;            // compact index: [0, wf1) then [bf1, total)
@@ -859,7 +859,12 @@ __global__ void __launch_bounds__(32 * kFinWarps) finalize_grads_kernel(const Fi
             strided_sum(a.c3, [&](int z) { return a.bp3[z * 64 + n]; });
         } else if (i < L.bf1 + H) {         // fc1 bias
             int j = i - L.bf1;
-            strided_sum(a.G, [&](int z) { return a.hp[((size_t)z * H + j) * 4 + 3]; });
+            if constexpr (kC51) strided_sum(a.G, [&](int z) { return a.hp[z * c51_partial_stride(Lc) + (size_t)(H + 1) * c51_cols(Lc) + j]; });
+            else strided_sum(a.G, [&](int z) { return a.hp[((size_t)z * H + j) * 4 + 3]; });
+        } else if constexpr (kC51) {        // C51 head: partials [G][c51_partial_stride]
+            int j, c;
+            c51_column(Lc, i, &j, &c);
+            strided_sum(a.G, [&](int z) { return a.hp[z * c51_partial_stride(Lc) + (size_t)j * c51_cols(Lc) + c]; });
         } else if (!L.dueling) {
             if (i < L.bf2) { int e = i - L.wf2; strided_sum(a.G, [&](int z) { return a.hp[((size_t)z * H + (e >> 1)) * 4 + (e & 1)]; }); }
             else { int e = i - L.bf2; strided_sum(a.G, [&](int z) { return a.hb[z * 4 + e]; }); }
@@ -1453,7 +1458,7 @@ constexpr int kFc1Splits = 5;                    // fc1 forward: 25 K-blocks in 
 // fully pipelined kernels (bwd 172 us against 125 us; whole update 721 against 607 us): above this batch the separate kernels run.
 constexpr int kFuseMaxBatch = 512;
 // the fused head kernel (fc1_head_train_kernel<16>) serves the reference's hidden width; other widths keep the two-kernel form
-bool fused_head_ok(const QnetLayout &L) { return L.hidden == 512; }
+bool fused_head_ok(const NetLayout &L) { return L.hidden == 512 && L.atoms == 0; }
 int head_ctas(const TcState *t, int B) { const int c = (B + 3) / 4, m = t->n_sms < kMaxHeadCtas ? t->n_sms : kMaxHeadCtas; return c < m ? c : m; }
 
 // slab geometry (rows of 128 bytes): tile or K-block rows + the largest tap offset, rounded up to 8
@@ -1707,14 +1712,15 @@ struct TrainFwd {
     float gscale;               // power of two carried by the gradient tensors (GradFmt)
     bool x2_early;              // conv1 from the u8 frames, X2 packed early by the caller; else X2 is packed here and feeds conv1
 };
+// probs: a C51 net's p [B][2][N] (may be nullptr; the training forward keeps p and log p of s in the net's own buffers)
 static int run_forward(fb_qnet *n, int slot, int w, const float *params_dev, FrameView fv, int B, float *q_out, const TrainFwd *tr,
-                       cudaStream_t st) {
+                       cudaStream_t st, float *probs = nullptr) {
     TcState *t = n->tc;
     FB_REQUIRE(t != nullptr && B > 0 && B <= n->max_batch && (w == 0 || w == 1), "tc_forward: bad argument");
     TcPlan *p;
     int rc = make_plan(n, B, &p);
     if (rc) return rc;
-    const QnetLayout &L = n->L;
+    const NetLayout &L = n->L;
     const TcWeightMaps &wm = t->wm[slot];
     const FwdWs &f = t->ws[w];
     const int P1 = B * kP1, P2 = B * kP2;
@@ -1740,6 +1746,16 @@ static int run_forward(fb_qnet *n, int slot, int w, const float *params_dev, Fra
     FB_CUDA_OK((launch_tc_gemm<128, 2>(p->a3_k[w], wm.wf1n, p->fc1, dim3((B + 127) / 128, L.hidden / 128, p->sf),
                                        EpiStoreF32{f.parth, B, L.hidden, (size_t)n->max_batch * L.hidden}, st)));
     if (keep) FB_CUDA_OK(cudaStreamWaitEvent(st, tr->join, 0));
+    if (L.atoms) {                             // C51 head (fb_c51.cu); training: h1, p and log p of s kept, then the loss
+        const size_t sstride = (size_t)n->max_batch * L.hidden;
+        rc = c51_launch_head_forward(f.parth, p->sf, sstride, nullptr, params_dev, L, B, keep ? f.h1 : nullptr, keep ? n->c51_ps : probs,
+                                     keep ? n->c51_logps : nullptr, q_out, st);
+        if (rc || !keep) return rc;
+        const TdFuse &td = tr->td;
+        return c51_launch_loss(L, B, td.variant, td.loss_sum, td.global_batch, td.gamma, n->c51_ps, n->c51_logps, n->c51_pn, td.q_next,
+                               td.q_next_online, td.actions, td.rewards, td.terminals, td.isw, td.ret, td.disc, n->c51_dl, n->c51_terms,
+                               td.abs_err, td.q_target, st);
+    }
     if (keep && fused_head_ok(L))              // training step: head forward + TD loss + head backward in one kernel
         FB_CUDA_OK(tc::launch_pdl(fc1_head_train_kernel<16>, dim3(head_ctas(t, B)), dim3(128), 0, st, f.parth, p->sf,
                                   (size_t)n->max_batch * L.hidden, params_dev, L, B, q_out, tr->td, HeadBwd{t->dh1, t->hp, t->hb, GradFmt{t->f16, tr->gscale}},
@@ -1753,14 +1769,14 @@ static int run_forward(fb_qnet *n, int slot, int w, const float *params_dev, Fra
                                   keep ? f.h1 : nullptr, q_out, keep ? tr->td : TdFuse{}));
     return FB_OK;
 }
-int tc_forward(fb_qnet *n, int slot, int w, const float *params_dev, FrameView fv, int B, float *q_out, cudaStream_t st) {
-    return run_forward(n, slot, w, params_dev, fv, B, q_out, nullptr, st);
+int tc_forward(fb_qnet *n, int slot, int w, const float *params_dev, FrameView fv, int B, float *q_out, cudaStream_t st, float *probs) {
+    return run_forward(n, slot, w, params_dev, fv, B, q_out, nullptr, st, probs);
 }
 
 // Acting over more samples than one workspace holds: chunks alternate between the two forward workspaces and the two
 // streams, so one chunk's latency chain (seven kernels) overlaps the other's.
 int tc_forward_chunks(fb_qnet *n, int slot, const float *params_dev, const uint8_t *frames_dev, long long sample_stride,
-                      const int32_t *chan_off, int batch, float *q_out_dev, cudaStream_t st) {
+                      const int32_t *chan_off, int batch, float *q_out_dev, cudaStream_t st, float *probs_dev) {
     TcState *t = n->tc;
     FB_REQUIRE(t != nullptr, "tc_forward_chunks: no tensor-core state");
     const int nchunks = (batch + n->max_batch - 1) / n->max_batch;
@@ -1772,7 +1788,8 @@ int tc_forward_chunks(fb_qnet *n, int slot, const float *params_dev, const uint8
         FrameView fv;
         fv.base = frames_dev + (size_t)b0 * sample_stride; fv.sample_stride = sample_stride; fv.tab = nullptr; fv.tab_stride = 0;
         for (int k = 0; k < 4; k++) fv.chan_off[k] = chan_off[k];
-        int rc = tc_forward(n, slot, w, params_dev, fv, B, q_out_dev + (size_t)b0 * 2, w ? t->aux : st);
+        int rc = tc_forward(n, slot, w, params_dev, fv, B, q_out_dev + (size_t)b0 * 2, w ? t->aux : st,
+                            probs_dev ? probs_dev + (size_t)b0 * 2 * n->L.atoms : nullptr);
         if (rc) return rc;
     }
     if (two) { FB_CUDA_OK(cudaEventRecord(t->ev[kEvChunkOut], t->aux)); FB_CUDA_OK(cudaStreamWaitEvent(st, t->ev[kEvChunkOut], 0)); }
@@ -1790,7 +1807,7 @@ int train_step_launch(fb_qnet *n, const QnetStep &a, int pack_online, int pack_t
     TcPlan *p;
     int rc = make_plan(n, a.B, &p);
     if (rc) return rc;
-    const QnetLayout &L = n->L;
+    const NetLayout &L = n->L;
     const TcWeightMaps &wm = t->wm[0];
     const FwdWs &f = t->ws[0];
     const int B = a.B, H = L.hidden, P1 = B * kP1, P2 = B * kP2;
@@ -1826,7 +1843,7 @@ int train_step_launch(fb_qnet *n, const QnetStep &a, int pack_online, int pack_t
     // ---- aux: Q(s') with the net the variant names (and the online net too for Double)
     if (a.variant != 0 && pack_target) { rc = tc_pack_weights(n, a.target, 1, sx); if (rc) return rc; }
     if (a.variant == 2) { rc = tc_forward(n, 0, 1, a.params, a.fn, B, n->q_next_online, sx); if (rc) return rc; }
-    rc = a.variant == 0 ? tc_forward(n, 0, 1, a.params, a.fn, B, n->q_next, sx) : tc_forward(n, 1, 1, a.target, a.fn, B, n->q_next, sx);
+    rc = a.variant == 0 ? tc_forward(n, 0, 1, a.params, a.fn, B, n->q_next, sx, n->c51_pn) : tc_forward(n, 1, 1, a.target, a.fn, B, n->q_next, sx, n->c51_pn);
     if (rc) return rc;
     if (sampled) FB_CUDA_OK(cudaStreamWaitEvent(sx, t->ev[kEvGather], 0));     // the event below then also says: minibatch buffers complete
     // ---- main: Q(s) with the online net; its activations stay in workspace 0 for the backward pass
@@ -1865,8 +1882,12 @@ int train_step_launch(fb_qnet *n, const QnetStep &a, int pack_online, int pack_t
     // ---- backward.  The head's backward pass rode in the forward's last kernel when hidden = 512 (fc1_head_train_kernel);
     // otherwise: fp32 gradients of the head variables and the fc1 bias straight into partials, dh1 as bf16
     const bool fused_head = fused_head_ok(L);
-    const int G = fused_head ? head_ctas(t, B) : (B + kHeadRows - 1) / kHeadRows;
-    if (!fused_head)
+    const int G = L.atoms ? (B + kC51Rows - 1) / kC51Rows : fused_head ? head_ctas(t, B) : (B + kHeadRows - 1) / kHeadRows;
+    if (L.atoms) {                              // C51: dh1 and the head's partials per row group (fb_c51.cu)
+        rc = c51_launch_head_backward(L, B, f.h1, n->c51_dl, a.params, n->c51_terms, nullptr, nullptr, nullptr, n->c51_hp, n->c51_hb, t->dh1,
+                                      t->f16, gscale, tr.ap, st);
+        if (rc) return rc;
+    } else if (!fused_head)
         FB_CUDA_OK(tc::launch_pdl(head_backward_tc_kernel, dim3(H / 32 + 1, G), dim3(256), 0, st, f.h1, n->dq, a.params, L, B, t->hp, t->hb,
                                   t->loss_terms, t->dh1, tr.ap, GradFmt{t->f16, gscale}));
     cudaStream_t sy = t->aux2;                  // third stream: bias column sums and the early Adam on W_fc1, all off the critical path
@@ -1944,10 +1965,12 @@ int train_step_launch(fb_qnet *n, const QnetStep &a, int pack_online, int pack_t
     FB_CUDA_OK((launch_tc_wgrad<32, 2, kSlabW1, 1, 6>(p->x2_w, p->dz1_b, p->conv1_w, p->s1, EpiStoreF32{t->part1, 256, 32, (size_t)256 * 32}, st)));
     if ((rc = fork(sx, st))) return rc;
     if ((rc = fork(sy, st))) return rc;
-    FinalizeArgs fa{t->part1, t->part2, t->part3, p->s1, p->s2, p->s3, t->bp1, t->bp2, t->bp3, c1, c23, c23, t->hp, t->hb, G, a.loss_out, 1.f / gscale};
+    FinalizeArgs fa{t->part1, t->part2, t->part3, p->s1, p->s2, p->s3, t->bp1, t->bp2, t->bp3, c1, c23, c23, L.atoms ? n->c51_hp : t->hp,
+                    L.atoms ? n->c51_hb : t->hb, G, a.loss_out, 1.f / gscale};
     const int n_compact = L.wf1 + (L.total - L.bf1);
     const int nb_fin = (n_compact + 31) / 32;
-    FB_CUDA_OK(tc::launch_pdl(finalize_grads_kernel, dim3(nb_fin), dim3(32 * kFinWarps), 0, st, fa, L, a.grads, ad, t->pw[0]));
+    FB_CUDA_OK(tc::launch_pdl(L.atoms ? finalize_grads_kernel<true> : finalize_grads_kernel<false>, dim3(nb_fin), dim3(32 * kFinWarps), 0, st, fa,
+                              L, a.grads, ad, t->pw[0], L));
     if (a.ad.on && a.xch != nullptr) {          // the rest of the vector (79,522 parameters): the only exchange left at the tail
         rc = dist_launch_bucket(a.xch, n, 1, const_cast<float *>(a.params), a.ad.m, a.ad.v, t->adam_pow + 2, a.ad.beta1, a.ad.beta2, a.ad.eps,
                                 a.ad.grad_scale, st);

@@ -52,8 +52,15 @@ class FrameBatch:
 class QNetwork:
     def __init__(self, device="cuda:0", hidden: int = 512, dueling: bool = False, max_batch: int = 256, seed: int = 0,
                  lr: float = 1e-6, beta1: float = 0.9, beta2: float = 0.999, adam_eps: float = 1e-8,
-                 copy_target_at_init: bool = False, precision: str = "fp16", noisy: bool = False, sigma0: float = 0.5):
-        """``noisy``: NoisyNet (Fortunato et al. 2018) with factorised Gaussian noise on fc1 and the head (csrc/fb_noisy.cu).
+                 copy_target_at_init: bool = False, precision: str = "fp16", noisy: bool = False, sigma0: float = 0.5,
+                 distributional: bool = False, atoms: int = 51, v_min: float = -10.0, v_max: float = 20.0):
+        """``distributional``: the C51 head (Bellemare et al. 2017, csrc/fb_c51.cu) -- per action a categorical distribution over
+        ``atoms`` atoms spread evenly over [v_min, v_max]; Q is its expectation, so acting is unchanged, and the update minimises the
+        cross-entropy against the projected target distribution (``abs_err`` then receives that cross-entropy, Rainbow's priority).
+        The support defaults to [-10, 20], not the paper's [-10, 10]: with this game's rewards (0.1 per step, +3 per pipe, -3 for a
+        crash) a bird that keeps flying reaches a discounted return near 20 at gamma = 0.99, and a crash gives about -3.
+
+        ``noisy``: NoisyNet (Fortunato et al. 2018) with factorised Gaussian noise on fc1 and the head (csrc/fb_noisy.cu).
         ``params`` / ``target`` are then mu (initialised exactly as without noise), ``sigma`` / ``target_sigma`` start at
         sigma0 / sqrt(fan-in) on the noisy layers and 0 elsewhere, and training and acting run on the effective weights
         mu + sigma * eps of a fresh draw; the noise stream is (``seed``, draw id), the same on every rank."""
@@ -63,7 +70,13 @@ class QNetwork:
         torch.cuda.set_device(self.device)
         self._L = _lib.lib()
         h = C.c_void_p()
-        _lib.check(self._L.fb_qnet_create(hidden, int(dueling), max_batch, C.byref(h)), "fb_qnet_create")
+        self.distributional = bool(distributional)
+        self.atoms, self.v_min, self.v_max = (int(atoms), float(v_min), float(v_max)) if self.distributional else (0, 0.0, 0.0)
+        if self.distributional:
+            _lib.check(self._L.fb_qnet_create_c51(hidden, int(dueling), max_batch, self.atoms, self.v_min, self.v_max, C.byref(h)),
+                       "fb_qnet_create_c51")
+        else:
+            _lib.check(self._L.fb_qnet_create(hidden, int(dueling), max_batch, C.byref(h)), "fb_qnet_create")
         self._h = h
         self.hidden, self.dueling, self.max_batch = hidden, bool(dueling), max_batch
         # "bf16" / "fp16": tcgen05 tensor cores (16-bit operands, fp32 accumulation; fp16 has TF32's significand); "fp32": strict CUDA-core FMA
@@ -160,6 +173,9 @@ class QNetwork:
         """Multi-GPU: keep the gradient vector in an NVLink-mapped exchange buffer and let adam_step() sum every rank's
         gradients from peer memory inside the Adam kernel (csrc/fb_dist.cu) instead of a separate all-reduce."""
         from .dist import PeerGradExchange
+        if self.distributional:
+            raise ValueError("a C51 net takes the all-reduce path (loss_backward, all_reduce(grads), adam_step): the in-step peer exchange "
+                             "is not available with it")
         if self.noisy:
             raise ValueError("a noisy net takes the all-reduce path (loss_backward, all_reduce(grads), adam_step): the peer exchange "
                              "applies plain Adam inside its own kernels")
@@ -194,9 +210,10 @@ class QNetwork:
 
     def view(self, name: str, which: str = "params") -> torch.Tensor:
         """Named slice of a flat vector (which in params/target/grads/adam_m/adam_v), TF shapes."""
+        nv, na = (self.atoms, 2 * self.atoms) if self.distributional else (1, 2)     # C51: column a N + i of the A / plain head
         shapes = {"w1": (8, 8, 4, 32), "b1": (32,), "w2": (4, 4, 32, 64), "b2": (64,), "w3": (3, 3, 64, 64), "b3": (64,),
-                  "wf1": (1600, self.hidden), "bf1": (self.hidden,), "wf2": (self.hidden, 2), "bf2": (2,),
-                  "wv": (self.hidden, 1), "bv": (1,), "wa": (self.hidden, 2), "ba": (2,)}
+                  "wf1": (1600, self.hidden), "bf1": (self.hidden,), "wf2": (self.hidden, na), "bf2": (na,),
+                  "wv": (self.hidden, nv), "bv": (nv,), "wa": (self.hidden, na), "ba": (na,)}
         o = self.offsets[name]
         shp = shapes[name]
         return getattr(self, which)[o:o + int(np.prod(shp))].view(shp)
@@ -224,6 +241,21 @@ class QNetwork:
         _lib.check(self._L.fb_qnet_forward(self._h, p.data_ptr(), fb.ptr, fb.sample_stride, fb.chan_off, fb.batch,
                                            q.data_ptr(), self._stream()), "fb_qnet_forward")
         return q
+
+    def forward_dist(self, fb: FrameBatch, target: bool = False, noise: bool | None = None):
+        """C51 net: (probs f32[B][2][atoms], q f32[B][2]) -- the per-action distributions and their expectations
+        (fb_qnet_forward_dist); a noisy net evaluates the next acting draw as forward() does"""
+        if not self.distributional:
+            raise ValueError("forward_dist needs distributional=True")
+        probs = torch.empty((fb.batch, 2, self.atoms), dtype=torch.float32, device=self.device)
+        q = torch.empty((fb.batch, 2), dtype=torch.float32, device=self.device)
+        p = self.target if target else self.params
+        self._sync_versions()
+        if self.noisy and noise is not False:
+            p = self._act_weights(target)
+        _lib.check(self._L.fb_qnet_forward_dist(self._h, p.data_ptr(), fb.ptr, fb.sample_stride, fb.chan_off, fb.batch, probs.data_ptr(),
+                                                q.data_ptr(), self._stream()), "fb_qnet_forward_dist")
+        return probs, q
 
     def act(self, fb: FrameBatch, epsilon: float, seed: int, first_env_id: int, rng_pos: torch.Tensor,
             actions_out: torch.Tensor, q_out: torch.Tensor, noise: bool | None = None):
@@ -343,7 +375,10 @@ class QNetwork:
     def state_dict(self):
         return {"params": self.params.clone(), "target": self.target.clone(), "adam_m": self.adam_m.clone(),
                 "adam_v": self.adam_v.clone(), "beta1_power": float(self.beta1_power), "beta2_power": float(self.beta2_power),
-                "adam_steps": self.adam_steps, "hidden": self.hidden, "dueling": self.dueling, **self._noise_state()}
+                "adam_steps": self.adam_steps, "hidden": self.hidden, "dueling": self.dueling, **self._noise_state(), **self._dist_state()}
+
+    def _dist_state(self):
+        return {"atoms": self.atoms, "v_min": self.v_min, "v_max": self.v_max} if self.distributional else {}
 
     _NOISE_TENSORS = ("sigma", "target_sigma", "sigma_m", "sigma_v")
 
@@ -356,6 +391,8 @@ class QNetwork:
     def load_state_dict(self, sd):
         assert sd["hidden"] == self.hidden and sd["dueling"] == self.dueling
         assert bool(sd.get("noisy", False)) == self.noisy, "plain and noisy checkpoints are not interchangeable"
+        assert (sd.get("atoms", 0), sd.get("v_min", 0.0), sd.get("v_max", 0.0)) == (self.atoms, self.v_min, self.v_max), \
+            "expected-value and C51 checkpoints (or C51 ones with another support) are not interchangeable"
         for k in ("params", "target", "adam_m", "adam_v") + (self._NOISE_TENSORS if self.noisy else ()):
             getattr(self, k).copy_(sd[k])
         self.beta1_power, self.beta2_power = np.float32(sd["beta1_power"]), np.float32(sd["beta2_power"])

@@ -148,6 +148,17 @@ int fb_resize_tables(int32_t *out_host);
  * the frame ring (acting) or of a gathered replay batch (training). */
 typedef struct fb_qnet fb_qnet;
 int fb_qnet_create(int hidden, int dueling, int max_batch, fb_qnet **out);
+/* The distributional (C51) head (Bellemare et al. 2017; csrc/fb_c51.cu) on the same trunk: per action a categorical
+ * distribution over `atoms` N (2..64) atoms z_i = (float)(v_min + i dz), dz = (v_max - v_min) / (N - 1) in float64.  The head
+ * variables keep their slots in fb_qnet_layout with N outputs per action: W_fc2[H,2N] b_fc2[2N] (column a N + i), or dueling
+ * W_fc2_v[H,N] b_fc2_v[N] W_fc2_a[H,2N] b_fc2_a[2N] with logits v_i + (a_{a,i} - (a_{0,i} + a_{1,i}) / 2).  p = softmax over the
+ * atoms (fp32), Q[a] = sum_i z_i p[a][i]: fb_qnet_forward / fb_qnet_act return Q and act on it unchanged.  In fb_qnet_step the
+ * TD loss becomes the cross-entropy of p[a](s) against the float64 projection m of R + disc z under p[a*](s') (a* the variant's
+ * first argmax of Q(s')): loss = sum_b w_b CE_b (mean losses: / global batch), abs_err_out = CE_b (the Rainbow priority, unweighted
+ * and unscaled), q_target_out = sum_i z_i m_i.  hidden must be a multiple of 32 and at most 2048.  FB_ERR_INVALID for atoms
+ * outside 2..64 or a support that is not finite with v_min < v_max.  A C51 net refuses a step with fb_qnet_set_per_broadcast on and
+ * a non-NULL fb_qnet_attach_exchange (it takes the all-reduce path on several GPUs). */
+int fb_qnet_create_c51(int hidden, int dueling, int max_batch, int atoms, double v_min, double v_max, fb_qnet **out);
 int fb_qnet_destroy(fb_qnet *net);
 
 /* Arithmetic of the contractions (the TF ops of BrainDQN.py:123-154 and their gradients):
@@ -186,6 +197,11 @@ int fb_qnet_layout(const fb_qnet *net, int32_t *out16_host);
 /* QValue.eval (BrainDQN.py:100): q_out_dev f32[batch][2] */
 int fb_qnet_forward(fb_qnet *net, const float *params_dev, const uint8_t *frames_dev, long long sample_stride,
                     const int32_t *chan_off_host4, int batch, float *q_out_dev, void *stream);
+
+/* C51 net only (FB_ERR_INVALID otherwise): the distributions probs_out_dev f32[batch][2][atoms] beside q_out_dev f32[batch][2];
+ * chunked above max_batch like fb_qnet_forward */
+int fb_qnet_forward_dist(fb_qnet *net, const float *params_dev, const uint8_t *frames_dev, long long sample_stride,
+                         const int32_t *chan_off_host4, int batch, float *probs_out_dev, float *q_out_dev, void *stream);
 
 /* getAction (BrainDQN.py:99-108) for `batch` envs: forward, then random.random() <= epsilon ?
  * randrange(2) : argmax.  Env e draws from Philox stream (seed, purpose 2, first_env_id + e) at
@@ -392,6 +408,11 @@ int fb_debug_host_step(int32_t *state16, int action, const uint8_t *gaps, int ga
                        uint64_t env_id, float *reward, uint8_t *terminal, int32_t *score);
 int fb_debug_host_obs(const int32_t *state16, int mode /* 0 tables, 1 per-pixel */, uint8_t *out6400);
 int fb_debug_host_mixed(const int32_t *state16);
+/* device test hook, C51 net: m_out_dev f32[batch][atoms] = the target projection of the training step's loss kernel (the same
+ * device function) of p_next_dev f32[batch][atoms] under the 1-step target (ret_dev / disc_dev NULL: R = r, disc = terminal ? 0 :
+ * gamma) or the n-step one (f64[batch] R and disc) */
+int fb_debug_c51_project(fb_qnet *net, const float *p_next_dev, const float *rewards_dev, const uint8_t *terminals_dev, const double *ret_dev,
+                         const double *disc_dev, double gamma, int batch, float *m_out_dev, void *stream);
 /* device test hook: one raw bf16 GEMM through the tcgen05 kernel of the Q-network path (descriptor self-test).
  * mode 0: D[M][N] = A[M][K] Bt[N][K]^T;  mode 1: D[M][N] = A[K][M]^T B[K][N];  bn = N tile (32/64/128). */
 int fb_debug_tc_gemm(int mode, int bn, int M, int N, int K, const void *a_bf16_dev, const void *b_bf16_dev, float *d_dev,
