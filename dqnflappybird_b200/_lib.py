@@ -124,6 +124,9 @@ _SIGNATURES = {
     "fb_qnet_create_c51": ([C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.c_double, C.POINTER(C.c_void_p)], C.c_int),
     "fb_qnet_forward_dist": ([_vp, _f32p, _u8p, C.c_longlong, _i32p, C.c_int, _f32p, _f32p, _vp], C.c_int),
     "fb_debug_c51_project": ([_vp, _f32p, _f32p, _u8p, _vp, _vp, C.c_double, C.c_int, _f32p, _vp], C.c_int),
+    "fb_qnet_create_qr": ([C.c_int, C.c_int, C.c_int, C.c_int, C.c_double, C.POINTER(C.c_void_p)], C.c_int),
+    "fb_qnet_forward_quantiles": ([_vp, _f32p, _u8p, C.c_longlong, _i32p, C.c_int, _f32p, _f32p, _vp], C.c_int),
+    "fb_debug_qr_loss": ([_vp, _f32p, _f32p, _u8p, _f32p, _u8p, _vp, _vp, C.c_double, C.c_int, _f32p, _f32p, _vp], C.c_int),
     "fb_qnet_destroy": ([_vp], C.c_int),
     "fb_qnet_set_precision": ([_vp, C.c_int], C.c_int),
     "fb_qnet_get_precision": ([_vp], C.c_int),

@@ -32,6 +32,11 @@ on the cross-entropy against the projected target distribution (qnet.py, csrc/fb
 It composes with ``n_step``, ``noisy``, the dueling head and prioritized replay (the cross-entropy is the priority).  The reference's
 broadcast PER loss (``reference_quirks``) has no C51 form, and on several ranks it takes the NCCL all-reduce path.
 
+``quantile=True`` gives the net the QR-DQN head (Dabney et al. 2018) instead: ``quantiles`` learned quantile locations per action
+(32 by default, not the paper's 200), trained by quantile-Huber regression with threshold ``kappa`` (qnet.py, csrc/fb_qr.cu), so
+there is no support to choose; acting takes the argmax of their mean.  It follows the same rules as ``distributional``, and the
+per-sample loss is the priority.
+
 All math runs in libflappy_b200.so; with torch.distributed initialised every rank trains on its own env /
 replay shard and the replicated learner sums the ranks' gradients inside the update's CUDA graph over NVLink
 peer memory (fb_dist.cu), or with an NCCL all-reduce before the Adam step when ``peer_exchange=False``.
@@ -77,7 +82,8 @@ class BrainDQN:
                  reference_quirks: bool = False, copy_target_at_init: bool = False, record: bool = False, max_act_batch: int = 4096,
                  precision: str = "fp16", peer_exchange: bool | None = None, root_dir: str | None = None, save_every: int = SAVE_EVERY,
                  log_capacity: int = 1 << 20, n_step: int = 1, noisy: bool = False, noisy_sigma0: float = 0.5,
-                 distributional: bool = False, atoms: int = 51, v_min: float = -10.0, v_max: float = 20.0):
+                 distributional: bool = False, atoms: int = 51, v_min: float = -10.0, v_max: float = 20.0,
+                 quantile: bool = False, quantiles: int = 32, kappa: float = 1.0):
         if actionNum != 2:
             raise ValueError("the Flappy Bird hot path has two actions (FlappyBirdDQN.py:38)")
         self.actionNum, self.gameName = actionNum, gameName
@@ -98,6 +104,12 @@ class BrainDQN:
             raise ValueError("reference_quirks=True reproduces the reference's squared TD loss; distributional=True replaces it")
         if self.distributional and peer_exchange:
             raise ValueError("distributional=True trains through loss_backward + all_reduce + Adam; the in-step peer exchange is not "
+                             "available with it")
+        self.quantile = bool(quantile)
+        if self.quantile and reference_quirks:
+            raise ValueError("reference_quirks=True reproduces the reference's squared TD loss; quantile=True replaces it")
+        if self.quantile and peer_exchange:
+            raise ValueError("quantile=True trains through loss_backward + all_reduce + Adam; the in-step peer exchange is not "
                              "available with it")
         # distributed: one process per GPU, replicated learner (SURVEY 8e)
         self.world = torch.distributed.get_world_size() if torch.distributed.is_available() and torch.distributed.is_initialized() else 1
@@ -121,7 +133,8 @@ class BrainDQN:
         dueling = self.dueling and not (reference_quirks and type(self).__name__ == "BrainDuelingDQN")
         self.net = QNetwork(self.device, hidden=hidden, dueling=dueling, max_batch=max(self.local_batch, min(N, max_act_batch)),
                             seed=seed, lr=lr, copy_target_at_init=copy_target_at_init, precision=precision, noisy=self.noisy,
-                            sigma0=noisy_sigma0, distributional=self.distributional, atoms=atoms, v_min=v_min, v_max=v_max)
+                            sigma0=noisy_sigma0, distributional=self.distributional, atoms=atoms, v_min=v_min, v_max=v_max,
+                            quantile=self.quantile, quantiles=quantiles, kappa=kappa)
         if self.prioritized and reference_quirks:
             # what the shipped graph really minimises: ISWeights [B,1] x square(...) [B] broadcasts to [B,B], so every sample is
             # weighted by mean(ISWeights) (BrainPrioritizedReplyDQN.py:243-251); the default is the intended per-sample weight
@@ -131,7 +144,8 @@ class BrainDQN:
             raise ValueError("noisy=True trains through loss_backward + all_reduce + the noisy Adam; the in-step peer exchange "
                              "applies plain Adam and is not available with it")
         if peer_exchange is None:
-            peer_exchange = not self.noisy and not self.distributional and self.world > 1 and torch.distributed.get_backend() == "nccl"
+            peer_exchange = (not self.noisy and not self.distributional and not self.quantile and self.world > 1
+                             and torch.distributed.get_backend() == "nccl")
         if peer_exchange and self.world > 1:
             self.net.enable_peer_exchange()
         if self.n_step > 1 and self.prioritized and self.world > 1 and not self.net.exchange_in_step:

@@ -91,7 +91,9 @@ constexpr int kMaxSplits = 5;                        // fc1's K-splits on the te
 size_t fwd_smem(int H, int nc, int N) {
     return sizeof(float) * ((size_t)kFwdSamples * H + (size_t)kFwdWarps * kFwdSamples * nc + nc + N + kFwdWarps * 6 * N);
 }
-template <int KC>
+// kQR: the QR head's per-sample stage instead (fb_qr.cu) -- theta[a][i] = the logit formula, written to probs when set, and
+// Q[a] = (sum_i theta[a][i] in ascending i, fp32 adds) / N; no softmax, logp unused.  The h1 finish and the weight walk are shared.
+template <int KC, bool kQR>
 __global__ void __launch_bounds__(kFwdThreads) c51_head_forward_kernel(const float *__restrict__ part, int splits, size_t split_stride,
                                                                       const float *__restrict__ h1_in, const float *__restrict__ params,
                                                                       NetLayout L, int B, float *__restrict__ h1_out,
@@ -186,6 +188,17 @@ __global__ void __launch_bounds__(kFwdThreads) c51_head_forward_kernel(const flo
         for (int e = lane; e < N2; e += 32) {                 // logits (dueling: v + (alpha - mean_a alpha))
             const int i = e % N;
             ls[e] = L.dueling ? out(i) + (out(N + e) - 0.5f * (out(N + i) + out(N2 + i))) : out(e);
+            if (kQR && probs != nullptr) probs[(size_t)b * N2 + e] = ls[e];
+        }
+        if constexpr (kQR) {
+            __syncwarp();
+            if (lane < 2) {
+                float acc = 0.f;
+                for (int i = 0; i < N; i++) acc += ls[lane * N + i];
+                q[b * 2 + lane] = acc / (float)N;
+            }
+            __syncwarp();
+            continue;
         }
         // max and sum of exp per action: each lane over its own logits, then a butterfly (a fixed order)
         float mx[2] = {-INFINITY, -INFINITY}, sum[2] = {0.f, 0.f};
@@ -231,8 +244,7 @@ __global__ void __launch_bounds__(128) c51_loss_kernel(const LossArgs a, NetLayo
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, N = L.atoms, nc = c51_cols(L);
     const int b = blockIdx.x * 4 + warp;
     if (b >= B) return;
-    const float *qn = a.variant == 2 ? a.q_next_online : a.q_next;
-    const int astar = qn[b * 2 + 1] > qn[b * 2] ? 1 : 0;            // first max on ties
+    const int astar = dist_astar(a.variant == 2 ? a.q_next_online : a.q_next, b);
     double R, d;
     c51_return(a.rewards, a.terminals, a.ret, a.disc, b, a.gamma, &R, &d);
     c51_project_warp(a.pn + ((size_t)b * 2 + astar) * N, R, d, L, scr[warp], ms[warp]);
@@ -242,14 +254,8 @@ __global__ void __launch_bounds__(128) c51_loss_kernel(const LossArgs a, NetLayo
     const float w = a.isw ? a.isw[b] : 1.f, scale = a.loss_sum ? 1.f : 1.f / (float)a.global_batch;
     const float *p = a.ps + ((size_t)b * 2 + act) * N;
     for (int c = lane; c < nc; c += 32) {
-        const int i = c % N, col = L.dueling ? c - N : c;           // col: a N + i of the logit (dueling A columns), < 0 for V
-        const float g = w * scale * (p[i] - m32[warp][i]);
-        const float d0 = act == 0 ? g : 0.f, d1 = act == 1 ? g : 0.f;
-        float v;
-        if (!L.dueling) v = col / N == act ? g : 0.f;
-        else if (col < 0) v = d0 + d1;
-        else v = (col / N == 0 ? d0 : d1) - 0.5f * (d0 + d1);
-        a.dl[(size_t)b * nc + c] = v;
+        const int i = c % N;
+        a.dl[(size_t)b * nc + c] = dist_route(L, c, act, w * scale * (p[i] - m32[warp][i]));
     }
     if (lane == 0) {
         const float *lp = a.logps + ((size_t)b * 2 + act) * N;
@@ -385,9 +391,10 @@ __global__ void __launch_bounds__(128) c51_project_kernel(const float *p_next, c
 int c51_prepare() {
     FB_CUDA_OK(cudaFuncSetAttribute(c51_head_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bwd_smem(kMaxCols)));
     const int fs = (int)fwd_smem(2048, kMaxCols, kC51MaxAtoms);
-    FB_CUDA_OK(cudaFuncSetAttribute(c51_head_forward_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, fs));
-    FB_CUDA_OK(cudaFuncSetAttribute(c51_head_forward_kernel<4>, cudaFuncAttributeMaxDynamicSharedMemorySize, fs));
-    FB_CUDA_OK(cudaFuncSetAttribute(c51_head_forward_kernel<6>, cudaFuncAttributeMaxDynamicSharedMemorySize, fs));
+    for (const void *k : {(const void *)c51_head_forward_kernel<2, false>, (const void *)c51_head_forward_kernel<4, false>,
+                          (const void *)c51_head_forward_kernel<6, false>, (const void *)c51_head_forward_kernel<2, true>,
+                          (const void *)c51_head_forward_kernel<4, true>, (const void *)c51_head_forward_kernel<6, true>})
+        FB_CUDA_OK(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, fs));
     return FB_OK;
 }
 
@@ -395,7 +402,8 @@ int c51_launch_head_forward(const float *part, int splits, size_t split_stride, 
                             int B, float *h1_out, float *probs, float *logp, float *q, cudaStream_t st) {
     FB_REQUIRE(part == nullptr || splits <= kMaxSplits, "c51_launch_head_forward: more fc1 K-splits than the head kernel sums");
     const int nc = c51_cols(L);
-    auto kern = nc <= 64 ? c51_head_forward_kernel<2> : nc <= 128 ? c51_head_forward_kernel<4> : c51_head_forward_kernel<6>;
+    auto kern = L.quantile ? (nc <= 64 ? c51_head_forward_kernel<2, true> : nc <= 128 ? c51_head_forward_kernel<4, true> : c51_head_forward_kernel<6, true>)
+                           : (nc <= 64 ? c51_head_forward_kernel<2, false> : nc <= 128 ? c51_head_forward_kernel<4, false> : c51_head_forward_kernel<6, false>);
     kern<<<(B + kFwdSamples - 1) / kFwdSamples, kFwdThreads, fwd_smem(L.hidden, nc, L.atoms), st>>>(part, splits, split_stride, h1_in, params, L,
                                                                                                     B, h1_out, probs, logp, q);
     FB_CUDA_OK(cudaGetLastError());

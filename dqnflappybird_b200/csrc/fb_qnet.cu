@@ -369,7 +369,7 @@ static void wgrad(fb_qnet *n, int M, int N, int K, int kchunk, AL al, const floa
     splitk_reduce_kernel<<<(unsigned)((mn + 255) / 256), 256, 0, st>>>(n->partial, splits, mn, gout);
 }
 
-// probs / logp (C51 net only, may be nullptr): p and log p of every action's atoms, [B][2][N]
+// probs / logp (C51 net only, may be nullptr): p and log p of every action's atoms, [B][2][N]; a QR net's theta in probs
 static int forward_chunk(fb_qnet *n, const float *params, FrameView fv, int B, float *q_out, cudaStream_t st, float *probs = nullptr,
                          float *logp = nullptr) {
     const NetLayout &L = n->L;
@@ -388,10 +388,10 @@ static int forward_chunk(fb_qnet *n, const float *params, FrameView fv, int B, f
     return FB_OK;
 }
 
-static int create_net(int hidden, int dueling, int max_batch, int atoms, double v_min, double v_max, fb_qnet **out) {
+static int create_net(int hidden, int dueling, int max_batch, int atoms, double v_min, double v_max, int quantile, double kappa, fb_qnet **out) {
     fb_qnet *n = new (std::nothrow) fb_qnet();
     FB_REQUIRE(n != nullptr, "fb_qnet_create: out of host memory");
-    n->L = NetLayout{qnet_layout(hidden, dueling ? 1 : 0, atoms), atoms, v_min, v_max};
+    n->L = NetLayout{qnet_layout(hidden, dueling ? 1 : 0, atoms), atoms, v_min, v_max, quantile, kappa};
     n->max_batch = max_batch;
     n->precision = FB_PRECISION_FP32;
     n->tc = nullptr;
@@ -414,7 +414,8 @@ static int create_net(int hidden, int dueling, int max_batch, int atoms, double 
     FB_CUDA_OK(alloc(&n->loss_dev, 4));
     if (atoms) {
         const size_t G = (B + kC51Rows - 1) / kC51Rows;
-        FB_CUDA_OK(alloc(&n->c51_ps, B * 2 * atoms)); FB_CUDA_OK(alloc(&n->c51_logps, B * 2 * atoms)); FB_CUDA_OK(alloc(&n->c51_pn, B * 2 * atoms));
+        FB_CUDA_OK(alloc(&n->c51_ps, B * 2 * atoms)); FB_CUDA_OK(alloc(&n->c51_pn, B * 2 * atoms));
+        if (!quantile) FB_CUDA_OK(alloc(&n->c51_logps, B * 2 * atoms));
         FB_CUDA_OK(alloc(&n->c51_dl, B * c51_cols(n->L))); FB_CUDA_OK(alloc(&n->c51_terms, B));
         FB_CUDA_OK(alloc(&n->c51_hp, G * c51_partial_stride(n->L))); FB_CUDA_OK(alloc(&n->c51_hb, G * 4));
     }
@@ -424,7 +425,7 @@ static int create_net(int hidden, int dueling, int max_batch, int atoms, double 
 
 extern "C" int fb_qnet_create(int hidden, int dueling, int max_batch, fb_qnet **out) {
     FB_REQUIRE(out != nullptr && hidden > 0 && hidden % 4 == 0 && max_batch > 0, "fb_qnet_create: bad argument");
-    return create_net(hidden, dueling, max_batch, 0, 0.0, 0.0, out);
+    return create_net(hidden, dueling, max_batch, 0, 0.0, 0.0, 0, 0.0, out);
 }
 
 // The distributional (C51) head: atoms outputs per action over the support v_min .. v_max (fb_c51.cu)
@@ -435,7 +436,18 @@ extern "C" int fb_qnet_create_c51(int hidden, int dueling, int max_batch, int at
     FB_REQUIRE(isfinite(v_min) && isfinite(v_max) && v_min < v_max, "fb_qnet_create_c51: the support needs finite v_min < v_max");
     int rc = c51_prepare();
     if (rc) return rc;
-    return create_net(hidden, dueling, max_batch, atoms, v_min, v_max, out);
+    return create_net(hidden, dueling, max_batch, atoms, v_min, v_max, 0, 0.0, out);
+}
+
+// The quantile-regression (QR-DQN) head: `quantiles` outputs per action, quantile-Huber threshold kappa (fb_qr.cu)
+extern "C" int fb_qnet_create_qr(int hidden, int dueling, int max_batch, int quantiles, double kappa, fb_qnet **out) {
+    FB_REQUIRE(out != nullptr && hidden > 0 && hidden % 32 == 0 && hidden <= 2048 && max_batch > 0,
+               "fb_qnet_create_qr: bad argument (hidden must be a multiple of 32, at most 2048)");
+    FB_REQUIRE(quantiles >= 1 && quantiles <= kC51MaxAtoms, "fb_qnet_create_qr: quantiles must be 1..64");
+    FB_REQUIRE(isfinite(kappa) && kappa >= 0.0, "fb_qnet_create_qr: kappa must be finite and >= 0");
+    int rc = c51_prepare();
+    if (rc) return rc;
+    return create_net(hidden, dueling, max_batch, quantiles, 0.0, 0.0, 1, kappa, out);
 }
 
 extern "C" int fb_qnet_destroy(fb_qnet *n) {
@@ -464,7 +476,7 @@ extern "C" int fb_qnet_get_precision(const fb_qnet *n) { return n ? n->precision
 // current buffer (fb_dist_grads / fb_dist_parity) and the caller calls fb_dist_advance after each step.  NULL detaches.
 extern "C" int fb_qnet_attach_exchange(fb_qnet *n, fb_dist *d) {
     FB_REQUIRE(n != nullptr, "fb_qnet_attach_exchange: NULL argument");
-    FB_REQUIRE(d == nullptr || n->L.atoms == 0, "fb_qnet_attach_exchange: a C51 net takes the all-reduce path (no in-step exchange)");
+    FB_REQUIRE(d == nullptr || n->L.atoms == 0, "fb_qnet_attach_exchange: a C51 or QR net takes the all-reduce path (no in-step exchange)");
     n->xch = d;
     return tc_drop_graphs(n);
 }
@@ -531,8 +543,16 @@ extern "C" int fb_qnet_forward(fb_qnet *n, const float *params_dev, const uint8_
 extern "C" int fb_qnet_forward_dist(fb_qnet *n, const float *params_dev, const uint8_t *frames_dev, long long sample_stride,
                                     const int32_t *chan_off, int batch, float *probs_out_dev, float *q_out_dev, void *stream) {
     FB_REQUIRE(n && params_dev && frames_dev && chan_off && probs_out_dev && q_out_dev && batch > 0, "fb_qnet_forward_dist: bad argument");
-    FB_REQUIRE(n->L.atoms > 0, "fb_qnet_forward_dist: the net has the expected-value head (create it with fb_qnet_create_c51)");
+    FB_REQUIRE(n->L.atoms > 0 && !n->L.quantile, "fb_qnet_forward_dist: not a C51 net (create it with fb_qnet_create_c51)");
     return forward_impl(n, params_dev, frames_dev, sample_stride, chan_off, batch, probs_out_dev, q_out_dev, (cudaStream_t)stream);
+}
+
+// QR net: the per-action quantile locations theta_out [batch][2][quantiles] and their means q_out [batch][2]
+extern "C" int fb_qnet_forward_quantiles(fb_qnet *n, const float *params_dev, const uint8_t *frames_dev, long long sample_stride,
+                                         const int32_t *chan_off, int batch, float *theta_out_dev, float *q_out_dev, void *stream) {
+    FB_REQUIRE(n && params_dev && frames_dev && chan_off && theta_out_dev && q_out_dev && batch > 0, "fb_qnet_forward_quantiles: bad argument");
+    FB_REQUIRE(n->L.quantile, "fb_qnet_forward_quantiles: not a QR net (create it with fb_qnet_create_qr)");
+    return forward_impl(n, params_dev, frames_dev, sample_stride, chan_off, batch, theta_out_dev, q_out_dev, (cudaStream_t)stream);
 }
 
 extern "C" int fb_qnet_act(fb_qnet *n, const float *params_dev, const uint8_t *frames_dev, long long sample_stride,
@@ -556,9 +576,12 @@ static int loss_backward_impl(fb_qnet *n, const QnetStep &a, cudaStream_t st) {
     if (a.variant == 2) { rc = forward_chunk(n, a.params, a.fn, B, n->q_next_online, st); if (rc) return rc; }
     rc = forward_chunk(n, a.variant == 0 ? a.params : a.target, a.fn, B, n->q_next, st, n->c51_pn); if (rc) return rc;
     rc = forward_chunk(n, a.params, a.fs, B, n->q, st, n->c51_ps, n->c51_logps); if (rc) return rc;
-    if (L.atoms) {              // C51: projection + cross-entropy, then the head's backward pass (fb_c51.cu)
-        rc = c51_launch_loss(L, B, a.variant, a.loss_sum, a.global_batch, a.gamma, n->c51_ps, n->c51_logps, n->c51_pn, n->q_next, n->q_next_online,
-                             a.actions, a.rewards, a.terminals, a.isw, a.ret, a.disc, n->c51_dl, n->c51_terms, a.abs_err, a.q_target, st);
+    if (L.atoms) {              // C51: projection + cross-entropy (QR: quantile-Huber loss), then the head's backward pass (fb_c51.cu)
+        rc = L.quantile ? qr_launch_loss(L, B, a.variant, a.loss_sum, a.global_batch, a.gamma, n->c51_ps, n->c51_pn, n->q_next, n->q_next_online,
+                                         a.actions, a.rewards, a.terminals, a.isw, a.ret, a.disc, n->c51_dl, n->c51_terms, a.abs_err, a.q_target, st)
+                        : c51_launch_loss(L, B, a.variant, a.loss_sum, a.global_batch, a.gamma, n->c51_ps, n->c51_logps, n->c51_pn, n->q_next,
+                                          n->q_next_online, a.actions, a.rewards, a.terminals, a.isw, a.ret, a.disc, n->c51_dl, n->c51_terms, a.abs_err,
+                                          a.q_target, st);
         if (rc == FB_OK)
             rc = c51_launch_head_backward(L, B, n->h1, n->c51_dl, a.params, n->c51_terms, a.grads, a.loss_out, n->dh1, nullptr, nullptr, nullptr, 0,
                                           1.f, AdamPow{}, st);
@@ -617,7 +640,7 @@ extern "C" int fb_qnet_step(fb_qnet *n, const fb_qnet_step_args *a, void *stream
     } else {
         FB_REQUIRE(a->frames_dev && a->actions_dev && a->rewards_dev && a->terminals_dev, "fb_qnet_step: NULL argument");
     }
-    FB_REQUIRE(n->L.atoms == 0 || !n->per_broadcast, "fb_qnet_step: the reference's broadcast PER loss (fb_qnet_set_per_broadcast) has no C51 form");
+    FB_REQUIRE(n->L.atoms == 0 || !n->per_broadcast, "fb_qnet_step: the reference's broadcast PER loss (fb_qnet_set_per_broadcast) has no C51 or QR form");
     const int batch = sp ? sp->batch : a->batch;
     FB_REQUIRE(batch > 0 && batch <= n->max_batch, "fb_qnet_step: batch outside 1..max_batch");
     const bool tc = tc_precision(n->precision);

@@ -23,12 +23,16 @@ struct QnetLayout {             // offsets (in floats) into the flat parameter v
     int wv, bv, wa, ba;         // dueling heads [H,1],[1],[H,2],[2]  (C51: [H,N],[N],[H,2N],[2N])
     int total;
 };
-// The net's layout with its head: atoms 0 is the expected-value head, 2..64 the distributional (C51) head over N = atoms
-// (fb_c51.cu) with the support z_i = (float)(v_min + i dz), dz = (v_max - v_min) / (N - 1) in float64.  Kept apart from
-// QnetLayout, which the trunk and expected-value head kernels take by value, so that their parameters and code stay as they are.
+// The net's layout with its head: atoms 0 is the expected-value head; atoms N > 0 outputs per action are either the
+// distributional (C51) head over N = 2..64 atoms (fb_c51.cu) with the support z_i = (float)(v_min + i dz), dz = (v_max - v_min) /
+// (N - 1) in float64, or -- quantile set -- the quantile-regression (QR-DQN) head with N = 1..64 quantiles and the quantile-Huber
+// threshold kappa (fb_qr.cu).  Kept apart from QnetLayout, which the trunk and expected-value head kernels take by value, so that
+// their parameters and code stay as they are.
 struct NetLayout : QnetLayout {
     int atoms;
     double v_min, v_max;
+    int quantile;
+    double kappa;
 };
 
 // the offsets; atoms > 0 sizes the C51 head
@@ -92,7 +96,7 @@ __device__ __forceinline__ void adam_pow_advance(const AdamPow &ap) {
     ap.pow[0] = b1p * ap.beta1; ap.pow[1] = b2p * ap.beta2;
 }
 
-// ---- distributional (C51) head, L.atoms > 0 (fb_c51.cu).  Column space of the head's outputs: plain c = a N + i (W_fc2 /
+// ---- distributional heads, L.atoms > 0: C51 (fb_c51.cu) and QR (fb_qr.cu).  Column space of the head's outputs: plain c = a N + i (W_fc2 /
 // b_fc2); dueling c < N the V head's atom c, c = N + a N + i the A head's (a, i).  Per-sample loss gradients are kept in that
 // space ([B][c51_cols]); the backward pass writes per row group partials [G][(H + 1) cols + H]: weight (j, c) at j cols + c,
 // head bias c at H cols + c, fc1 bias j at (H + 1) cols + j.
@@ -117,9 +121,21 @@ __host__ __device__ inline void c51_column(const NetLayout &L, int i, int *j, in
     else if (i < L.ba) { const int e = i - L.wa; *j = e / (2 * N); *c = N + e % (2 * N); }
     else { *j = H; *c = N + i - L.ba; }
 }
+// The loss kernels' shared steps.  a* of sample b: the first argmax of the variant's Q(s') (Double: qn is the online net's)
+__device__ __forceinline__ int dist_astar(const float *qn, int b) { return qn[b * 2 + 1] > qn[b * 2] ? 1 : 0; }
+// dLoss/d(head output c) when g = dLoss/d(output (act, c mod N)) and the other action's outputs get 0: plain, the column of the
+// taken action; dueling, dv_i = sum_a d[a][i] for V columns, dalpha[a][i] = d[a][i] - sum_a d[.][i] / 2 for A columns
+__device__ __forceinline__ float dist_route(const NetLayout &L, int c, int act, float g) {
+    const int N = L.atoms, col = L.dueling ? c - N : c;         // col: a N + i of the output (dueling A columns), < 0 for V
+    const float d0 = act == 0 ? g : 0.f, d1 = act == 1 ? g : 0.f;
+    if (!L.dueling) return col / N == act ? g : 0.f;
+    if (col < 0) return d0 + d1;
+    return (col / N == 0 ? d0 : d1) - 0.5f * (d0 + d1);
+}
 int c51_prepare();              // kernel attributes (once per process, at create)
 // head forward, one warp per sample: h1 from fc1's split-K partials (part != nullptr: sum in order + bias + ReLU, kept in h1_out
-// when that is set) or read from h1_in; probs / logp [B][2][N] when set; q [B][2]
+// when that is set) or read from h1_in; probs / logp [B][2][N] when set; q [B][2].  A QR net (L.quantile): probs receives the
+// quantile locations theta, logp is not written, q = the mean of theta
 int c51_launch_head_forward(const float *part, int splits, size_t split_stride, const float *h1_in, const float *params, const NetLayout &L,
                             int B, float *h1_out, float *probs, float *logp, float *q, cudaStream_t st);
 // target projection, cross-entropy, dLoss/dlogits (column space) and the per-sample outputs.  pn: p of the Q(s') forward
@@ -128,6 +144,12 @@ int c51_launch_loss(const NetLayout &L, int B, int variant, int loss_sum, int gl
                     const float *pn, const float *q_next, const float *q_next_online, const uint8_t *actions, const float *rewards,
                     const uint8_t *terminals, const float *isw, const double *ret, const double *disc, float *dl, float *terms, float *abs_err,
                     float *q_target, cudaStream_t st);
+// QR net: quantile-Huber loss, dLoss/dtheta (column space) and the per-sample outputs (fb_qr.cu).  ths: theta of the training
+// forward on s, thn: theta of the Q(s') forward whose argmax (or, for Double, q_next_online's) picks a*, both [B][2][N]
+int qr_launch_loss(const NetLayout &L, int B, int variant, int loss_sum, int global_batch, double gamma, const float *ths, const float *thn,
+                   const float *q_next, const float *q_next_online, const uint8_t *actions, const float *rewards, const uint8_t *terminals,
+                   const float *isw, const double *ret, const double *disc, float *dl, float *terms, float *abs_err, float *q_target,
+                   cudaStream_t st);
 // head backward.  grads != nullptr (fp32 path): one row group, head weights / biases written into grads, dh1 fp32 into dh1_f32, the
 // loss (terms in order) into loss_out.  Else: row groups of kC51Rows, partials into hp and the loss partial into hb[g * 4 + 2], dh1
 // times gscale rounded to the 16-bit format (f16) into dh1_16, the fc1 bias partial from the rounded values; ap: the fused Adam's alpha
@@ -153,7 +175,8 @@ struct fb_qnet {
     int per_broadcast;            // PER loss as the reference's graph really computes it: every sample weighted by mean(ISWeights)
     const float *packed_src[2];   // parameter vectors the bf16 operand copies (slot 0 online, 1 target) were made from
     // C51 head (L.atoms > 0), allocated at create for max_batch: p and log p of the training forward on s, p of the Q(s')
-    // forward [B][2][N]; dLoss/dlogits [B][c51_cols]; loss terms [B]; head-backward partials [G][c51_partial_stride], [G][4]
+    // forward [B][2][N]; dLoss/dlogits [B][c51_cols]; loss terms [B]; head-backward partials [G][c51_partial_stride], [G][4].
+    // A QR net keeps theta of s in c51_ps and theta of s' in c51_pn, and has no c51_logps
     float *c51_ps, *c51_logps, *c51_pn, *c51_dl, *c51_terms, *c51_hp, *c51_hb;
 };
 
@@ -209,7 +232,7 @@ int tc_drop_graphs(fb_qnet *n);                 // captured steps embed the net'
 void tc_state_destroy(fb_qnet *n);
 int tc_pack_weights(fb_qnet *n, const float *params_dev, int slot /* 0 online, 1 target */, cudaStream_t st);
 int tc_slot_for(fb_qnet *n, const float *params_dev, int want_slot, cudaStream_t st, int *slot_out);
-// probs (C51 net, may be nullptr): p [B][2][N] beside Q
+// probs (C51 / QR net, may be nullptr): p (QR: theta) [B][2][N] beside Q
 int tc_forward(fb_qnet *n, int slot, int ws, const float *params_dev, FrameView fv, int B, float *q_out, cudaStream_t st, float *probs = nullptr);
 int tc_forward_chunks(fb_qnet *n, int slot, const float *params_dev, const uint8_t *frames_dev, long long sample_stride,
                       const int32_t *chan_off, int batch, float *q_out_dev, cudaStream_t st, float *probs_dev = nullptr);

@@ -1746,12 +1746,15 @@ static int run_forward(fb_qnet *n, int slot, int w, const float *params_dev, Fra
     FB_CUDA_OK((launch_tc_gemm<128, 2>(p->a3_k[w], wm.wf1n, p->fc1, dim3((B + 127) / 128, L.hidden / 128, p->sf),
                                        EpiStoreF32{f.parth, B, L.hidden, (size_t)n->max_batch * L.hidden}, st)));
     if (keep) FB_CUDA_OK(cudaStreamWaitEvent(st, tr->join, 0));
-    if (L.atoms) {                             // C51 head (fb_c51.cu); training: h1, p and log p of s kept, then the loss
+    if (L.atoms) {                             // C51 / QR head (fb_c51.cu); training: h1, p and log p (QR: theta) of s kept, then the loss
         const size_t sstride = (size_t)n->max_batch * L.hidden;
         rc = c51_launch_head_forward(f.parth, p->sf, sstride, nullptr, params_dev, L, B, keep ? f.h1 : nullptr, keep ? n->c51_ps : probs,
                                      keep ? n->c51_logps : nullptr, q_out, st);
         if (rc || !keep) return rc;
         const TdFuse &td = tr->td;
+        if (L.quantile)                        // quantile-Huber loss (fb_qr.cu)
+            return qr_launch_loss(L, B, td.variant, td.loss_sum, td.global_batch, td.gamma, n->c51_ps, n->c51_pn, td.q_next, td.q_next_online,
+                                  td.actions, td.rewards, td.terminals, td.isw, td.ret, td.disc, n->c51_dl, n->c51_terms, td.abs_err, td.q_target, st);
         return c51_launch_loss(L, B, td.variant, td.loss_sum, td.global_batch, td.gamma, n->c51_ps, n->c51_logps, n->c51_pn, td.q_next,
                                td.q_next_online, td.actions, td.rewards, td.terminals, td.isw, td.ret, td.disc, n->c51_dl, n->c51_terms,
                                td.abs_err, td.q_target, st);

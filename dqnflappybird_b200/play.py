@@ -77,13 +77,16 @@ def main(argv=None):
     parser.add_argument("--atoms", type=int, default=51, help="atoms of the C51 support")
     parser.add_argument("--v-min", type=float, default=-10.0, help="lowest atom of the C51 support")
     parser.add_argument("--v-max", type=float, default=20.0, help="highest atom of the C51 support")
+    parser.add_argument("--quantile", action="store_true", help="QR-DQN head: --quantiles learned quantiles per action")
+    parser.add_argument("--quantiles", type=int, default=32, help="quantiles per action of the QR-DQN head (1..64)")
+    parser.add_argument("--kappa", type=float, default=1.0, help="threshold of the quantile-Huber loss (0: pure quantile regression)")
     parser.add_argument("--initial-epsilon", type=float, default=None,
                         help="start of the epsilon-greedy schedule (default: the reference's 0.03; 0 explores by noise alone)")
     a = parser.parse_args(argv)
     brain, _, stats = playFlappyBird(a.model, a.envs, a.steps, seed=a.seed, replay_memory_per_env=a.replay_per_env, report_every=a.report_every,
                                      batch_size=a.batch, root_dir=a.root_dir, record=a.root_dir is not None, n_step=a.n_step,
                                      noisy=a.noisy, noisy_sigma0=a.noisy_sigma0, distributional=a.distributional, atoms=a.atoms,
-                                     v_min=a.v_min, v_max=a.v_max,
+                                     v_min=a.v_min, v_max=a.v_max, quantile=a.quantile, quantiles=a.quantiles, kappa=a.kappa,
                                      **({} if a.initial_epsilon is None else {"initial_epsilon": a.initial_epsilon}))
     if a.root_dir is not None:
         brain.save()

@@ -53,8 +53,15 @@ class QNetwork:
     def __init__(self, device="cuda:0", hidden: int = 512, dueling: bool = False, max_batch: int = 256, seed: int = 0,
                  lr: float = 1e-6, beta1: float = 0.9, beta2: float = 0.999, adam_eps: float = 1e-8,
                  copy_target_at_init: bool = False, precision: str = "fp16", noisy: bool = False, sigma0: float = 0.5,
-                 distributional: bool = False, atoms: int = 51, v_min: float = -10.0, v_max: float = 20.0):
-        """``distributional``: the C51 head (Bellemare et al. 2017, csrc/fb_c51.cu) -- per action a categorical distribution over
+                 distributional: bool = False, atoms: int = 51, v_min: float = -10.0, v_max: float = 20.0,
+                 quantile: bool = False, quantiles: int = 32, kappa: float = 1.0):
+        """``quantile``: the QR-DQN head (Dabney et al. 2018, csrc/fb_qr.cu) -- per action ``quantiles`` N (1..64) learned quantile
+        locations at the fractions (2i + 1) / (2N); Q is their mean, so acting is unchanged, and the update minimises the
+        quantile-Huber loss with threshold ``kappa`` (0: the paper's QR-DQN-0, pure quantile regression).  ``abs_err`` receives the
+        per-sample loss.  N defaults to 32, not the paper's 200: the head kernels take at most 64 outputs per action.  There is no
+        support to choose.  Not together with ``distributional``.
+
+        ``distributional``: the C51 head (Bellemare et al. 2017, csrc/fb_c51.cu) -- per action a categorical distribution over
         ``atoms`` atoms spread evenly over [v_min, v_max]; Q is its expectation, so acting is unchanged, and the update minimises the
         cross-entropy against the projected target distribution (``abs_err`` then receives that cross-entropy, Rainbow's priority).
         The support defaults to [-10, 20], not the paper's [-10, 10]: with this game's rewards (0.1 per step, +3 per pipe, -3 for a
@@ -70,11 +77,17 @@ class QNetwork:
         torch.cuda.set_device(self.device)
         self._L = _lib.lib()
         h = C.c_void_p()
+        if quantile and distributional:
+            raise ValueError("quantile=True and distributional=True are two different heads; choose one")
+        self.quantile = bool(quantile)
+        self.quantiles, self.kappa = (int(quantiles), float(kappa)) if self.quantile else (0, 0.0)
         self.distributional = bool(distributional)
         self.atoms, self.v_min, self.v_max = (int(atoms), float(v_min), float(v_max)) if self.distributional else (0, 0.0, 0.0)
         if self.distributional:
             _lib.check(self._L.fb_qnet_create_c51(hidden, int(dueling), max_batch, self.atoms, self.v_min, self.v_max, C.byref(h)),
                        "fb_qnet_create_c51")
+        elif self.quantile:
+            _lib.check(self._L.fb_qnet_create_qr(hidden, int(dueling), max_batch, self.quantiles, self.kappa, C.byref(h)), "fb_qnet_create_qr")
         else:
             _lib.check(self._L.fb_qnet_create(hidden, int(dueling), max_batch, C.byref(h)), "fb_qnet_create")
         self._h = h
@@ -173,6 +186,9 @@ class QNetwork:
         """Multi-GPU: keep the gradient vector in an NVLink-mapped exchange buffer and let adam_step() sum every rank's
         gradients from peer memory inside the Adam kernel (csrc/fb_dist.cu) instead of a separate all-reduce."""
         from .dist import PeerGradExchange
+        if self.quantile:
+            raise ValueError("a QR net takes the all-reduce path (loss_backward, all_reduce(grads), adam_step): the in-step peer exchange "
+                             "is not available with it")
         if self.distributional:
             raise ValueError("a C51 net takes the all-reduce path (loss_backward, all_reduce(grads), adam_step): the in-step peer exchange "
                              "is not available with it")
@@ -210,7 +226,8 @@ class QNetwork:
 
     def view(self, name: str, which: str = "params") -> torch.Tensor:
         """Named slice of a flat vector (which in params/target/grads/adam_m/adam_v), TF shapes."""
-        nv, na = (self.atoms, 2 * self.atoms) if self.distributional else (1, 2)     # C51: column a N + i of the A / plain head
+        n = self.atoms or self.quantiles                                             # C51 / QR: column a N + i of the A / plain head
+        nv, na = (n, 2 * n) if n else (1, 2)
         shapes = {"w1": (8, 8, 4, 32), "b1": (32,), "w2": (4, 4, 32, 64), "b2": (64,), "w3": (3, 3, 64, 64), "b3": (64,),
                   "wf1": (1600, self.hidden), "bf1": (self.hidden,), "wf2": (self.hidden, na), "bf2": (na,),
                   "wv": (self.hidden, nv), "bv": (nv,), "wa": (self.hidden, na), "ba": (na,)}
@@ -256,6 +273,21 @@ class QNetwork:
         _lib.check(self._L.fb_qnet_forward_dist(self._h, p.data_ptr(), fb.ptr, fb.sample_stride, fb.chan_off, fb.batch, probs.data_ptr(),
                                                 q.data_ptr(), self._stream()), "fb_qnet_forward_dist")
         return probs, q
+
+    def forward_quantiles(self, fb: FrameBatch, target: bool = False, noise: bool | None = None):
+        """QR net: (theta f32[B][2][quantiles], q f32[B][2]) -- the per-action quantile locations and their means
+        (fb_qnet_forward_quantiles); a noisy net evaluates the next acting draw as forward() does"""
+        if not self.quantile:
+            raise ValueError("forward_quantiles needs quantile=True")
+        theta = torch.empty((fb.batch, 2, self.quantiles), dtype=torch.float32, device=self.device)
+        q = torch.empty((fb.batch, 2), dtype=torch.float32, device=self.device)
+        p = self.target if target else self.params
+        self._sync_versions()
+        if self.noisy and noise is not False:
+            p = self._act_weights(target)
+        _lib.check(self._L.fb_qnet_forward_quantiles(self._h, p.data_ptr(), fb.ptr, fb.sample_stride, fb.chan_off, fb.batch, theta.data_ptr(),
+                                                     q.data_ptr(), self._stream()), "fb_qnet_forward_quantiles")
+        return theta, q
 
     def act(self, fb: FrameBatch, epsilon: float, seed: int, first_env_id: int, rng_pos: torch.Tensor,
             actions_out: torch.Tensor, q_out: torch.Tensor, noise: bool | None = None):
@@ -378,6 +410,8 @@ class QNetwork:
                 "adam_steps": self.adam_steps, "hidden": self.hidden, "dueling": self.dueling, **self._noise_state(), **self._dist_state()}
 
     def _dist_state(self):
+        if self.quantile:
+            return {"quantiles": self.quantiles, "kappa": self.kappa}
         return {"atoms": self.atoms, "v_min": self.v_min, "v_max": self.v_max} if self.distributional else {}
 
     _NOISE_TENSORS = ("sigma", "target_sigma", "sigma_m", "sigma_v")
@@ -393,6 +427,8 @@ class QNetwork:
         assert bool(sd.get("noisy", False)) == self.noisy, "plain and noisy checkpoints are not interchangeable"
         assert (sd.get("atoms", 0), sd.get("v_min", 0.0), sd.get("v_max", 0.0)) == (self.atoms, self.v_min, self.v_max), \
             "expected-value and C51 checkpoints (or C51 ones with another support) are not interchangeable"
+        assert (sd.get("quantiles", 0), sd.get("kappa", 0.0)) == (self.quantiles, self.kappa), \
+            "QR checkpoints are not interchangeable with other heads, nor with QR ones of another quantile count or kappa"
         for k in ("params", "target", "adam_m", "adam_v") + (self._NOISE_TENSORS if self.noisy else ()):
             getattr(self, k).copy_(sd[k])
         self.beta1_power, self.beta2_power = np.float32(sd["beta1_power"]), np.float32(sd["beta2_power"])

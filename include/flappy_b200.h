@@ -159,6 +159,18 @@ int fb_qnet_create(int hidden, int dueling, int max_batch, fb_qnet **out);
  * outside 2..64 or a support that is not finite with v_min < v_max.  A C51 net refuses a step with fb_qnet_set_per_broadcast on and
  * a non-NULL fb_qnet_attach_exchange (it takes the all-reduce path on several GPUs). */
 int fb_qnet_create_c51(int hidden, int dueling, int max_batch, int atoms, double v_min, double v_max, fb_qnet **out);
+/* The quantile-regression (QR-DQN) head (Dabney, Rowland, Bellemare and Munos 2018; csrc/fb_qr.cu) on the same trunk: per action
+ * `quantiles` N (1..64) quantile locations theta[a][i] at the fractions tau_i = (2i + 1) / (2N).  The head variables keep the C51
+ * head's slots and column routing with N outputs per action (theta takes the place of the logits; dueling: v_i + (a_{a,i} -
+ * (a_{0,i} + a_{1,i}) / 2)).  Q[a] = (1/N) sum_i theta[a][i] (fp32, ascending i): fb_qnet_forward / fb_qnet_act return Q and act
+ * on it unchanged.  In fb_qnet_step the TD loss becomes the quantile-Huber loss: a* the variant's first argmax of Q(s') (Double:
+ * online argmax, target theta), T_j = the expected-value head's TD target of theta[a*][j](s') (1-step or n-step, same rounding),
+ * u_ij = T_j - theta[a_b][i](s), L_b = sum_i (1/N) sum_j |tau_i - 1{u_ij < 0}| H(u_ij) with H(u) = u^2 / (2 kappa) for |u| <= kappa,
+ * else |u| - kappa / 2 (kappa = 0: H(u) = |u|); loss = sum_b w_b L_b (mean losses: / global batch), abs_err_out = L_b (the priority,
+ * unweighted and unscaled), q_target_out = (1/N) sum_j T_j.  hidden must be a multiple of 32 and at most 2048.  FB_ERR_INVALID for
+ * quantiles outside 1..64 or a kappa that is negative or not finite.  A QR net refuses what a C51 net refuses (fb_qnet_set_per_broadcast
+ * in a step, a non-NULL fb_qnet_attach_exchange) and fb_qnet_forward_dist. */
+int fb_qnet_create_qr(int hidden, int dueling, int max_batch, int quantiles, double kappa, fb_qnet **out);
 int fb_qnet_destroy(fb_qnet *net);
 
 /* Arithmetic of the contractions (the TF ops of BrainDQN.py:123-154 and their gradients):
@@ -202,6 +214,11 @@ int fb_qnet_forward(fb_qnet *net, const float *params_dev, const uint8_t *frames
  * chunked above max_batch like fb_qnet_forward */
 int fb_qnet_forward_dist(fb_qnet *net, const float *params_dev, const uint8_t *frames_dev, long long sample_stride,
                          const int32_t *chan_off_host4, int batch, float *probs_out_dev, float *q_out_dev, void *stream);
+
+/* QR net only (FB_ERR_INVALID otherwise): the quantile locations theta_out_dev f32[batch][2][quantiles] beside their means
+ * q_out_dev f32[batch][2]; chunked above max_batch like fb_qnet_forward */
+int fb_qnet_forward_quantiles(fb_qnet *net, const float *params_dev, const uint8_t *frames_dev, long long sample_stride,
+                              const int32_t *chan_off_host4, int batch, float *theta_out_dev, float *q_out_dev, void *stream);
 
 /* getAction (BrainDQN.py:99-108) for `batch` envs: forward, then random.random() <= epsilon ?
  * randrange(2) : argmax.  Env e draws from Philox stream (seed, purpose 2, first_env_id + e) at
@@ -413,6 +430,13 @@ int fb_debug_host_mixed(const int32_t *state16);
  * gamma) or the n-step one (f64[batch] R and disc) */
 int fb_debug_c51_project(fb_qnet *net, const float *p_next_dev, const float *rewards_dev, const uint8_t *terminals_dev, const double *ret_dev,
                          const double *disc_dev, double gamma, int batch, float *m_out_dev, void *stream);
+/* device test hook, QR net: the training step's quantile-Huber loss (the same device function) on given theta.  theta_s_dev
+ * f32[batch][2][quantiles] (theta of s), theta_next_astar_dev f32[batch][quantiles] (theta[a*] of s'), actions u8[batch]; the 1-step
+ * target (ret_dev / disc_dev NULL: rewards and terminals) or the n-step one (f64[batch] R and disc).  dtheta_out_dev
+ * f32[batch][quantiles] = dL_b/dtheta[a_b][i] and loss_b_out_dev f32[batch] = L_b, unweighted and unscaled */
+int fb_debug_qr_loss(fb_qnet *net, const float *theta_s_dev, const float *theta_next_astar_dev, const uint8_t *actions_dev, const float *rewards_dev,
+                     const uint8_t *terminals_dev, const double *ret_dev, const double *disc_dev, double gamma, int batch, float *dtheta_out_dev,
+                     float *loss_b_out_dev, void *stream);
 /* device test hook: one raw bf16 GEMM through the tcgen05 kernel of the Q-network path (descriptor self-test).
  * mode 0: D[M][N] = A[M][K] Bt[N][K]^T;  mode 1: D[M][N] = A[K][M]^T B[K][N];  bn = N tile (32/64/128). */
 int fb_debug_tc_gemm(int mode, int bn, int M, int N, int K, const void *a_bf16_dev, const void *b_bf16_dev, float *d_dev,
